@@ -81,6 +81,9 @@ def parse_args():
                          "bit-identical to the CPU oracle (modes 0)")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the strong-scaling, config-4 and H2D-roof records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (audio, frame and group counts, groups "
+                         "and block status of a fixed sample of rank 0's channels) to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -347,6 +350,35 @@ class Workload:
         barrier()
         return ev0.elapsed_time(ev1), self.eng.launch_count() - l0
 
+    def dump_outputs(self, out_dir: str, max_bytes: int = 60 << 20):
+        """What the last step returned, for comparing two builds output for output (the seeded inputs
+        and the number of steps fix it): audio [k, 2, cap] (float32, zero past n_audio) and, as
+        float64, n_audio [k], groups [k, gcap, 6] (a, b, c, d, errors, block_index; zero past
+        n_groups), n_groups [k] and status [k, blocks, 5] (n_audio, stereo, pilot_tenths, clip_ratio,
+        n_groups) of the channels listed in channels [k], a seeded sample when all of them would
+        exceed max_bytes."""
+        import numpy as np
+        import torch
+        C = self.C
+        per_channel = 4 * 2 * self.acap + 8 * (2 + 6 * self.gcap + 5 * self.B + 1)
+        k = min(C, max_bytes // per_channel)
+        pick = np.sort(np.random.default_rng(0).choice(C, k, replace=False)) if k < C else np.arange(C)
+        idx = torch.from_numpy(pick).to(self.dev)
+        n_audio = self.n_audio.index_select(0, idx).cpu().numpy()
+        n_groups = self.n_groups.index_select(0, idx).cpu().numpy()
+        audio = self.audio.index_select(0, idx).cpu().numpy()
+        audio = np.where(np.arange(self.acap)[None, None, :] < n_audio[:, None, None], audio, np.float32(0))
+        g = self.groups.index_select(0, idx).cpu().numpy().view(self.fm.GROUP_DTYPE).reshape(k, self.gcap)
+        groups = np.stack([g[f].astype(np.float64) for f in ("a", "b", "c", "d", "errors", "block_index")], -1)
+        groups[np.arange(self.gcap)[None, :] >= n_groups[:, None]] = 0.0
+        st = self.status.index_select(0, idx).cpu().numpy().view(self.fm.STATUS_DTYPE).reshape(k, self.B)
+        status = np.stack([st[f].astype(np.float64) for f in self.fm.STATUS_DTYPE.names], -1)
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in (("channels", pick.astype(np.float64)), ("audio", audio),
+                        ("n_audio", n_audio.astype(np.float64)), ("groups", groups),
+                        ("n_groups", n_groups.astype(np.float64)), ("status", status)):
+            np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
     def stage_times(self, stream, reps=3):
         """Every stage's kernels alone: the block pipeline queued on ONE stream (overlap off)."""
         import torch
@@ -488,6 +520,8 @@ def run_b200(args, rank: int, local_rank: int, world: int):
     w1 = time.time()
     clocks = sampler.stop(w0, w1)
     ms = shard.max_over_ranks(ms_rank, dev)
+    if args.dump_outputs and rank == 0:
+        wl.dump_outputs(args.dump_outputs)   # before stage_times() runs further steps
     samples_per_step_rank = C * wl.n_iq
     value = shard.aggregate_throughput(samples_per_step_rank, args.steps, world, ms)  # MS/s, whole job
 

@@ -30,7 +30,7 @@ def build(force: bool = False) -> None:
     ref_deps = ("oracle_capi.cpp", "liquid_restated.hpp", "Makefile",
                 os.path.join("liquid_shim", "liquid_shim.cpp"),
                 os.path.join("liquid_shim", "liquid", "liquid.h"))
-    need = force or stale("liboracle_libm.so", oracle_deps) or stale("liboracle_fm.so", oracle_deps) \
+    need = force or any(stale(f"liboracle_{m}.so", oracle_deps) for m in ("libm", "libm_contract", "fm")) \
         or stale("libsiggen.so", ("siggen.cpp", "Makefile"))
     have_ref_src = os.path.isdir("/root/reference/src/redsea_port")
     ref_missing = have_ref_src and not all(
@@ -100,7 +100,8 @@ def _p(a, t):
 
 class OracleLib:
     """One flavour of the oracle: math='libm' (faithful) or 'fm' (engine-shared kernels) are the
-    restated pipeline; 'ref' is the REFERENCE's own sources compiled unmodified over
+    restated pipeline, 'libm_contract' the faithful one with gcc's default FMA contraction; 'ref'
+    is the REFERENCE's own sources compiled unmodified over
     liquid_shim/ (oracle/_ref/libfmref.so, -ffp-contract=off) and 'ref_contract' the same with
     gcc's default FMA contraction. The reference flavours have the channel- and class-level
     entry points only (no design getters, no block-sync / math hooks)."""

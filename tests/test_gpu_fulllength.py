@@ -9,16 +9,17 @@
     (tests/test_oracle_vs_reference.py) — with PI / PS / RT decoded from the groups and compared.
 (b) config 5: 320 distinct channels, SNR 10..40 dB, 3 s each, blend mode c % 3, dsp_agc fast,
     against the reference-faithful flavour: per 5 dB bucket the RDS group exact-match rate, audio
-    max-abs error and SNR after lock, lock-block equality, pilot level difference; the table goes
-    to gpurun_out/parity_sweep.json (copied to profiles/ and DESIGN.md). Gate, every bucket at or
-    above 20 dB: on every channel that the reference's own two builds (strict -ffp-contract=off
-    and stock -mfma contraction, libfmref_contract.so) decode identically, the engine's groups
-    are byte-equal; lock blocks equal, pilot level within 1, audio in tolerance. Groups may
+    max-abs error and SNR after lock, lock-block equality, pilot level difference; the table is
+    printed and saved as JSON (copied to profiles/ and DESIGN.md). Gate, every bucket at or
+    above 20 dB: on every channel that the faithful flavour's two builds (strict -ffp-contract=off
+    and stock -mfma contraction: oracle/_ref/libfmref_contract.so when the reference was built,
+    else the restatement's oracle/liboracle_libm_contract.so) decode identically, the engine's
+    groups are byte-equal; lock blocks equal, pilot level within 1, audio in tolerance. Groups may
     differ only on channels at the RDS decoding threshold, where any change of rounding — the
     reference's own compiler flags, the engine's last-ulp sin/cos/atan2/exp/log, the tensor-core
     decimator's single rounding — decides marginal bits; there the aligned group sequences may
-    differ in no more than twice as many groups as the reference's stock build differs from its
-    strict build. With the FP32 decimator (mode 0) the
+    differ in no more than twice as many groups as the stock build differs from the strict
+    build. With the FP32 decimator (mode 0) the
     engine additionally reproduces every group the reference decodes clean.
 """
 import difflib
@@ -41,6 +42,15 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def faithful_lib():
     """The reference-faithful CPU flavour: the reference's own code when it was built."""
     return orc.OracleLib("ref") if orc.OracleLib.have_ref("ref") else orc.OracleLib("libm")
+
+
+def stock_build_lib():
+    """The faithful flavour built with gcc's default FMA contraction: the reference's own stock build
+    when it was built, else the restatement's. The sweep checks that the one it uses marks as many
+    threshold channels, differing in as many groups, per SNR bucket as the reference's stock build
+    did (tests/golden/reference_sweep_buckets.json)."""
+    return (orc.OracleLib("ref_contract") if orc.OracleLib.have_ref("ref_contract")
+            else orc.OracleLib("libm_contract"))
 
 
 def audio_start(status, extra_blocks=2, never=8):
@@ -100,7 +110,7 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
     iq_rate, decim = rates("240k")
     n_ch, nblk, chunk, per_pass = 320, 88, 8, 80     # 88 blocks = 3.0 s
     faith_lib = faithful_lib()
-    stock_lib = orc.OracleLib("ref_contract") if orc.OracleLib.have_ref("ref_contract") else None
+    stock_lib = stock_build_lib()
     rows = []
     orc.config1_signal(fs_iq=iq_rate).generate(16)   # builds the generator's pulse table once
 
@@ -108,7 +118,7 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
         sig = _sweep_signal(c, n_ch, iq_rate)
         iq = sig.generate(nblk * 8192 * decim)
         cfg = orc.make_config(iq_rate=iq_rate, decimation=decim, dsp_agc=1, stereo_blend=c % 3)
-        stock = orc.Channel(stock_lib, cfg).process(iq).groups if stock_lib else None
+        stock = orc.Channel(stock_lib, cfg).process(iq).groups
         return (iq, orc.Channel(faith_lib, cfg).process(iq), orc.Channel(orc_fm, cfg).process(iq),
                 sig.snr_db, stock)
 
@@ -152,7 +162,7 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
                 clean = [k for k in range(nref) if faith.groups[k]["errors"] == 0]
                 clean_same = sum(same_at(g, k) for k in clean)
                 gpu_diff = unmatched(g)
-                stock_diff = unmatched(stock) if stock is not None else None
+                stock_diff = unmatched(stock)
                 err = max(float(np.abs(a[0][s0:] - faith.left[s0:]).max()),
                           float(np.abs(a[1][s0:] - faith.right[s0:]).max()))
                 rows.append(dict(
@@ -160,8 +170,8 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
                     groups_same=int(same), groups_equal=bool(groups_equal(g, faith.groups)),
                     clean_ref=len(clean), clean_same=int(clean_same), stock_build_diff=stock_diff,
                     gpu_diff=int(gpu_diff),
-                    # "robust": the reference's own two builds decode this channel identically
-                    robust=bool(stock is None or (stock_diff == 0)),
+                    # "robust": the faithful flavour's two builds decode this channel identically
+                    robust=bool(stock_diff == 0),
                     lock_ref=lock, lock_gpu=lock_gpu,
                     stereo_flags_equal=bool(np.array_equal(st["stereo"], faith.status["stereo"])),
                     pilot_diff=int(np.abs(st["pilot_tenths"] - faith.status["pilot_tenths"]).max()),
@@ -180,8 +190,7 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
                                     if sum(r["groups_ref"] for r in b) else
                                     float(sum(r["groups_gpu"] for r in b) == 0)),
             groups_different=sum(r["gpu_diff"] for r in b),
-            reference_stock_build_groups_different=(sum(r["stock_build_diff"] for r in b)
-                                                    if stock_lib else None),
+            reference_stock_build_groups_different=sum(r["stock_build_diff"] for r in b),
             clean_groups_ref=sum(r["clean_ref"] for r in b),
             clean_group_match_rate=(sum(r["clean_same"] for r in b) / sum(r["clean_ref"] for r in b)
                                     if sum(r["clean_ref"] for r in b) else 1.0),
@@ -195,7 +204,7 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
             audio_maxabs=max(r["audio_maxabs"] for r in b),
             audio_snr_db_min=min(r["audio_snr_db"] for r in b)))
     out = dict(config="BASELINE config 5: 320 channels x 3 s, SNR 10-40 dB, blend c%3, dsp_agc fast",
-               reference_flavour=faith_lib.math,
+               reference_flavour=faith_lib.math, stock_build_flavour=stock_lib.math,
                arithmetic=("fast: tensor-core int8 decimator, fused tensor-core channel filter + discriminator "
                            "(AGC elided), tensor-core pilot / low-pass FIRs, scans (modes 1)" if mode else
                            "reference order everywhere (modes 0)"),
@@ -204,6 +213,14 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
     with open(os.path.join(ROOT, "gpurun_out", f"parity_sweep_mode{mode}.json"), "w") as f:
         json.dump(out, f, indent=1)
     print(json.dumps(out, indent=1))
+    # The reference side of the table as the reference's own two builds computed it: the faithful
+    # flavour's groups and locks, and which channels its stock build decodes differently (the
+    # channels the gate below treats as threshold channels) must be what the reference gave.
+    with open(os.path.join(ROOT, "tests", "golden", "reference_sweep_buckets.json")) as f:
+        recorded = json.load(f)["buckets"]
+    assert len(recorded) == len(table)
+    for t, r in zip(table, recorded):
+        assert {k: t[k] for k in r} == r, (t, r)
     for t in table:
         if int(t["snr_bucket_db"].split("-")[0]) >= 20:
             # bit-exact wherever the reference is bit-stable under its own build variation
@@ -211,9 +228,8 @@ def test_config5_weak_signal_sweep_vs_faithful_reference(orc_fm, mode):
             if mode == 0:
                 assert t["clean_groups_ref"] > 1000 and t["clean_group_match_rate"] == 1.0, t
                 assert t["group_exact_match_rate"] >= 0.99, t
-            if stock_lib:
-                # threshold channels: no further from the strict reference than its own stock build
-                # (aligned sequences; twice its count leaves room for which marginal bits flip)
-                assert t["groups_different"] <= max(2, 2 * t["reference_stock_build_groups_different"]), t
+            # threshold channels: no further from the strict reference than its own stock build
+            # (aligned sequences; twice its count leaves room for which marginal bits flip)
+            assert t["groups_different"] <= max(2, 2 * t["reference_stock_build_groups_different"]), t
             assert t["lock_block_equal"] == 1.0 and t["pilot_tenths_maxdiff"] <= 1, t
             assert t["audio_maxabs"] <= 1e-4 or t["audio_snr_db_min"] >= 90.0, t
