@@ -61,7 +61,6 @@ constexpr int TC_B_BYTES = TC_B_CHUNKS * TC_N * TC_CHUNK;   // 112 KB
 // TMEM: a slot is free again as soon as its four tcgen05.cp retire, so the ring only covers the TMA
 // latency (five slots; B takes 112 KB of the CTA's 194 KB).
 constexpr int TC_RING_TMEM_A = 5;
-constexpr int TC_RING_MAX = 6;
 constexpr int TC_ACC = 2;             // (the form with the A operand in shared memory is not built any more)
 // TMEM: columns [0, 256) hold a ring of eight chunks (32 columns = 128 bytes of K per lane; a tile's
 // window touches up to eight), columns [256, 512) two accumulators of 128 columns
@@ -550,7 +549,7 @@ cudaError_t launchDecimTc(int M, int L, const uint8_t *iq, size_t iq_stride, siz
     for (const void *f : fs) {
       if (err == cudaSuccess) {
         err = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   static_cast<int>(tcSmemBytes(TC_RING_MAX)));
+                                   static_cast<int>(tcSmemBytes(TC_RING_TMEM_A)));
       }
     }
     return err;
@@ -582,14 +581,8 @@ cudaError_t launchDecimTc(int M, int L, const uint8_t *iq, size_t iq_stride, siz
     return cudaErrorInvalidValue;
   }
   const int grid = std::min(sm_count, p.row_tiles * p.n_seg);
-  // FMGPU_TC_RING: measurement override of the shared-memory ring depth
-  static const int ring_slots = [] {
-    const char *v = getenv("FMGPU_TC_RING");
-    const int r = v ? atoi(v) : TC_RING_TMEM_A;
-    return std::min(TC_RING_MAX, std::max(2, r));
-  }();
-  p.ring = ring_slots;
-  const size_t smem_bytes = tcSmemBytes(ring_slots);
+  p.ring = TC_RING_TMEM_A;
+  const size_t smem_bytes = tcSmemBytes(TC_RING_TMEM_A);
   const uint4 *bi = reinterpret_cast<const uint4 *>(b_image_dev);
   const int2 *of = reinterpret_cast<const int2 *>(offs_dev);
 #define FMGPU_TC_LAUNCH(KSV)                                                                              \

@@ -1306,11 +1306,6 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
   // K >= 3: a producer waits for the readers of block q - K + 1 (their halo is the tail of the slot
   // it overwrites), so three slots are what lets neighbouring stages of successive blocks overlap
   e->K = (e->N % 32 == 0) ? std::max(3, e->maxBlocks) : 1;
-  if (const char *rk = getenv("FMGPU_RING_K")) {  // deeper ring: stages may run further ahead
-    if (e->K > 1) {
-      e->K = std::max(e->K, std::min(16, atoi(rk)));
-    }
-  }
   if (e->K == 1 && e->maxBlocks > 1) {
     e->lastError = "fmgpu_engine_create: max_blocks > 1 needs block_samples to be a multiple of 32";
     g_create_error = e->lastError;
@@ -1372,9 +1367,6 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
       e->smCount = sms;
     }
     e->k.sm_rot = e->smCount;
-    if (const char *sr = getenv("FMGPU_STEREO_ROT")) {   // measurement override: 0 = no rotation
-      e->k.sm_rot = atoi(sr);
-    }
     if (e->M > 1 && decimTcSupported(e->M, e->decL, e->N)) {
       std::vector<uint8_t> bimg;
       std::vector<int32_t> offs;

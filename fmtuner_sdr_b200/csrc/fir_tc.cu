@@ -699,15 +699,6 @@ static cudaError_t firTcAttrs() {
   });
 }
 
-// staging depth: FMGPU_FT_NSTG is a measurement override
-static int firTcStages() {
-  static const int n = [] {
-    const char *v = getenv("FMGPU_FT_NSTG");
-    return std::min(FT_NSTG_MAX, std::max(2, v ? atoi(v) : FT_NSTG_DEFAULT));
-  }();
-  return n;
-}
-
 cudaError_t launchFirTc(const FirRealJob &job, int nsig, int nch, const FirTcTables &t,
                         const uint8_t *b_image_dev, int data_shift, int sm_count, cudaStream_t stream) {
   const cudaError_t attr_err = firTcAttrs();
@@ -733,7 +724,7 @@ cudaError_t launchFirTc(const FirRealJob &job, int nsig, int nch, const FirTcTab
   p.off4 = t.off[2];
   p.dscale = static_cast<float>(std::ldexp(1.0, data_shift));
   p.out_scale = static_cast<float>(std::ldexp(static_cast<double>(job.scale), -(t.shift + data_shift)));
-  p.nstg = firTcStages();
+  p.nstg = FT_NSTG_DEFAULT;
   const size_t smem = ftSmemBytes(t.ksteps, p.nstg);
   CUtensorMap tm_in[2], tm_out[2];
   for (int s = 0; s < 2; s++) {
@@ -861,7 +852,7 @@ cudaError_t launchChanDemodTc(const float2 *x2, size_t x2_pitch, int in_off, flo
   p.dscale = static_cast<float>(std::ldexp(1.0, data_shift));
   p.out_scale = static_cast<float>(std::ldexp(static_cast<double>(chan_scale), -(t.shift + data_shift)));
   p.nch = nch;
-  p.nstg = firTcStages();
+  p.nstg = FT_NSTG_DEFAULT;
   const size_t smem = ftSmemBytes(t.ksteps, p.nstg);
   p.fd_ref = fd_ref;
   p.y_prev = y_io + static_cast<size_t>(ch0) * y_pitch + Y_OFF - 1;

@@ -142,19 +142,15 @@ __device__ __forceinline__ float divBy57000(float a) {
 // result is bit-identical to two fmaf() calls. ptxas folds the {h, h} pair into a scalar
 // (uniform-register) operand. The FIR kernels are issue-bound (ncu r01: 83 % of issue slots,
 // FMA pipe 50 %): halving the FMA instruction count frees the slots for the LDS / LDCU traffic.
-template <bool PACK>
 __device__ __forceinline__ float2 fma2(float h, float2 x, float2 acc) {
-  if (PACK) {
-    unsigned long long hh, xx, aa, r;
-    asm("mov.b64 %0, {%1, %1};" : "=l"(hh) : "f"(h));
-    asm("mov.b64 %0, {%1, %2};" : "=l"(xx) : "f"(x.x), "f"(x.y));
-    asm("mov.b64 %0, {%1, %2};" : "=l"(aa) : "f"(acc.x), "f"(acc.y));
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(hh), "l"(xx), "l"(aa));
-    float2 o;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(o.x), "=f"(o.y) : "l"(r));
-    return o;
-  }
-  return make_float2(fmaf(h, x.x, acc.x), fmaf(h, x.y, acc.y));
+  unsigned long long hh, xx, aa, r;
+  asm("mov.b64 %0, {%1, %1};" : "=l"(hh) : "f"(h));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(xx) : "f"(x.x), "f"(x.y));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(aa) : "f"(acc.x), "f"(acc.y));
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(hh), "l"(xx), "l"(aa));
+  float2 o;
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(o.x), "=f"(o.y) : "l"(r));
+  return o;
 }
 
 // One uint8 IQ pair (I in byte 0, Q in byte 1) -> ((float)byte - 127.5f) * (1 / 127.5f), the
@@ -191,17 +187,11 @@ __device__ __forceinline__ float2 iqBytesToFloat(uint32_t w) {
 // 16-byte transfers and a warp's 128-bit row access is conflict-free (32-bit accesses of the same
 // rows hit only 8 banks).
 // ---------------------------------------------------------------------------
-#ifndef FMGPU_LT
-#define FMGPU_LT 32
-#endif
-#ifndef FMGPU_ST
-#define FMGPU_ST 16
-#endif
 // samples per tile row of the lane kernels (LT: k_dcblock, k_agc, k_rds; ST: k_stereo). Measured:
 // the shared memory the lane kernels hold does not move the 10,000-channel step (DESIGN.md 4a);
 // shorter k_stereo tiles lengthen that kernel by 10 % (one block barrier per tile).
-constexpr int LT = FMGPU_LT;
-constexpr int STEREO_ST = FMGPU_ST;
+constexpr int LT = 32;
+constexpr int STEREO_ST = 16;
 
 __device__ __forceinline__ void cpAsync16(void *smem, const void *gmem) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(
@@ -420,89 +410,15 @@ __global__ void k_save_tail(const float *src, size_t src_pitch, int src_off, flo
 // Input bytes are fetched as 128-bit words from the 16-byte aligned virtual stream
 // hist ++ input.
 // ---------------------------------------------------------------------------
-// Measurement variant (build_variant with -DFMGPU_EXP_FUSED_LEVEL, never the shipped library): the
-// RF level meter's sums (k_siglevel below; signal_level.cpp:145-178) taken inside the FP32
-// decimator's tile fill, from the bytes the fill holds in registers anyway — SURVEY §8(f) row 2 as
-// worded. Every sample of the call is counted by exactly one tile (the one whose NEW samples it
-// belongs to); totals per channel accumulate in one fmgpu_level_sums each. In the shipped library
-// LevelAcc is empty and every call below compiles to nothing.
-#ifdef FMGPU_EXP_FUSED_LEVEL
-#define FMGPU_LVL_PARAM , fmgpu_level_sums *lvl
-#define FMGPU_LVL_ARG , expLevelBuf()
-struct LevelAcc {
-  uint32_t si = 0, sq = 0, sii = 0, sqq = 0, hard = 0, nearc = 0, cnt = 0;
-  __device__ __forceinline__ void word(uint32_t w) {  // two samples: bytes I0, Q0, I1, Q1
-    si = __dp4a(w, 0x00010001u, si);
-    sq = __dp4a(w, 0x01000100u, sq);
-    sii = __dp4a(w, w & 0x00ff00ffu, sii);
-    sqq = __dp4a(w, w & 0xff00ff00u, sqq);
-    const uint32_t t = ((w & 0x7f7f7f7fu) + 0x09090909u) ^ (w & 0x80808080u);
-    if ((t - 0x12121212u) & ~t & 0x80808080u) {
-      const uint32_t i0 = w & 0xffu, q0 = (w >> 8) & 0xffu, i1 = (w >> 16) & 0xffu, q1 = w >> 24;
-      hard += (i0 <= 1u || i0 >= 254u || q0 <= 1u || q0 >= 254u) ? 1u : 0u;
-      hard += (i1 <= 1u || i1 >= 254u || q1 <= 1u || q1 >= 254u) ? 1u : 0u;
-      nearc += (i0 <= 8u || i0 >= 247u || q0 <= 8u || q0 >= 247u) ? 1u : 0u;
-      nearc += (i1 <= 8u || i1 >= 247u || q1 <= 8u || q1 >= 247u) ? 1u : 0u;
-    }
-    cnt += 2;
-  }
-  __device__ __forceinline__ void one(uint32_t w16) {  // one sample: bytes I, Q
-    const uint32_t vi = w16 & 0xffu, vq = (w16 >> 8) & 0xffu;
-    si += vi;
-    sq += vq;
-    sii += vi * vi;
-    sqq += vq * vq;
-    hard += (vi <= 1u || vi >= 254u || vq <= 1u || vq >= 254u) ? 1u : 0u;
-    nearc += (vi <= 8u || vi >= 247u || vq <= 8u || vq >= 247u) ? 1u : 0u;
-    cnt++;
-  }
-  // a CTA sees (T + Pp) * M samples at most: every partial stays far below 2^32 across a warp
-  __device__ __forceinline__ void flush(fmgpu_level_sums *o) {
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      si += __shfl_down_sync(0xffffffffu, si, d);
-      sq += __shfl_down_sync(0xffffffffu, sq, d);
-      sii += __shfl_down_sync(0xffffffffu, sii, d);
-      sqq += __shfl_down_sync(0xffffffffu, sqq, d);
-      hard += __shfl_down_sync(0xffffffffu, hard, d);
-      nearc += __shfl_down_sync(0xffffffffu, nearc, d);
-      cnt += __shfl_down_sync(0xffffffffu, cnt, d);
-    }
-    if ((threadIdx.x & 31) == 0) {
-      atomicAdd(reinterpret_cast<unsigned long long *>(&o->sum_i), (unsigned long long)si);
-      atomicAdd(reinterpret_cast<unsigned long long *>(&o->sum_q), (unsigned long long)sq);
-      atomicAdd(reinterpret_cast<unsigned long long *>(&o->sum_ii), (unsigned long long)sii);
-      atomicAdd(reinterpret_cast<unsigned long long *>(&o->sum_qq), (unsigned long long)sqq);
-      atomicAdd(&o->hard_clip, hard);
-      atomicAdd(&o->near_clip, nearc);
-      atomicAdd(&o->n_samples, cnt);
-    }
-  }
-};
-#else
-#define FMGPU_LVL_PARAM
-#define FMGPU_LVL_ARG
-struct LevelAcc {
-  __device__ __forceinline__ void word(uint32_t) {}
-  __device__ __forceinline__ void one(uint32_t) {}
-};
-#endif
-
-#ifndef FMGPU_DECIM_NT
-#define FMGPU_DECIM_NT 128
-#endif
 // loads in flight per thread while the tile is filled (the fill is global-latency-bound)
-#ifndef FMGPU_DECIM_FILL_UNROLL
-#define FMGPU_DECIM_FILL_UNROLL 7
-#endif
-constexpr int DECIM_FILL_UNROLL = FMGPU_DECIM_FILL_UNROLL;
-constexpr int DECIM_NT = FMGPU_DECIM_NT;  // threads per decimator CTA (4 outputs each)
+constexpr int DECIM_FILL_UNROLL = 7;
+constexpr int DECIM_NT = 128;  // threads per decimator CTA (4 outputs each)
 
-template <int M, bool PACK>
+template <int M>
 __global__ void __launch_bounds__(DECIM_NT)
 k_decim(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restrict__ hist,
         const int *__restrict__ hist_valid, float2 *__restrict__ x1, size_t x1_pitch, int n_out,
-        int ch0, int Pp, float scale, const __grid_constant__ TapsParam taps FMGPU_LVL_PARAM) {
+        int ch0, int Pp, float scale, const __grid_constant__ TapsParam taps) {
   constexpr int R = 4;
   constexpr int T = DECIM_NT * R;
   constexpr int RM = R * M;
@@ -536,9 +452,6 @@ k_decim(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restr
     const int a_hist = (int)max(0L, min((long)tile_len, (long)H_IQ - v0));
     const unsigned short *p_hist = hist_c + v0;
     const unsigned short *p_in = in_c + (v0 - H_IQ);
-    // level sums (measurement variant only): this tile's NEW samples start at element a_own
-    [[maybe_unused]] LevelAcc lv;
-    [[maybe_unused]] const int a_own = max((Pp - 1) * M, a_hist);
     auto fill = [&](auto fast_tag) {
       constexpr bool FAST = decltype(fast_tag)::value;  // whole tile inside the input row
 #pragma unroll DECIM_FILL_UNROLL
@@ -557,9 +470,6 @@ k_decim(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restr
         if (!FAST && !ok) {
           f = make_float2(0.0f, 0.0f);
         }
-        if (ok && (int)a >= a_own) {
-          lv.one(w);
-        }
         xs[a + SK * (a / RM)] = f;
       }
     };
@@ -567,56 +477,18 @@ k_decim(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restr
       if (M % 2 == 0) {
         // even M: tile_len, RM and the skew are even, so elements (a, a + 1), a even, are one
         // 16-byte aligned pair in shared memory: two 16-bit loads, one 128-bit store per lane
-#ifdef FMGPU_EXP_FUSED_LEVEL
-        // measurement variant: the loads of DECIM_FILL_UNROLL iterations first (the clip counters'
-        // branch would otherwise keep the compiler from batching them: 3.46 instead of 2.01 ms per
-        // launch in the first form), then convert + store + level sums
-        constexpr int U = DECIM_FILL_UNROLL;
-        for (unsigned a0 = 2 * t; a0 < (unsigned)tile_len; a0 += 2 * DECIM_NT * U) {
-          uint32_t w0[U], w1[U];
-#pragma unroll
-          for (int u = 0; u < U; u++) {
-            const unsigned a = a0 + u * 2 * DECIM_NT;
-            const bool in = a < (unsigned)tile_len;
-            w0[u] = in ? (uint32_t)__ldg(p_in + a) : 0u;
-            w1[u] = in ? (uint32_t)__ldg(p_in + a + 1) : 0u;
-          }
-#pragma unroll
-          for (int u = 0; u < U; u++) {
-            const unsigned a = a0 + u * 2 * DECIM_NT;
-            if (a < (unsigned)tile_len) {
-              const float2 f0 = iqBytesToFloat(w0[u]);
-              const float2 f1 = iqBytesToFloat(w1[u]);
-              *reinterpret_cast<float4 *>(xs + a + SK * (a / RM)) = make_float4(f0.x, f0.y, f1.x, f1.y);
-              if ((int)a >= a_own) {  // a_own is even here: a pair is owned whole or not at all
-                lv.word(w0[u] | (w1[u] << 16));
-              }
-            }
-          }
-        }
-#else
 #pragma unroll DECIM_FILL_UNROLL
         for (unsigned a = 2 * t; a < (unsigned)tile_len; a += 2 * DECIM_NT) {
           const float2 f0 = iqBytesToFloat(__ldg(p_in + a));
           const float2 f1 = iqBytesToFloat(__ldg(p_in + a + 1));
           *reinterpret_cast<float4 *>(xs + a + SK * (a / RM)) = make_float4(f0.x, f0.y, f1.x, f1.y);
         }
-#endif
       } else {
         fill(std::true_type{});
       }
     } else {
       fill(std::false_type{});
     }
-#ifdef FMGPU_EXP_FUSED_LEVEL
-    // the last M - 1 samples of the call lie behind the newest sample of the last output
-    if (blockIdx.x == gridDim.x - 1) {
-      for (long s2 = o + tile_len + t; s2 < n_in; s2 += DECIM_NT) {
-        lv.one(in_c[s2]);
-      }
-    }
-    lv.flush(lvl + c);
-#endif
   }
   __syncthreads();
 
@@ -656,7 +528,7 @@ k_decim(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restr
         const float h = taps.h[(pp + ps) * M + r];
 #pragma unroll
         for (int j = 0; j < R; j++) {
-          acc[j] = fma2<PACK>(h, seg[(j + ps) & 3][r], acc[j]);
+          acc[j] = fma2(h, seg[(j + ps) & 3][r], acc[j]);
         }
       }
     }
@@ -918,7 +790,7 @@ k_dcblock_scan(const float2 *__restrict__ x1, size_t x1_pitch, float2 *__restric
         t.x = __shfl_up_sync(0xffffffffu, v[u].x, 1 << k);
         t.y = __shfl_up_sync(0xffffffffu, v[u].y, 1 << k);
         if (lane >= (1 << k)) {
-          v[u] = fma2<true>(pw[k], t, v[u]);
+          v[u] = fma2(pw[k], t, v[u]);
         }
       }
     }
@@ -926,7 +798,7 @@ k_dcblock_scan(const float2 *__restrict__ x1, size_t x1_pitch, float2 *__restric
     for (int u = 0; u < U; u++) {
       const int base = i0 + 32 * u;
       if (base < n_total) {   // warp-uniform
-        v[u] = fma2<true>(sl, carry, v[u]);   // v0[j] of the serial loop
+        v[u] = fma2(sl, carry, v[u]);   // v0[j] of the serial loop
         float2 p;
         p.x = __shfl_up_sync(0xffffffffu, v[u].x, 1);
         p.y = __shfl_up_sync(0xffffffffu, v[u].y, 1);
@@ -958,7 +830,6 @@ k_dcblock_scan(const float2 *__restrict__ x1, size_t x1_pitch, float2 *__restric
 // K2: channel filter (firfilt_crcf, 81/121 real taps on complex data, per-channel
 // bandwidth). 128 threads x 8 consecutive complex outputs, sliding register window.
 // ---------------------------------------------------------------------------
-template <bool PACK>
 __global__ void __launch_bounds__(128)
 k_chanfir(const float2 *__restrict__ x2, size_t x2_pitch, float2 *__restrict__ ybuf,
           size_t y_pitch, const float *__restrict__ chan_taps, const int *__restrict__ chan_lp,
@@ -999,7 +870,7 @@ k_chanfir(const float2 *__restrict__ x2, size_t x2_pitch, float2 *__restrict__ y
       const float h = hs[i + u];
 #pragma unroll
       for (int j = 0; j < R; j++) {
-        acc[j] = fma2<PACK>(h, win[(j + u) & (R - 1)], acc[j]);
+        acc[j] = fma2(h, win[(j + u) & (R - 1)], acc[j]);
       }
       win[u] = wp[u];
     }
@@ -1125,71 +996,6 @@ k_freqdem(const float2 *__restrict__ ybuf, size_t y_pitch, float *__restrict__ m
 }
 
 // ---------------------------------------------------------------------------
-// K3 / K5: real FIR with taps in the kernel-parameter constant bank
-// (pilot band-pass 305/325 taps; 2 x 121-tap 15 kHz low-pass via gridDim.z = 2)
-// ---------------------------------------------------------------------------
-template <int R>
-__global__ void __launch_bounds__(128)
-k_fir_real(FirRealJob job, const __grid_constant__ TapsParam taps) {
-  constexpr int T = 128 * R;
-  constexpr int SH = (R == 16) ? 4 : 3;  // one skew word per R samples: odd per-thread stride
-  extern __shared__ float fs_x[];
-  const int c = blockIdx.y + job.ch0;
-  const int z = blockIdx.z;
-  const int n0 = blockIdx.x * T;
-  const int t = threadIdx.x;
-  const int Lp = job.Lp;  // multiple of 8
-  const float *row = job.in[z] + (size_t)c * job.in_pitch + job.in_off;
-  const int b0 = n0 - (Lp - 1);
-  const int tile_len = T + Lp - 1 + R;
-  for (int a = t; a < tile_len; a += 128) {
-    const int s = b0 + a;
-    fs_x[a + (a >> SH)] = (s < job.n_total) ? row[s] : 0.0f;
-  }
-  __syncthreads();
-  float acc[R], win[R];
-#pragma unroll
-  for (int j = 0; j < R; j++) {
-    acc[j] = 0.0f;
-    const int a = t * R + j;
-    win[j] = fs_x[a + (a >> SH)];
-  }
-  int i = 0;
-  const float *wp = fs_x + (R + 1) * (t + 1);  // element t*R + i + u + R, see k_fir_pair
-  for (; i + R <= Lp; i += R) {
-#pragma unroll
-    for (int u = 0; u < R; u++) {
-      const float h = taps.h[i + u];
-#pragma unroll
-      for (int j = 0; j < R; j++) {
-        acc[j] = fmaf(h, win[(j + u) & (R - 1)], acc[j]);
-      }
-      win[u] = wp[u];
-    }
-    wp += R + 1;
-  }
-  if (R == 16 && i < Lp) {  // Lp is a multiple of 8: one half round left
-#pragma unroll
-    for (int u = 0; u < 8; u++) {
-      const float h = taps.h[i + u];
-#pragma unroll
-      for (int j = 0; j < R; j++) {
-        acc[j] = fmaf(h, win[(j + u) & (R - 1)], acc[j]);
-      }
-      win[u] = wp[u];
-    }
-  }
-  float *out = job.out[z] + (size_t)c * job.out_pitch + job.out_off;
-#pragma unroll
-  for (int j = 0; j < R; j++) {
-    const int n = n0 + t * R + j;
-    if (n < job.n_total) {
-      out[n] = acc[j] * job.scale;
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------
 // S4: 19 kHz pilot PLL, quality metrics, blend, L-R matrix, per-block lock logic
 // (stereo_decoder.cpp:92-286). One lane per channel, the per-sample work split over a
 // four-warp software pipeline, one tile of STEREO_ST samples apart (each warp on its own SM
@@ -1210,20 +1016,12 @@ constexpr int STEREO_TILES = 23;
 constexpr int STEREO_THREADS = 128;
 // channels per CTA of the two lane kernels (one lane each; lanes past it idle). These kernels are
 // bound by dependent-issue latency, not by lanes: fewer channels per warp = more chains per scheduler.
-#ifndef FMGPU_STEREO_CPC
-#define FMGPU_STEREO_CPC 32
-#endif
-#ifndef FMGPU_RDS_CPC
-#define FMGPU_RDS_CPC 32
-#endif
-constexpr int STEREO_CPC = FMGPU_STEREO_CPC;
-constexpr int RDS_CPC = FMGPU_RDS_CPC;
+constexpr int STEREO_CPC = 32;
+constexpr int RDS_CPC = 32;
 static_assert(STEREO_CPC >= 1 && STEREO_CPC <= 32 && RDS_CPC >= 1 && RDS_CPC <= 32, "one lane per channel");
-#ifndef FMGPU_STEREO_MINB
-#define FMGPU_STEREO_MINB 6  // at most 85 registers per thread
-#endif
+constexpr int STEREO_MINB = 6;  // at most 85 registers per thread
 
-__global__ void __launch_bounds__(STEREO_THREADS, FMGPU_STEREO_MINB)
+__global__ void __launch_bounds__(STEREO_THREADS, STEREO_MINB)
 k_stereo(const float *__restrict__ mpx, size_t mpx_pitch, const float *__restrict__ pilot,
          size_t pilot_pitch, float *__restrict__ lraw, float *__restrict__ rraw, size_t lr_pitch,
          StereoState *st, const ChanParams *cp, fmgpu_block_status *status, int status_pitch,
@@ -2673,60 +2471,19 @@ __global__ void k_pack_pcm16(const float *__restrict__ audio, size_t acap,
 // ---------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------
-// FMGPU_FFMA2=0 falls back to scalar FFMA in the FIR kernels (same results, for A/B timing)
-static bool usePackedFma() {
-  static int v = -1;
-  if (v < 0) {
-    const char *s = getenv("FMGPU_FFMA2");
-    v = (s && atoi(s) == 0) ? 0 : 1;
-  }
-  return v != 0;
-}
-
-#ifdef FMGPU_EXP_FUSED_LEVEL
-// measurement variant: per-channel totals of the fused level sums, read back by the check script
-constexpr int EXP_LEVEL_CH = 65536;
-static fmgpu_level_sums *expLevelBuf() {
-  static fmgpu_level_sums *buf = nullptr;
-  if (!buf) {
-    cudaMalloc(&buf, EXP_LEVEL_CH * sizeof(fmgpu_level_sums));
-    cudaMemset(buf, 0, EXP_LEVEL_CH * sizeof(fmgpu_level_sums));
-  }
-  return buf;
-}
-extern "C" int fmgpu_exp_fused_level_read(fmgpu_level_sums *out, int n_channels, int reset) {
-  if (n_channels > EXP_LEVEL_CH) {
-    return -1;
-  }
-  cudaDeviceSynchronize();
-  cudaMemcpy(out, expLevelBuf(), n_channels * sizeof(fmgpu_level_sums), cudaMemcpyDeviceToHost);
-  if (reset) {
-    cudaMemset(expLevelBuf(), 0, EXP_LEVEL_CH * sizeof(fmgpu_level_sums));
-  }
-  return cudaGetLastError() == cudaSuccess ? 0 : -2;
-}
-#endif
-
 #define FMGPU_DECIM_CASE(MM)                                                                     \
   case MM: {                                                                                     \
-    constexpr int T = 4 * DECIM_NT;                                                                     \
+    constexpr int T = 4 * DECIM_NT;                                                              \
     const int tile_len = (T + Pp - 1) * MM;                                                      \
     const size_t smem = (size_t)(tile_len + 2 * (tile_len / (4 * MM)) + 4) * sizeof(float2);     \
     static DeviceOnce attrs; /* per device: device_once.h */                                     \
     attrs.run([] {                                                                               \
-      cudaFuncSetAttribute(k_decim<MM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
-                           160 * 1024);                                                          \
-      return cudaFuncSetAttribute(k_decim<MM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+      return cudaFuncSetAttribute(k_decim<MM>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
                                   160 * 1024);                                                   \
     });                                                                                          \
     dim3 grid((n_out + T - 1) / T, nch);                                                         \
-    if (usePackedFma()) {                                                                        \
-      k_decim<MM, true><<<grid, DECIM_NT, smem, stream>>>(iq, iq_stride, hist, hist_valid, x1,        \
-                                                     x1_pitch, n_out, ch0, Pp, scale, taps FMGPU_LVL_ARG); \
-    } else {                                                                                     \
-      k_decim<MM, false><<<grid, DECIM_NT, smem, stream>>>(iq, iq_stride, hist, hist_valid, x1,       \
-                                                      x1_pitch, n_out, ch0, Pp, scale, taps FMGPU_LVL_ARG); \
-    }                                                                                            \
+    k_decim<MM><<<grid, DECIM_NT, smem, stream>>>(iq, iq_stride, hist, hist_valid, x1, x1_pitch, \
+                                                  n_out, ch0, Pp, scale, taps);                  \
     break;                                                                                       \
   }
 
@@ -2803,13 +2560,8 @@ void launchChanFir(const float2 *x2, size_t x2_pitch, float2 *ybuf, size_t y_pit
   const int tile_len = T + CHAN_TAPS_PITCH - 1 + 8;
   const size_t smem = (size_t)(tile_len + (tile_len >> 3) + 2) * sizeof(float2);
   dim3 grid((n_total + T - 1) / T, nch);
-  if (usePackedFma()) {
-    k_chanfir<true><<<grid, 128, smem, stream>>>(x2, x2_pitch, ybuf, y_pitch, chan_taps, chan_lp,
-                                                 chan_scale, cp, n_total, ch0);
-  } else {
-    k_chanfir<false><<<grid, 128, smem, stream>>>(x2, x2_pitch, ybuf, y_pitch, chan_taps, chan_lp,
-                                                  chan_scale, cp, n_total, ch0);
-  }
+  k_chanfir<<<grid, 128, smem, stream>>>(x2, x2_pitch, ybuf, y_pitch, chan_taps, chan_lp, chan_scale, cp,
+                                         n_total, ch0);
 }
 
 void launchAgc(float2 *ybuf, size_t y_pitch, DemodState *st, const ChanParams *cp, int n_total,
@@ -2826,12 +2578,13 @@ void launchFreqDem(const float2 *ybuf, size_t y_pitch, float *mpx, size_t mpx_pi
   k_freqdem<<<grid, 256, 0, stream>>>(ybuf, y_pitch, mpx, mpx_pitch, n_total, ch0, ref);
 }
 
-// K3 / K5, packed form: two real signals that share the taps ride in the two halves of FFMA2 —
-// the L and R rows of one channel (15 kHz low-pass), or the same row of two neighbouring
-// channels (pilot band-pass). The tile is interleaved into float2 {a, b} in shared memory; the
-// inner loop is the complex FIR's (8 outputs x 2 signals per thread, one LDS.64 and 8 FFMA2 per
-// tap, taps as uniform-register scalars). Each half is the same oldest-first fmaf chain as
-// k_fir_real: results are bit-identical.
+// K3 / K5: real FIR with taps in the kernel-parameter constant bank (pilot band-pass 305/325 taps;
+// 2 x 121-tap 15 kHz low-pass). Two real signals that share the taps ride in the two halves of
+// FFMA2 — the L and R rows of one channel (15 kHz low-pass), or the same row of two neighbouring
+// channels (pilot band-pass; with an odd channel count the last CTA computes one row, has_b =
+// false). The tile is interleaved into float2 {a, b} in shared memory; the inner loop is the
+// complex FIR's (8 outputs x 2 signals per thread, one LDS.64 and 8 FFMA2 per tap, taps as
+// uniform-register scalars). Each half is the oldest-first fmaf chain of a scalar FIR.
 __global__ void __launch_bounds__(128)
 k_fir_pair(FirRealJob job, int pair_channels, int nch, const __grid_constant__ TapsParam taps) {
   constexpr int R = 8;
@@ -2874,7 +2627,7 @@ k_fir_pair(FirRealJob job, int pair_channels, int nch, const __grid_constant__ T
       const float h = taps.h[i + u];
 #pragma unroll
       for (int j = 0; j < R; j++) {
-        acc[j] = fma2<true>(h, win[(j + u) & (R - 1)], acc[j]);
+        acc[j] = fma2(h, win[(j + u) & (R - 1)], acc[j]);
       }
       win[u] = wp[u];
     }
@@ -2894,37 +2647,14 @@ k_fir_pair(FirRealJob job, int pair_channels, int nch, const __grid_constant__ T
   }
 }
 
-int g_fir_r = -1;  // FMGPU_FIR_R=16 selects 16 outputs per thread (default 8; measured no faster)
-
 void launchFirReal(const FirRealJob &job, int nsig, int nch, const TapsParam &taps,
                    cudaStream_t stream) {
-  if (g_fir_r < 0) {
-    const char *v = getenv("FMGPU_FIR_R");
-    g_fir_r = (v && atoi(v) == 16) ? 16 : 8;
-  }
-  if (usePackedFma() && (nsig == 2 || nch >= 2)) {
-    constexpr int T = 1024;
-    const int tile_len = T + job.Lp - 1 + 8;
-    const size_t smem = (size_t)(tile_len + (tile_len >> 3) + 2) * sizeof(float2);
-    const int pair_channels = (nsig == 2) ? 0 : 1;
-    dim3 grid((job.n_total + T - 1) / T, pair_channels ? (nch + 1) / 2 : nch);
-    k_fir_pair<<<grid, 128, smem, stream>>>(job, pair_channels, nch, taps);
-    return;
-  }
-  // short inputs gain nothing from the wider tile
-  if (g_fir_r == 16 && job.n_total >= 2048) {
-    constexpr int T = 128 * 16;
-    const int tile_len = T + job.Lp - 1 + 16;
-    const size_t smem = (size_t)(tile_len + (tile_len >> 4) + 2) * sizeof(float);
-    dim3 grid((job.n_total + T - 1) / T, nch, nsig);
-    k_fir_real<16><<<grid, 128, smem, stream>>>(job, taps);
-    return;
-  }
   constexpr int T = 1024;
   const int tile_len = T + job.Lp - 1 + 8;
-  const size_t smem = (size_t)(tile_len + (tile_len >> 3) + 2) * sizeof(float);
-  dim3 grid((job.n_total + T - 1) / T, nch, nsig);
-  k_fir_real<8><<<grid, 128, smem, stream>>>(job, taps);
+  const size_t smem = (size_t)(tile_len + (tile_len >> 3) + 2) * sizeof(float2);
+  const int pair_channels = (nsig == 2) ? 0 : 1;
+  dim3 grid((job.n_total + T - 1) / T, pair_channels ? (nch + 1) / 2 : nch);
+  k_fir_pair<<<grid, 128, smem, stream>>>(job, pair_channels, nch, taps);
 }
 
 void launchStereo(const float *mpx, size_t mpx_pitch, const float *pilot, size_t pilot_pitch,

@@ -220,38 +220,6 @@ def test_clipping_statistics(orc_fm):
     eng.close()
 
 
-@pytest.mark.parametrize("rate", ["240k", "256k"])
-def test_eight_output_decimator_variant_bit_exact(rate):
-    """k_decim8 (eight outputs per thread, the second four running four tap segments behind the
-    first four; opt-in through FMGPU_DECIM8=1, read once per process) must produce the decimated IQ of
-    the default decimator, i.e. of the oracle: run it in a child process."""
-    import os
-    import subprocess
-    import sys
-
-    code = f"""
-import numpy as np
-import fmtuner_sdr_b200 as fm
-from oracle import orc
-from tests.common import rates, run_engine_chunks
-iq_rate, decim = rates({rate!r})
-nblk = 6
-iq = orc.config1_signal(fs_iq=iq_rate).generate(nblk * 8192 * decim)
-kw = dict(iq_rate=iq_rate, decimation=decim)
-ref = orc.Channel(orc.OracleLib("fm"), orc.make_config(**kw)).process(iq, debug=True)
-eng = fm.Engine(fm.make_config(max_blocks=3, **kw), 1, 0)
-audio, groups, status, dbg = run_engine_chunks(eng, iq.reshape(1, -1), nblk, 3, debug_channel=0)
-assert np.array_equal(dbg["dec"].view(np.float32), ref.dec.view(np.float32))
-assert np.array_equal(audio[0][0], ref.left) and np.array_equal(audio[0][1], ref.right)
-print("decim8 ok")
-"""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, FMGPU_DECIM8="1", PYTHONPATH=root)
-    r = subprocess.run([sys.executable, "-c", code], env=env, cwd=root, capture_output=True,
-                       text=True, timeout=600)
-    assert r.returncode == 0 and "decim8 ok" in r.stdout, r.stdout + r.stderr
-
-
 def test_one_channel_reset_leaves_the_lanes_out_of_step(orc_fm):
     """Retune of ONE channel of a batch (dspRuntime.reset + rdsReset, main.cpp:1028-1062) while its
     neighbours keep going: afterwards the lanes of a warp sit at different /24 decimation phases,
