@@ -27,10 +27,6 @@ std::string g_create_error;
 
 size_t roundUp(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
-struct StageTimer {
-  std::vector<std::pair<const char *, std::pair<cudaEvent_t, cudaEvent_t>>> spans;
-};
-
 }  // namespace
 
 struct fmgpu_engine {
@@ -111,7 +107,6 @@ struct fmgpu_engine {
   uint32_t *dNAudio = nullptr, *dNGroups = nullptr;
   uint8_t *dBits = nullptr;
   unsigned long long *dWords = nullptr;
-  uint32_t *dBitEnd = nullptr;
   size_t x2Pitch = 0, yPitch = 0, mpxPitch = 0, lrPitch = 0, lfPitch = 0;
   cudaStream_t stream = nullptr;  // stage-level (single-channel) entry points, resets, reads
 
@@ -391,7 +386,7 @@ int fillStateField(fmgpu_engine *e, S *base, size_t fieldOffset, const void *val
 }
 
 // ---------------------------------------------------------------------------
-// pipeline stages on channels [ch0, ch0 + nch)
+// pipeline stages: one logical block of channels [ch0, ch0 + nch) on stream s
 // ---------------------------------------------------------------------------
 // the decimating FIR of n_out outputs per channel into x1 (history in dHistIq), either flavour
 void runDecim(fmgpu_engine *e, const uint8_t *iq, size_t stride, float2 *x1, int n_out, int ch0,
@@ -425,146 +420,36 @@ void runFirReal(fmgpu_engine *e, const FirRealJob &j, int nsig, int nch, const T
   launchFirReal(j, nsig, nch, taps, s);
 }
 
-void stageDecimate(fmgpu_engine *e, const uint8_t *iq, size_t stride, int n_out, int ch0, int nch,
-                   cudaStream_t s) {
-  Span sp(e, "decimate", s);
-  if (e->M == 1) {
-    launchConvertU8(iq, stride, e->dX1, e->pitch, n_out, ch0, nch, s);
-    e->launches += 1;
-    return;
-  }
-  runDecim(e, iq, stride, e->dX1, n_out, ch0, nch, s);
-  launchCarryIq(e->dHistIq, e->dHistValid, iq, stride, static_cast<long>(n_out) * e->M, ch0, nch, s);
-  e->launches += 2;
+// Measurement variant (build_variant with -DFMGPU_EXP_SKIP, never the shipped library): leave the
+// main kernel of the stages named in FMGPU_SKIP out of the block pipeline, to see what each one
+// costs the step beside the others. Results are WRONG with any stage skipped.
+#ifdef FMGPU_EXP_SKIP
+static bool expSkip(const char *name) {
+  static const std::string v = getenv("FMGPU_SKIP") ? getenv("FMGPU_SKIP") : "";
+  return v.find(name) != std::string::npos;
 }
+#else
+constexpr bool expSkip(const char *) { return false; }
+#endif
 
-// Lane kernels (one warp per 32 channels, latency-bound) go to a HIGH-PRIORITY stream so that
-// their few CTAs are scheduled ahead of the thousands of queued CTAs of other groups' FIR
-// kernels; `hop` chains the two streams with an event. lane == s means: no split.
-static void hop(cudaStream_t from, cudaStream_t to, cudaEvent_t ev) {
-  if (from != to) {
-    cudaEventRecord(ev, from);
-    cudaStreamWaitEvent(to, ev, 0);
-  }
-}
+struct BatchOut {
+  float *audio = nullptr;  // [C][2][acap]
+  size_t acap = 0;
+  uint32_t *nAudio = nullptr;
+  fmgpu_rds_group *groups = nullptr;
+  uint32_t gcap = 0;
+  uint32_t *nGroups = nullptr;
+  fmgpu_block_status *status = nullptr;  // [C][n_blocks]
+};
 
-// x1 (or raw u8) -> mpx
-void stageDemod(fmgpu_engine *e, const uint8_t *iq_u8, size_t stride, fmgpu_block_status *status,
-                int nblk, int blk_len, int n, int ch0, int nch, cudaStream_t s,
-                cudaStream_t lane = nullptr, cudaEvent_t ev = nullptr) {
-  if (!lane) {
-    lane = s;
-  }
-  {
-    hop(s, lane, ev);
-    Span sp(e, "dcblock", lane);
-    launchDcBlock(iq_u8 ? nullptr : e->dX1, e->pitch, iq_u8, stride, e->dX2, e->x2Pitch, e->dDemod,
-                  status, nblk, nblk, blk_len, n, ch0, nch, e->k.dc_a1_iq, lane);
-  }
-  hop(lane, s, ev);
-  {
-    Span sp(e, "chanfir", s);
-    launchChanFir(e->dX2, e->x2Pitch, e->dY, e->yPitch, e->dChanTaps, e->dChanLp, e->dChanScale,
-                  e->dParams, n, ch0, nch, s);
-  }
-  bool anyAgc = false;
-  for (int c = ch0; c < ch0 + nch; c++) {
-    anyAgc = anyAgc || e->hParams[c].agc_mode != 0;
-  }
-  if (anyAgc) {
-    hop(s, lane, ev);
-    {
-      Span sp(e, "agc", lane);
-      launchAgc(e->dY, e->yPitch, e->dDemod, e->dParams, n, ch0, nch, lane);
-    }
-    hop(lane, s, ev);
-    e->launches += 1;
-  }
-  {
-    Span sp(e, "freqdem", s);
-    launchFreqDem(e->dY, e->yPitch, e->dMpx, e->mpxPitch, n, ch0, nch, e->k.fd_ref, s);
-    launchCarryF2(e->dY, e->yPitch, Y_OFF, n, ch0, nch, s);  // slot Y_OFF-1 <- last output
-    launchCarryF2(e->dX2, e->x2Pitch, H_X2, n, ch0, nch, s);
-  }
-  e->launches += 5;
-}
-
-// mpx -> lf/rf (DSP-rate stereo) ; carries the stereo decoder's halos
-void stageStereo(fmgpu_engine *e, fmgpu_block_status *status, int nblk, int blk_len, int n, int ch0,
-                 int nch, cudaStream_t s, cudaStream_t lane = nullptr, cudaEvent_t ev = nullptr) {
-  if (!lane) {
-    lane = s;
-  }
-  {
-    Span sp(e, "pilot_fir", s);
-    FirRealJob j{};
-    j.in[0] = e->dMpx;
-    j.out[0] = e->dPilot;
-    j.in_pitch = e->mpxPitch;
-    j.out_pitch = e->pitch;
-    j.in_off = H_MPX;
-    j.out_off = 0;
-    j.n_total = n;
-    j.Lp = e->pilLp;
-    j.scale = 1.0f;
-    j.ch0 = ch0;
-    runFirReal(e, j, 1, nch, e->pilParam, e->pilTcOk, e->pilTc, e->dPilB, 22, s);
-  }
-  hop(s, lane, ev);
-  {
-    Span sp(e, "stereo_pll", lane);
-    launchStereo(e->dMpx, e->mpxPitch, e->dPilot, e->pitch, e->dLraw, e->dRraw, e->lrPitch,
-                 e->dStereo, e->dParams, status, nblk, nblk, blk_len, n, ch0, nch, e->k, lane);
-  }
-  hop(lane, s, ev);
-  {
-    Span sp(e, "audio_lpf", s);
-    FirRealJob j{};
-    j.in[0] = e->dLraw;
-    j.in[1] = e->dRraw;
-    j.out[0] = e->dLf;
-    j.out[1] = e->dRf;
-    j.in_pitch = e->lrPitch;
-    j.out_pitch = e->lfPitch;
-    j.in_off = H_LR;
-    j.out_off = H_LF;
-    j.n_total = n;
-    j.Lp = e->audLp;
-    j.scale = e->k.aud_scale;
-    j.ch0 = ch0;
-    runFirReal(e, j, 2, nch, e->audParam, e->audTcOk, e->audTc, e->dAudB, 20, s);
-    launchCarryF32(e->dLraw, e->lrPitch, H_LR, n, ch0, nch, s);
-    launchCarryF32(e->dRraw, e->lrPitch, H_LR, n, ch0, nch, s);
-    launchCarryF32(e->dMpx, e->mpxPitch, H_MPX, n, ch0, nch, s);
-  }
-  e->launches += 6;
-}
-
-// lf/rf -> audio rows (resample + de-emphasis + DC block [+ clamp])
-void stageAfPost(fmgpu_engine *e, int n, int clamp, int ch0, int nch, cudaStream_t s) {
-  Span sp(e, "afpost", s);
-  const int maxOut = static_cast<int>(std::min<size_t>(
-      e->acap, static_cast<size_t>((static_cast<double>(n) * 16777216.0) / e->k.aud_step) + 2));
-  launchResample(e->dLf, e->dRf, e->lfPitch, H_LF, nullptr, 0, e->dAudio, e->acap, e->dAudBank,
-                 AUD_RS_LEN, e->k.aud_step, e->dAudioSt, 0, maxOut, ch0, nch, s);
-  launchAudioIir(e->dAudio, e->acap, e->dAudioSt, e->dParams, ch0, nch, e->k.dc_a1_af, 0, clamp, 0,
-                 s);
-  launchCarryF32(e->dLf, e->lfPitch, H_LF, n, ch0, nch, s);
-  launchCarryF32(e->dRf, e->lfPitch, H_LF, n, ch0, nch, s);
-  e->launches += 4;
-}
-
-// FMDemod mono chain: mpx -> audio row 0 (fm_demod.cpp:210-226)
-void stageMono(fmgpu_engine *e, int n, int clamp, int dup, int ch0, int nch, cudaStream_t s) {
-  Span sp(e, "mono", s);
-  const int maxOut = static_cast<int>(std::min<size_t>(
-      e->acap, static_cast<size_t>((static_cast<double>(n) * 16777216.0) / e->k.aud_step) + 2));
-  launchResample(e->dMpx, nullptr, e->mpxPitch, H_MPX, e->dMonoHist, 32, e->dAudio, e->acap,
-                 e->dAudBank, AUD_RS_LEN, e->k.aud_step, e->dAudioSt, 1, maxOut, ch0, nch, s);
-  launchAudioIir(e->dAudio, e->acap, e->dAudioSt, e->dParams, ch0, nch, e->k.mono_dc_a1, 1, clamp,
-                 dup, s);
-  launchSaveTail(e->dMpx, e->mpxPitch, H_MPX, e->dMonoHist, 32, AUD_RS_LEN - 1, n, ch0, nch, s);
-  e->launches += 3;
+// the engine's own result buffers (the stage-level entry points copy from them)
+BatchOut engineOut(const fmgpu_engine *e) {
+  BatchOut out;
+  out.audio = e->dAudio;
+  out.acap = e->acap;
+  out.groups = e->dGroups;
+  out.gcap = static_cast<uint32_t>(e->gcap);
+  return out;
 }
 
 // upper bound of the 171 kHz samples n DSP-rate inputs produce (any resampler phase)
@@ -572,18 +457,282 @@ int max171(const fmgpu_engine *e, int n) {
   return static_cast<int>((static_cast<unsigned long long>(n) << 24) / e->k.rds_step) + 2;
 }
 
-void stageRds(fmgpu_engine *e, fmgpu_rds_group *groups, uint32_t gcap, fmgpu_block_status *status,
-              int nblk, int blk_len, int n, int ch0, int nch, cudaStream_t s) {
-  Span sp(e, "rds", s);
-  (void)blk_len;
-  launchRds(e->dMpx, e->mpxPitch, e->dRdsHist, 32, e->dRds, e->dRing, e->dRdsBank, e->dRdsLpf,
-            e->dMf, e->dDmf, e->dR171, e->r171Pitch, max171(e, n), e->dBits,
-            static_cast<uint32_t>(e->bitsCap), e->dBitEnd, ch0, nch, e->k, RdsRsRef{e->dRdsRs, 0}, s);
-  launchBlockSync(e->dBits, static_cast<uint32_t>(e->bitsCap), e->dBitEnd, e->dRds, e->dWords, groups,
-                  gcap, status, nblk, nblk, 0, ch0, nch, s);
-  e->launches += 1;
-  launchSaveTail(e->dMpx, e->mpxPitch, H_MPX, e->dRdsHist, 32, RDS_HIST, n, ch0, nch, s);
+// the 171 kHz rows of block parity par
+float *r171Rows(const fmgpu_engine *e, int par) {
+  return e->dR171 + static_cast<size_t>(par) * static_cast<size_t>(e->C) * e->r171Pitch;
+}
+
+bool anyAgc(const fmgpu_engine *e, int ch0, int nch) {
+  for (int c = ch0; c < ch0 + nch; c++) {
+    if (e->hParams[c].agc_mode != 0) {
+      return true;
+    }
+  }
+  return false;
+}
+
+// Ring buffers whose rows begin with a FIR / delay halo: the samples the next block's stage reads in
+// front of its own.
+enum Halo : unsigned { HALO_X2 = 1, HALO_Y = 2, HALO_MPX = 4, HALO_LR = 8, HALO_LF = 16 };
+
+// Copy the halo of every buffer in `which` from the samples just before position pos of the row (the
+// end of the last block written) to the front of the row, for channels [ch0, ch0 + nch).
+void carryHalos(fmgpu_engine *e, unsigned which, size_t pos, int ch0, int nch, cudaStream_t s) {
+  if (which & HALO_X2) {
+    launchCarryF2(e->dX2, e->x2Pitch, H_X2, pos, ch0, nch, s);
+    e->launches += 1;
+  }
+  if (which & HALO_Y) {
+    launchCarryF2(e->dY, e->yPitch, Y_OFF, pos, ch0, nch, s);  // slot Y_OFF-1 <- last output
+    e->launches += 1;
+  }
+  if (which & HALO_MPX) {
+    launchCarryF32(e->dMpx, e->mpxPitch, H_MPX, pos, ch0, nch, s);
+    e->launches += 1;
+  }
+  if (which & HALO_LR) {
+    launchCarryF32(e->dLraw, e->lrPitch, H_LR, pos, ch0, nch, s);
+    launchCarryF32(e->dRraw, e->lrPitch, H_LR, pos, ch0, nch, s);
+    e->launches += 2;
+  }
+  if (which & HALO_LF) {
+    launchCarryF32(e->dLf, e->lfPitch, H_LF, pos, ch0, nch, s);
+    launchCarryF32(e->dRf, e->lfPitch, H_LF, pos, ch0, nch, s);
+    e->launches += 2;
+  }
+}
+
+// One logical block for the stage functions below. The block pipeline (launchBlock) queues them on the
+// stage streams; the stage-level entry points call them on the engine's stream with t0 = 0 and carry
+// their halos themselves after the call.
+struct BlockRef {
+  int ch0, nch;
+  size_t t0;  // the block's offset in every ring buffer
+  int n;      // samples
+  fmgpu_block_status *status;  // the block's entry in channel 0's status row (nullptr: none)
+  int statusPitch;
+  bool carry;  // ring slot 0: bring the tail of the last slot in front of it first
+};
+
+BlockRef stageBlock(int channel, int n) { return BlockRef{channel, 1, 0, n, nullptr, 1, false}; }
+
+size_t ringEnd(const fmgpu_engine *e) { return static_cast<size_t>(e->K) * e->N; }
+
+// IQ bytes -> x1: the decimating FIR (M == 1: the conversion to float alone)
+void stageDecimate(fmgpu_engine *e, const BlockRef &k, const uint8_t *iq, size_t stride, cudaStream_t s) {
+  Span sp(e, "decimate", s);
+  if (e->M == 1) {
+    launchConvertU8(iq, stride, e->dX1 + k.t0, e->pitch, k.n, k.ch0, k.nch, s);
+    e->launches += 1;
+    return;
+  }
+  if (!expSkip("decimate")) runDecim(e, iq, stride, e->dX1 + k.t0, k.n, k.ch0, k.nch, s);
+  launchCarryIq(e->dHistIq, e->dHistValid, iq, stride, static_cast<long>(k.n) * e->M, k.ch0, k.nch, s);
   e->launches += 2;
+}
+
+// I/Q DC blockers: complex float rows x (else the IQ bytes iq at the DSP rate) -> x2. scan: the
+// warp-shuffle form (float input only; fast arithmetic)
+void stageDcBlock(fmgpu_engine *e, const BlockRef &k, const float2 *x, size_t xPitch, const uint8_t *iq,
+                  size_t iqStride, bool scan, cudaStream_t s) {
+  Span sp(e, "dcblock", s);
+  if (k.carry) {
+    carryHalos(e, HALO_X2, ringEnd(e), k.ch0, k.nch, s);
+  }
+  if (scan) {
+    if (!expSkip("dcblock")) launchDcBlockScan(x, xPitch, e->dX2 + k.t0, e->x2Pitch, e->dDemod, k.status,
+                                               k.statusPitch, k.n, k.ch0, k.nch, e->k.dc_a1_iq, s);
+  } else {
+    launchDcBlock(x, xPitch, iq, iqStride, e->dX2 + k.t0, e->x2Pitch, e->dDemod, k.status, k.statusPitch,
+                  k.n, k.ch0, k.nch, e->k.dc_a1_iq, s);
+  }
+  e->launches += 1;
+}
+
+// channel filter + discriminator as one tensor-core kernel, every channel on filter filt: x2 -> MPX (and
+// the discriminator's carried sample into the y row). False: refused before anything was launched
+// (alignment, pitch).
+bool stageChanDemod(fmgpu_engine *e, const BlockRef &k, int filt, cudaStream_t s) {
+  Span sp(e, "chan_demod", s);
+  if (k.carry) {
+    carryHalos(e, HALO_Y | HALO_MPX, ringEnd(e), k.ch0, k.nch, s);
+  }
+  const auto &f = e->filters[filt];
+  const cudaError_t err = expSkip("chan_demod") ? cudaSuccess :
+      launchChanDemodTc(e->dX2 + k.t0, e->x2Pitch, H_X2, e->dY + k.t0, e->yPitch, e->dMpx + k.t0, e->mpxPitch,
+                        H_MPX, k.n, k.ch0, k.nch, f.scale, e->k.fd_ref, f.tc, f.dB, 21, e->smCount, s);
+  e->launches += 1;
+  if (err != cudaSuccess) {
+    e->lastError = std::string("tensor-core channel filter + discriminator: ") + cudaGetErrorString(err);
+    return false;
+  }
+  return true;
+}
+
+// x2 -> y
+void stageChanFir(fmgpu_engine *e, const BlockRef &k, cudaStream_t s) {
+  Span sp(e, "chanfir", s);
+  launchChanFir(e->dX2 + k.t0, e->x2Pitch, e->dY + k.t0, e->yPitch, e->dChanTaps, e->dChanLp, e->dChanScale,
+                e->dParams, k.n, k.ch0, k.nch, s);
+  e->launches += 1;
+}
+
+// y in place
+void stageAgc(fmgpu_engine *e, const BlockRef &k, cudaStream_t s) {
+  // (running the discriminator inside this lane kernel was tried: its two IEEE divisions per
+  // sample do not hide behind the AGC recursion, the stage took 5.6 ms instead of 2.7 + 0.7)
+  Span sp(e, "agc", s);
+  launchAgc(e->dY + k.t0, e->yPitch, e->dDemod, e->dParams, k.n, k.ch0, k.nch, s);
+  e->launches += 1;
+}
+
+// y -> MPX
+void stageFreqDem(fmgpu_engine *e, const BlockRef &k, cudaStream_t s) {
+  Span sp(e, "freqdem", s);
+  if (k.carry) {
+    carryHalos(e, HALO_Y | HALO_MPX, ringEnd(e), k.ch0, k.nch, s);
+  }
+  launchFreqDem(e->dY + k.t0, e->yPitch, e->dMpx + k.t0, e->mpxPitch, k.n, k.ch0, k.nch, e->k.fd_ref, s);
+  e->launches += 1;
+}
+
+// MPX -> 171 kHz rows of parity par (tile kernel; the RDS demodulator of the previous block may run
+// beside it on the other parity's rows)
+void stageRdsResample(fmgpu_engine *e, const BlockRef &k, int par, cudaStream_t s) {
+  const RdsRsRef rr{e->dRdsRs, par};
+  Span sp(e, "rds_resample", s);
+  launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, k.n, k.ch0, k.nch, e->k.aud_step, e->k.rds_step, 0, 0,
+                PREPARE_RDS_RESAMPLER, 0, rr, s);
+  if (!expSkip("rds_resample")) launchRdsResample(e->dMpx + k.t0, e->mpxPitch, e->dRdsHist, 32, rr, e->dRdsBank,
+                                                  r171Rows(e, par), e->r171Pitch, max171(e, k.n), k.ch0, k.nch,
+                                                  e->k, s);
+  launchSaveTail(e->dMpx + k.t0, e->mpxPitch, H_MPX, e->dRdsHist, 32, RDS_HIST, k.n, k.ch0, k.nch, s);
+  launchCommit(e->dAudioSt, e->dRds, k.ch0, k.nch, 0, 0, 1, rr, s);
+  e->launches += 4;
+}
+
+// 171 kHz rows of parity par -> bits -> groups into out.groups, tagged with block number b. first: the
+// call's first block (its counters start at zero); last: store the call's group counts to out.nGroups.
+void stageRdsDemod(fmgpu_engine *e, const BlockRef &k, int par, const BatchOut &out, int b, bool first,
+                   bool last, cudaStream_t s) {
+  const RdsRsRef rr{e->dRdsRs, par};
+  {
+    Span sp(e, "rds", s);  // lane kernel: 57 kHz mix ... bits
+    if (first) {
+      launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, k.n, k.ch0, k.nch, e->k.aud_step, e->k.rds_step, 0, 0,
+                    PREPARE_RDS_COUNTERS, 1, rr, s);
+      e->launches += 1;
+    }
+    if (!expSkip("rds_demod")) launchRdsDemod(e->dRds, e->dRing, e->dRdsLpf, e->dMf, e->dDmf, r171Rows(e, par),
+                                              e->r171Pitch, e->dBits, static_cast<uint32_t>(e->bitsCap), k.ch0,
+                                              k.nch, e->k, rr, s);
+  }
+  e->launches += 1;
+  {
+    Span sp(e, "rds_sync", s);  // syndromes at every bit offset + block sync state machine
+    if (!expSkip("rds_sync")) launchBlockSync(e->dBits, static_cast<uint32_t>(e->bitsCap), e->dRds, e->dWords,
+                                              out.groups, out.gcap, k.status, k.statusPitch, b, k.ch0, k.nch, s);
+    if (last) {
+      // the call's group counts, from the stream that owns RdsState::n_groups: the next call's
+      // first k_prepare on this stream zeroes it again
+      launchStoreCounts(e->dAudioSt, e->dRds, nullptr, out.nGroups, k.ch0, k.nch, e->cfg.stereo ? 0 : 1,
+                        static_cast<uint32_t>(out.acap), out.gcap, s);
+      e->launches += 1;
+    }
+  }
+  e->launches += 1;
+}
+
+// MPX -> pilot (band-pass)
+void stagePilot(fmgpu_engine *e, const BlockRef &k, cudaStream_t s) {
+  Span sp(e, "pilot_fir", s);
+  FirRealJob j{};
+  j.in[0] = e->dMpx + k.t0;
+  j.out[0] = e->dPilot + k.t0;
+  j.in_pitch = e->mpxPitch;
+  j.out_pitch = e->pitch;
+  j.in_off = H_MPX;
+  j.out_off = 0;
+  j.n_total = k.n;
+  j.Lp = e->pilLp;
+  j.scale = 1.0f;
+  j.ch0 = k.ch0;
+  if (!expSkip("pilot_fir")) runFirReal(e, j, 1, k.nch, e->pilParam, e->pilTcOk, e->pilTc, e->dPilB, 22, s);
+  e->launches += 1;
+}
+
+// MPX + pilot -> L/R before the low-pass (PLL, blend, matrix)
+void stageStereo(fmgpu_engine *e, const BlockRef &k, cudaStream_t s) {
+  Span sp(e, "stereo_pll", s);
+  if (k.carry) {
+    carryHalos(e, HALO_LR, ringEnd(e), k.ch0, k.nch, s);
+  }
+  if (!expSkip("stereo_pll")) launchStereo(e->dMpx + k.t0, e->mpxPitch, e->dPilot + k.t0, e->pitch,
+                                           e->dLraw + k.t0, e->dRraw + k.t0, e->lrPitch, e->dStereo, e->dParams,
+                                           k.status, k.statusPitch, k.n, k.ch0, k.nch, e->k, s);
+  e->launches += 1;
+}
+
+// L/R -> 15 kHz low-pass
+void stageLpf(fmgpu_engine *e, const BlockRef &k, cudaStream_t s) {
+  Span sp(e, "audio_lpf", s);
+  if (k.carry) {
+    carryHalos(e, HALO_LF, ringEnd(e), k.ch0, k.nch, s);
+  }
+  FirRealJob j{};
+  j.in[0] = e->dLraw + k.t0;
+  j.in[1] = e->dRraw + k.t0;
+  j.out[0] = e->dLf + k.t0;
+  j.out[1] = e->dRf + k.t0;
+  j.in_pitch = e->lrPitch;
+  j.out_pitch = e->lfPitch;
+  j.in_off = H_LR;
+  j.out_off = H_LF;
+  j.n_total = k.n;
+  j.Lp = e->audLp;
+  j.scale = e->k.aud_scale;
+  j.ch0 = k.ch0;
+  if (!expSkip("audio_lpf")) runFirReal(e, j, 2, k.nch, e->audParam, e->audTcOk, e->audTc, e->dAudB, 20, s);
+  e->launches += 1;
+}
+
+int maxAudioOut(const fmgpu_engine *e, const BatchOut &out, int n) {
+  return static_cast<int>(std::min<size_t>(
+      out.acap, static_cast<size_t>((static_cast<double>(n) * 16777216.0) / e->k.aud_step) + 2));
+}
+
+// low-passed L/R -> out.audio rows (resample, de-emphasis, DC block; clamp: to +-1). first: the call's
+// first block (frames start at the row start); scan: the de-emphasis + DC blocker as a warp-shuffle scan
+void stageAfPost(fmgpu_engine *e, const BlockRef &k, const BatchOut &out, bool first, bool scan, int clamp,
+                 cudaStream_t s) {
+  Span sp(e, "afpost", s);
+  launchPrepare(e->dAudioSt, e->dRds, k.status, k.statusPitch, k.n, k.ch0, k.nch, e->k.aud_step,
+                e->k.rds_step, 1, 0, PREPARE_RDS_NONE, first ? 1 : 0, RdsRsRef{e->dRdsRs, 0}, s);
+  if (!expSkip("afpost")) launchResample(e->dLf + k.t0, e->dRf + k.t0, e->lfPitch, H_LF, nullptr, 0, out.audio,
+                                         out.acap, e->dAudBank, e->k.aud_step, e->dAudioSt, 0,
+                                         maxAudioOut(e, out, k.n), k.ch0, k.nch, s);
+  if (scan) {
+    launchAudioIirScan(out.audio, out.acap, e->dAudioSt, e->dParams, k.ch0, k.nch, e->k.dc_a1_af, clamp, s);
+  } else {
+    launchAudioIir(out.audio, out.acap, e->dAudioSt, e->dParams, k.ch0, k.nch, e->k.dc_a1_af, 0, clamp, 0, s);
+  }
+  launchCommit(e->dAudioSt, e->dRds, k.ch0, k.nch, 1, 0, 0, RdsRsRef{e->dRdsRs, 0}, s);
+  e->launches += 4;
+}
+
+// FMDemod mono chain (fm_demod.cpp:210-226, main.cpp:1267-1279): MPX -> resample -> de-emphasis -> DC
+// block into audio row 0; dup: x0.5 to both rows
+void stageMono(fmgpu_engine *e, const BlockRef &k, const BatchOut &out, bool first, int clamp, int dup,
+               cudaStream_t s) {
+  Span sp(e, "mono", s);
+  launchPrepare(e->dAudioSt, e->dRds, k.status, k.statusPitch, k.n, k.ch0, k.nch, e->k.aud_step,
+                e->k.rds_step, 0, 1, PREPARE_RDS_NONE, first ? 1 : 0, RdsRsRef{e->dRdsRs, 0}, s);
+  launchResample(e->dMpx + k.t0, nullptr, e->mpxPitch, H_MPX, e->dMonoHist, 32, out.audio, out.acap, e->dAudBank,
+                 e->k.aud_step, e->dAudioSt, 1, maxAudioOut(e, out, k.n), k.ch0, k.nch, s);
+  launchAudioIir(out.audio, out.acap, e->dAudioSt, e->dParams, k.ch0, k.nch, e->k.mono_dc_a1, 1, clamp, dup, s);
+  launchSaveTail(e->dMpx + k.t0, e->mpxPitch, H_MPX, e->dMonoHist, 32, AUD_RS_LEN - 1, k.n, k.ch0, k.nch, s);
+  launchCommit(e->dAudioSt, e->dRds, k.ch0, k.nch, 0, 1, 0, RdsRsRef{e->dRdsRs, 0}, s);
+  e->launches += 5;
 }
 
 void collectTimes(fmgpu_engine *e) {
@@ -615,16 +764,6 @@ void collectTimes(fmgpu_engine *e) {
 // ---------------------------------------------------------------------------
 // block pipeline (see fmgpu_engine::Pipe)
 // ---------------------------------------------------------------------------
-struct BatchOut {
-  float *audio = nullptr;  // [C][2][acap]
-  size_t acap = 0;
-  uint32_t *nAudio = nullptr;
-  fmgpu_rds_group *groups = nullptr;
-  uint32_t gcap = 0;
-  uint32_t *nGroups = nullptr;
-  fmgpu_block_status *status = nullptr;  // [C][n_blocks]
-};
-
 // channel range of pipeline group g (multiples of 32 channels: one warp of lane kernels)
 void groupRange(const fmgpu_engine *e, int g, int *ch0, int *nch) {
   const int per = static_cast<int>(roundUp((e->C + e->nGroups - 1) / e->nGroups, 32));
@@ -656,31 +795,11 @@ void realign(fmgpu_engine *e) {
     return;
   }
   const size_t pos = static_cast<size_t>(slot == 0 ? e->K : slot) * e->N;  // end of the last block
-  cudaStream_t s = e->stream;
-  launchCarryF2(e->dX2, e->x2Pitch, H_X2, pos, 0, e->C, s);
-  launchCarryF2(e->dY, e->yPitch, Y_OFF, pos, 0, e->C, s);
-  launchCarryF32(e->dMpx, e->mpxPitch, H_MPX, pos, 0, e->C, s);
-  launchCarryF32(e->dLraw, e->lrPitch, H_LR, pos, 0, e->C, s);
-  launchCarryF32(e->dRraw, e->lrPitch, H_LR, pos, 0, e->C, s);
-  launchCarryF32(e->dLf, e->lfPitch, H_LF, pos, 0, e->C, s);
-  launchCarryF32(e->dRf, e->lfPitch, H_LF, pos, 0, e->C, s);
-  cudaStreamSynchronize(s);
-  e->launches += 7;
+  carryHalos(e, HALO_X2 | HALO_Y | HALO_MPX | HALO_LR | HALO_LF, pos, 0, e->C, e->stream);
+  cudaStreamSynchronize(e->stream);
   e->seq = roundUp(e->seq, e->K);
   e->headFresh = true;
 }
-
-// Measurement variant (build_variant with -DFMGPU_EXP_SKIP, never the shipped library): leave the
-// main kernel of the stages named in FMGPU_SKIP out of the block pipeline, to see what each one
-// costs the step beside the others. Results are WRONG with any stage skipped.
-#ifdef FMGPU_EXP_SKIP
-static bool expSkip(const char *name) {
-  static const std::string v = getenv("FMGPU_SKIP") ? getenv("FMGPU_SKIP") : "";
-  return v.find(name) != std::string::npos;
-}
-#else
-constexpr bool expSkip(const char *) { return false; }
-#endif
 
 // One logical block (global number q, block b of a call of nb blocks) of channels
 // [ch0, ch0 + nch) through the stage streams of pipe P. iq / stride: this block's bytes.
@@ -690,12 +809,11 @@ void launchBlock(fmgpu_engine *e, fmgpu_engine::Pipe &P, int ch0, int nch, uint6
   using E = fmgpu_engine;
   const int K = e->K, N = e->N;
   const int slot = static_cast<int>(q % static_cast<uint64_t>(K));
-  const size_t t0 = static_cast<size_t>(slot) * N;  // the block's offset in every ring buffer
-  const size_t ringEnd = static_cast<size_t>(K) * N;
-  const bool carry = (slot == 0) && !e->headFresh;  // bring the tail of slot K-1 in front of slot 0
   const bool stereo = e->cfg.stereo != 0;
   const bool first = (b == 0), last = (b == nb - 1);
-  fmgpu_block_status *status = out.status ? out.status + b : nullptr;
+  // slot 0 brings the tail of slot K-1 in front of it
+  const BlockRef blk{ch0, nch, static_cast<size_t>(slot) * N, N, out.status ? out.status + b : nullptr, nb,
+                     (slot == 0) && !e->headFresh};
   auto ev = [&](int st, uint64_t qq) { return P.done[st][qq % static_cast<uint64_t>(e->ER)]; };
   // producers: stages of THIS block whose output the stage reads; overwritten: consumer stages
   // of the buffers it writes, which must have finished block q - K (same ring slot)
@@ -717,22 +835,15 @@ void launchBlock(fmgpu_engine *e, fmgpu_engine::Pipe &P, int ch0, int nch, uint6
 
   const bool decim = (e->M > 1) && !xcf;
   if (decim) {
-    cudaStream_t s = P.run[E::ST_DECIM];
     if (waitH2D) {
       need(E::ST_DECIM, {E::ST_H2D}, {E::ST_DC});
     } else {
       need(E::ST_DECIM, {}, {E::ST_DC});
     }
-    {
-      Span sp(e, "decimate", s);
-      if (!expSkip("decimate")) runDecim(e, iq, stride, e->dX1 + t0, N, ch0, nch, s);
-      launchCarryIq(e->dHistIq, e->dHistValid, iq, stride, static_cast<long>(N) * e->M, ch0, nch, s);
-      e->launches += 2;
-    }
+    stageDecimate(e, blk, iq, stride, P.run[E::ST_DECIM]);
     done(E::ST_DECIM);
   }
   {
-    cudaStream_t s = P.run[E::ST_DC];
     if (decim) {
       need(E::ST_DC, {E::ST_DECIM}, {E::ST_CHAN});
     } else if (waitH2D) {
@@ -740,25 +851,11 @@ void launchBlock(fmgpu_engine *e, fmgpu_engine::Pipe &P, int ch0, int nch, uint6
     } else {
       need(E::ST_DC, {}, {E::ST_CHAN});
     }
-    Span sp(e, "dcblock", s);
-    if (carry) {
-      launchCarryF2(e->dX2, e->x2Pitch, H_X2, ringEnd, ch0, nch, s);
-      e->launches += 1;
-    }
-    if (e->scanMode == 1 && (xcf || decim)) {
-      // float input: the two recursions as a warp-shuffle scan (fast arithmetic)
-      if (!expSkip("dcblock")) launchDcBlockScan(xcf ? xcf : e->dX1 + t0, xcf ? xcfStride : e->pitch, e->dX2 + t0, e->x2Pitch,
-                        e->dDemod, status, nb, N, ch0, nch, e->k.dc_a1_iq, s);
-    } else if (xcf) {
-      // complex-float input at the DSP rate (FMDemod::processSplitComplex): read in place
-      launchDcBlock(xcf, xcfStride, nullptr, 0, e->dX2 + t0, e->x2Pitch, e->dDemod, status, nb, 1, N,
-                    N, ch0, nch, e->k.dc_a1_iq, s);
-    } else {
-      launchDcBlock(decim ? e->dX1 + t0 : nullptr, e->pitch, decim ? nullptr : iq, stride,
-                    e->dX2 + t0, e->x2Pitch, e->dDemod, status, nb, 1, N, N, ch0, nch,
-                    e->k.dc_a1_iq, s);
-    }
-    e->launches += 1;
+    // float input (complex-float rows at the DSP rate, read in place, or the decimator's output) may
+    // take the scan form; IQ bytes at the DSP rate go to the serial recursions
+    const float2 *x = xcf ? xcf : (decim ? e->dX1 + blk.t0 : nullptr);
+    stageDcBlock(e, blk, x, xcf ? xcfStride : e->pitch, x ? nullptr : iq, stride, e->scanMode == 1 && x,
+                 P.run[E::ST_DC]);
   }
   done(E::ST_DC);
   // fused tensor-core form of channel filter + discriminator: every channel of the range on the same
@@ -775,223 +872,66 @@ void launchBlock(fmgpu_engine *e, fmgpu_engine::Pipe &P, int ch0, int nch, uint6
       fusedFilt = -1;
     }
   }
+  bool fused = false;
   if (fusedFilt >= 0) {
-    // one kernel on the channel-filter stream: reads x2, writes MPX (and the discriminator's carried
-    // sample into the y row); the AGC and discriminator stages of this block are empty
-    cudaStream_t s = P.run[E::ST_CHAN];
+    // one kernel on the channel-filter stream; the AGC and discriminator stages of this block are empty
     if (stereo) {
       need(E::ST_CHAN, {E::ST_DC}, {E::ST_AGC, E::ST_FD, E::ST_PILOT, E::ST_STEREO, E::ST_RDS, E::ST_RDSRS});
     } else {
       need(E::ST_CHAN, {E::ST_DC}, {E::ST_AGC, E::ST_FD, E::ST_RDS, E::ST_RDSRS, E::ST_AF});
     }
-    Span sp(e, "chan_demod", s);
-    if (carry) {
-      launchCarryF2(e->dY, e->yPitch, Y_OFF, ringEnd, ch0, nch, s);  // slot Y_OFF-1 <- last output
-      launchCarryF32(e->dMpx, e->mpxPitch, H_MPX, ringEnd, ch0, nch, s);
-      e->launches += 2;
-    }
-    const auto &f = e->filters[fusedFilt];
-    const cudaError_t err = expSkip("chan_demod") ? cudaSuccess :
-        launchChanDemodTc(e->dX2 + t0, e->x2Pitch, H_X2, e->dY + t0, e->yPitch, e->dMpx + t0, e->mpxPitch,
-                          H_MPX, N, ch0, nch, f.scale, e->k.fd_ref, f.tc, f.dB, 21, e->smCount, s);
-    if (err != cudaSuccess) {
-      // refused before anything was launched (alignment, pitch): the three-kernel path takes the block
-      e->lastError = std::string("tensor-core channel filter + discriminator: ") + cudaGetErrorString(err);
-      fusedFilt = -1;
-    }
-    e->launches += 1;
+    // refused: the three-kernel path takes the block
+    fused = stageChanDemod(e, blk, fusedFilt, P.run[E::ST_CHAN]);
   }
-  if (fusedFilt < 0) {
-    cudaStream_t s = P.run[E::ST_CHAN];
+  if (!fused) {
     need(E::ST_CHAN, {E::ST_DC}, {E::ST_AGC, E::ST_FD});
-    Span sp(e, "chanfir", s);
-    launchChanFir(e->dX2 + t0, e->x2Pitch, e->dY + t0, e->yPitch, e->dChanTaps, e->dChanLp,
-                  e->dChanScale, e->dParams, N, ch0, nch, s);
-    e->launches += 1;
+    stageChanFir(e, blk, P.run[E::ST_CHAN]);
   }
   done(E::ST_CHAN);
-  {
-    cudaStream_t s = P.run[E::ST_AGC];
-    need(E::ST_AGC, {E::ST_CHAN}, {E::ST_FD});
-    bool anyAgc = false;
-    for (int c = ch0; c < ch0 + nch && !anyAgc && fusedFilt < 0; c++) {
-      anyAgc = e->hParams[c].agc_mode != 0;
-    }
-    if (anyAgc) {
-      // (running the discriminator inside this lane kernel was tried: its two IEEE divisions per
-      // sample do not hide behind the AGC recursion, the stage took 5.6 ms instead of 2.7 + 0.7)
-      Span sp(e, "agc", s);
-      launchAgc(e->dY + t0, e->yPitch, e->dDemod, e->dParams, N, ch0, nch, s);
-      e->launches += 1;
-    }
+  need(E::ST_AGC, {E::ST_CHAN}, {E::ST_FD});
+  if (!fused && anyAgc(e, ch0, nch)) {
+    stageAgc(e, blk, P.run[E::ST_AGC]);
   }
   done(E::ST_AGC);
-  {
-    cudaStream_t s = P.run[E::ST_FD];
-    if (stereo) {
-      need(E::ST_FD, {E::ST_AGC}, {E::ST_PILOT, E::ST_STEREO, E::ST_RDS, E::ST_RDSRS});
-    } else {
-      need(E::ST_FD, {E::ST_AGC}, {E::ST_RDS, E::ST_RDSRS, E::ST_AF /* the mono chain reads MPX */});
-    }
-    if (fusedFilt < 0) {
-      Span sp(e, "freqdem", s);
-      if (carry) {
-        launchCarryF2(e->dY, e->yPitch, Y_OFF, ringEnd, ch0, nch, s);  // slot Y_OFF-1 <- last output
-        launchCarryF32(e->dMpx, e->mpxPitch, H_MPX, ringEnd, ch0, nch, s);
-        e->launches += 2;
-      }
-      launchFreqDem(e->dY + t0, e->yPitch, e->dMpx + t0, e->mpxPitch, N, ch0, nch, e->k.fd_ref, s);
-      e->launches += 1;
-    }
+  if (stereo) {
+    need(E::ST_FD, {E::ST_AGC}, {E::ST_PILOT, E::ST_STEREO, E::ST_RDS, E::ST_RDSRS});
+  } else {
+    need(E::ST_FD, {E::ST_AGC}, {E::ST_RDS, E::ST_RDSRS, E::ST_AF /* the mono chain reads MPX */});
+  }
+  if (!fused) {
+    stageFreqDem(e, blk, P.run[E::ST_FD]);
   }
   done(E::ST_FD);
   // ---- RDS branch --------------------------------------------------------------------------
   // two stages: the 171 kHz resampler (tile kernel) of block q + 1 runs beside the demodulator
   // (lane kernel) of block q; the 171 kHz rows and their counts are double-buffered by block parity
-  const RdsRsRef rr{e->dRdsRs, static_cast<int>(q & 1)};
-  float *r171 = e->dR171 + static_cast<size_t>(q & 1) * static_cast<size_t>(e->C) * e->r171Pitch;
-  {
-    cudaStream_t s = P.run[E::ST_RDSRS];
-    need(E::ST_RDSRS, {E::ST_FD}, {});
-    if (q >= 2) {
-      cudaStreamWaitEvent(s, ev(E::ST_RDS, q - 2), 0);   // the demodulator is done with this parity's rows
-    }
-    Span sp(e, "rds_resample", s);
-    launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, 1, N, N, ch0, nch, e->k.aud_step, e->k.rds_step, 0, 0,
-                  2, 0, rr, s);
-    if (!expSkip("rds_resample")) launchRdsResample(e->dMpx + t0, e->mpxPitch, e->dRdsHist, 32, rr, e->dRdsBank, r171, e->r171Pitch,
-                      max171(e, N), ch0, nch, e->k, s);
-    launchSaveTail(e->dMpx + t0, e->mpxPitch, H_MPX, e->dRdsHist, 32, RDS_HIST, N, ch0, nch, s);
-    launchCommit(e->dAudioSt, e->dRds, ch0, nch, 0, 0, 1, rr, s);
-    e->launches += 4;
+  const int par = static_cast<int>(q & 1);
+  need(E::ST_RDSRS, {E::ST_FD}, {});
+  if (q >= 2) {
+    cudaStreamWaitEvent(P.run[E::ST_RDSRS], ev(E::ST_RDS, q - 2), 0);   // the demodulator is done with this parity's rows
   }
+  stageRdsResample(e, blk, par, P.run[E::ST_RDSRS]);
   done(E::ST_RDSRS);
-  {
-    cudaStream_t s = P.run[E::ST_RDS];
-    need(E::ST_RDS, {E::ST_RDSRS}, {});
-    {
-      Span sp(e, "rds", s);  // lane kernel: 57 kHz mix ... bits
-      if (first) {
-        launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, 1, N, N, ch0, nch, e->k.aud_step, e->k.rds_step, 0,
-                      0, 3, 1, rr, s);   // the call's group / bit counters
-        e->launches += 1;
-      }
-      if (!expSkip("rds_demod")) launchRdsDemod(e->dRds, e->dRing, e->dRdsLpf, e->dMf, e->dDmf, r171, e->r171Pitch, e->dBits,
-                     static_cast<uint32_t>(e->bitsCap), e->dBitEnd, ch0, nch, e->k, rr, s);
-    }
-    e->launches += 1;
-    {
-      Span sp(e, "rds_sync", s);  // syndromes at every bit offset + block sync state machine
-      if (!expSkip("rds_sync")) launchBlockSync(e->dBits, static_cast<uint32_t>(e->bitsCap), e->dBitEnd, e->dRds, e->dWords,
-                      out.groups, out.gcap, status, nb, 1, b, ch0, nch, s);
-      if (last) {
-        // the call's group counts, from the stream that owns RdsState::n_groups: the next call's
-        // first k_prepare on this stream zeroes it again
-        launchStoreCounts(e->dAudioSt, e->dRds, nullptr, out.nGroups, ch0, nch, stereo ? 0 : 1,
-                          static_cast<uint32_t>(out.acap), out.gcap, s);
-        e->launches += 1;
-      }
-    }
-    e->launches += 1;
-  }
+  need(E::ST_RDS, {E::ST_RDSRS}, {});
+  stageRdsDemod(e, blk, par, out, b, first, last, P.run[E::ST_RDS]);
   done(E::ST_RDS);
   // ---- audio branch ------------------------------------------------------------------------
   cudaStream_t sAf = P.run[E::ST_AF];
   if (stereo) {
-    {
-      cudaStream_t s = P.run[E::ST_PILOT];
-      need(E::ST_PILOT, {E::ST_FD}, {E::ST_STEREO});
-      Span sp(e, "pilot_fir", s);
-      FirRealJob j{};
-      j.in[0] = e->dMpx + t0;
-      j.out[0] = e->dPilot + t0;
-      j.in_pitch = e->mpxPitch;
-      j.out_pitch = e->pitch;
-      j.in_off = H_MPX;
-      j.out_off = 0;
-      j.n_total = N;
-      j.Lp = e->pilLp;
-      j.scale = 1.0f;
-      j.ch0 = ch0;
-      if (!expSkip("pilot_fir")) runFirReal(e, j, 1, nch, e->pilParam, e->pilTcOk, e->pilTc, e->dPilB, 22, s);
-      e->launches += 1;
-    }
+    need(E::ST_PILOT, {E::ST_FD}, {E::ST_STEREO});
+    stagePilot(e, blk, P.run[E::ST_PILOT]);
     done(E::ST_PILOT);
-    {
-      cudaStream_t s = P.run[E::ST_STEREO];
-      need(E::ST_STEREO, {E::ST_PILOT}, {E::ST_LPF});
-      Span sp(e, "stereo_pll", s);
-      if (carry) {
-        launchCarryF32(e->dLraw, e->lrPitch, H_LR, ringEnd, ch0, nch, s);
-        launchCarryF32(e->dRraw, e->lrPitch, H_LR, ringEnd, ch0, nch, s);
-        e->launches += 2;
-      }
-      if (!expSkip("stereo_pll")) launchStereo(e->dMpx + t0, e->mpxPitch, e->dPilot + t0, e->pitch, e->dLraw + t0, e->dRraw + t0,
-                   e->lrPitch, e->dStereo, e->dParams, status, nb, 1, N, N, ch0, nch, e->k, s);
-      e->launches += 1;
-    }
+    need(E::ST_STEREO, {E::ST_PILOT}, {E::ST_LPF});
+    stageStereo(e, blk, P.run[E::ST_STEREO]);
     done(E::ST_STEREO);
-    {
-      cudaStream_t s = P.run[E::ST_LPF];
-      need(E::ST_LPF, {E::ST_STEREO}, {E::ST_AF});
-      Span sp(e, "audio_lpf", s);
-      if (carry) {
-        launchCarryF32(e->dLf, e->lfPitch, H_LF, ringEnd, ch0, nch, s);
-        launchCarryF32(e->dRf, e->lfPitch, H_LF, ringEnd, ch0, nch, s);
-        e->launches += 2;
-      }
-      FirRealJob j{};
-      j.in[0] = e->dLraw + t0;
-      j.in[1] = e->dRraw + t0;
-      j.out[0] = e->dLf + t0;
-      j.out[1] = e->dRf + t0;
-      j.in_pitch = e->lrPitch;
-      j.out_pitch = e->lfPitch;
-      j.in_off = H_LR;
-      j.out_off = H_LF;
-      j.n_total = N;
-      j.Lp = e->audLp;
-      j.scale = e->k.aud_scale;
-      j.ch0 = ch0;
-      if (!expSkip("audio_lpf")) runFirReal(e, j, 2, nch, e->audParam, e->audTcOk, e->audTc, e->dAudB, 20, s);
-      e->launches += 1;
-    }
+    need(E::ST_LPF, {E::ST_STEREO}, {E::ST_AF});
+    stageLpf(e, blk, P.run[E::ST_LPF]);
     done(E::ST_LPF);
-    {
-      need(E::ST_AF, {E::ST_LPF}, {});
-      Span sp(e, "afpost", sAf);
-      launchPrepare(e->dAudioSt, e->dRds, status, nb, 1, N, N, ch0, nch, e->k.aud_step, e->k.rds_step,
-                    1, 0, 0, first ? 1 : 0, RdsRsRef{e->dRdsRs, 0}, sAf);
-      const int maxOut = static_cast<int>(std::min<size_t>(
-          out.acap, static_cast<size_t>((static_cast<double>(N) * 16777216.0) / e->k.aud_step) + 2));
-      if (!expSkip("afpost")) launchResample(e->dLf + t0, e->dRf + t0, e->lfPitch, H_LF, nullptr, 0, out.audio, out.acap,
-                     e->dAudBank, AUD_RS_LEN, e->k.aud_step, e->dAudioSt, 0, maxOut, ch0, nch, sAf);
-      if (e->scanMode == 1) {
-        launchAudioIirScan(out.audio, out.acap, e->dAudioSt, e->dParams, ch0, nch, e->k.dc_a1_af, 1, sAf);
-      } else {
-        launchAudioIir(out.audio, out.acap, e->dAudioSt, e->dParams, ch0, nch, e->k.dc_a1_af, 0, 1, 0,
-                       sAf);
-      }
-      launchCommit(e->dAudioSt, e->dRds, ch0, nch, 1, 0, 0, RdsRsRef{e->dRdsRs, 0}, sAf);
-      e->launches += 4;
-    }
+    need(E::ST_AF, {E::ST_LPF}, {});
+    stageAfPost(e, blk, out, first, e->scanMode == 1, 1, sAf);
   } else {
-    // FMDemod mono chain (main.cpp:1267-1279): MPX -> resample -> de-emphasis -> DC block, x0.5 to
-    // both rows
     need(E::ST_AF, {E::ST_FD}, {});
-    Span sp(e, "mono", sAf);
-    launchPrepare(e->dAudioSt, e->dRds, status, nb, 1, N, N, ch0, nch, e->k.aud_step, e->k.rds_step,
-                  0, 1, 0, first ? 1 : 0, RdsRsRef{e->dRdsRs, 0}, sAf);
-    const int maxOut = static_cast<int>(std::min<size_t>(
-        out.acap, static_cast<size_t>((static_cast<double>(N) * 16777216.0) / e->k.aud_step) + 2));
-    launchResample(e->dMpx + t0, nullptr, e->mpxPitch, H_MPX, e->dMonoHist, 32, out.audio, out.acap,
-                   e->dAudBank, AUD_RS_LEN, e->k.aud_step, e->dAudioSt, 1, maxOut, ch0, nch, sAf);
-    launchAudioIir(out.audio, out.acap, e->dAudioSt, e->dParams, ch0, nch, e->k.mono_dc_a1, 1, 1, 1,
-                   sAf);
-    launchSaveTail(e->dMpx + t0, e->mpxPitch, H_MPX, e->dMonoHist, 32, AUD_RS_LEN - 1, N, ch0, nch,
-                   sAf);
-    launchCommit(e->dAudioSt, e->dRds, ch0, nch, 0, 1, 0, RdsRsRef{e->dRdsRs, 0}, sAf);
-    e->launches += 5;
+    stageMono(e, blk, out, first, 1, 1, sAf);
   }
   if (last) {
     // the call's counts, once both branches have finished its last block
@@ -1111,10 +1051,11 @@ int queueBlocks(fmgpu_engine *e, const uint8_t *iq_dev, const uint8_t *iq_host, 
   return FMGPU_OK;
 }
 
+// iq_dev: IQ bytes, or (cf32) complex floats at the DSP rate; stride in bytes either way
 int runBatch(fmgpu_engine *e, const uint8_t *iq_dev, size_t stride, int n_blocks, float *audio_dev,
              size_t audio_cap, uint32_t *n_audio_dev, fmgpu_rds_group *groups_dev, size_t group_cap,
              uint32_t *n_groups_dev, fmgpu_block_status *status_dev, cudaStream_t s,
-             bool join = true) {
+             bool join = true, bool cf32 = false) {
   int rc = checkBatchArgs(e, iq_dev, stride, n_blocks, true, audio_dev, audio_cap);
   if (rc != FMGPU_OK) {
     return rc;
@@ -1132,6 +1073,10 @@ int runBatch(fmgpu_engine *e, const uint8_t *iq_dev, size_t stride, int n_blocks
   // audio is produced straight into the caller's buffer when one is given
   out.audio = audio_dev ? audio_dev : e->dAudio;
   out.acap = audio_dev ? audio_cap : e->acap;
+  if (cf32) {
+    return queueBlocks(e, nullptr, nullptr, 0, n_blocks, out, s, join, reinterpret_cast<const float2 *>(iq_dev),
+                       stride / sizeof(float2));
+  }
   return queueBlocks(e, iq_dev, nullptr, stride, n_blocks, out, s, join);
 }
 
@@ -1443,7 +1388,6 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
   CKC(devAlloc(&e->dNGroups2, C));
   CKC(devAlloc(&e->dBits, C * e->bitsCap));
   CKC(devAlloc(&e->dWords, C * e->bitsCap));
-  CKC(devAlloc(&e->dBitEnd, C * static_cast<size_t>(e->maxBlocks)));
   CKC(cudaMemcpy(e->dAudBank, e->audRs.bank.data(), e->audRs.bank.size() * sizeof(float),
                  cudaMemcpyHostToDevice));
   CKC(cudaMemcpy(e->dRdsBank, e->rdsRs.bank.data(), e->rdsRs.bank.size() * sizeof(float),
@@ -1502,7 +1446,7 @@ void fmgpu_engine_destroy(fmgpu_engine *e) {
                   e->dRing,    e->dRdsHist, e->dMonoHist, e->dChanTaps, e->dChanScale, e->dChanLp,
                   e->dAudBank, e->dRdsBank, e->dRdsLpf, e->dMf,     e->dDmf,     e->dParams,
                   e->dDemod,   e->dStereo, e->dAudioSt, e->dRds,    e->dGroups,  e->dStatus,
-                  e->dNAudio,  e->dNGroups, e->dBits, e->dHistValid, e->dWords, e->dBitEnd,
+                  e->dNAudio,  e->dNGroups, e->dBits, e->dHistValid, e->dWords,
                   e->dAudio2,  e->dGroups2, e->dStatus2, e->dNAudio2, e->dNGroups2, e->dR171,
                   e->dDecB,    e->dDecOffs, e->dPilB, e->dAudB, e->dRdsRs};
   for (auto &f : e->filters) {
@@ -1940,26 +1884,9 @@ int fmgpu_process_batch_cf32(fmgpu_engine *e, const float *x_cf32_dev, size_t st
     e->lastError = "process_batch_cf32: bad input pointer, alignment, stride or block count";
     return FMGPU_EINVAL;
   }
-  const size_t n = static_cast<size_t>(n_blocks) * e->N;
-  const size_t needAudio = static_cast<size_t>((static_cast<double>(n) * 16777216.0) / e->k.aud_step) + 2;
-  if (audio_dev && audio_cap < needAudio) {
-    e->lastError = "process: audio capacity too small";
-    return FMGPU_ERANGE;
-  }
-  int rc = uploadParams(e);
-  if (rc != FMGPU_OK) {
-    return rc;
-  }
-  BatchOut out;
-  out.status = status_dev ? status_dev : e->dStatus;
-  out.groups = groups_dev ? groups_dev : e->dGroups;
-  out.gcap = static_cast<uint32_t>(groups_dev ? group_cap : e->gcap);
-  out.nAudio = n_audio_dev ? n_audio_dev : e->dNAudio;
-  out.nGroups = n_groups_dev ? n_groups_dev : e->dNGroups;
-  out.audio = audio_dev ? audio_dev : e->dAudio;
-  out.acap = audio_dev ? audio_cap : e->acap;
-  rc = queueBlocks(e, nullptr, nullptr, 0, n_blocks, out, static_cast<cudaStream_t>(stream), true,
-                   reinterpret_cast<const float2 *>(x_cf32_dev), stride_samples);
+  const int rc = runBatch(e, reinterpret_cast<const uint8_t *>(x_cf32_dev), stride_samples * sizeof(float2),
+                          n_blocks, audio_dev, audio_cap, n_audio_dev, groups_dev, group_cap, n_groups_dev,
+                          status_dev, static_cast<cudaStream_t>(stream), true, true);
   if (rc == FMGPU_OK && e->timing) {
     CK(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));
     collectTimes(e);
@@ -2262,7 +2189,7 @@ size_t fmgpu_decimate(fmgpu_engine *e, int channel, const uint8_t *iq, size_t in
   }
   uint8_t *dst = e->dIq + static_cast<size_t>(channel) * e->iqPitch;
   cudaMemcpyAsync(dst, iq, n_out * e->M * 2, cudaMemcpyHostToDevice, s);
-  stageDecimate(e, e->dIq, e->iqPitch, static_cast<int>(n_out), channel, 1, s);
+  stageDecimate(e, stageBlock(channel, static_cast<int>(n_out)), e->dIq, e->iqPitch, s);
   cudaMemcpyAsync(out_cf32, e->dX1 + static_cast<size_t>(channel) * e->pitch, n_out * sizeof(float2),
                   cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
@@ -2283,7 +2210,7 @@ size_t fmgpu_decimate_u8(fmgpu_engine *e, int channel, const uint8_t *iq, size_t
   }
   uint8_t *row = e->dIq + static_cast<size_t>(channel) * e->iqPitch;
   cudaMemcpyAsync(row, iq, n_out * e->M * 2, cudaMemcpyHostToDevice, s);
-  stageDecimate(e, e->dIq, e->iqPitch, static_cast<int>(n_out), channel, 1, s);
+  stageDecimate(e, stageBlock(channel, static_cast<int>(n_out)), e->dIq, e->iqPitch, s);
   // the uint8 result goes back through the front of the channel's (already consumed) input row
   launchRequantU8(e->dX1, e->pitch, e->dIq, e->iqPitch, static_cast<int>(n_out), channel, 1, s);
   e->launches += 1;
@@ -2307,19 +2234,23 @@ static size_t demodCommon(fmgpu_engine *e, int channel, const uint8_t *iq_u8, co
     cudaMemcpyAsync(e->dX1 + static_cast<size_t>(channel) * e->pitch, iq_cf32, n * sizeof(float2),
                     cudaMemcpyHostToDevice, s);
   }
-  if (mono_out) {
-    launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, 1, ni, ni, channel, 1, e->k.aud_step,
-                  e->k.rds_step, 0, 1, 0, 1, RdsRsRef{e->dRdsRs, 0}, s);
+  // the serial chain whatever the scan and demodulator modes: DC blocker -> channel FIR -> [AGC] ->
+  // discriminator
+  const BlockRef blk = stageBlock(channel, ni);
+  stageDcBlock(e, blk, iq_u8 ? nullptr : e->dX1, e->pitch, iq_u8 ? e->dIq : nullptr, e->iqPitch, false, s);
+  stageChanFir(e, blk, s);
+  if (anyAgc(e, channel, 1)) {
+    stageAgc(e, blk, s);
   }
-  stageDemod(e, iq_u8 ? e->dIq : nullptr, e->iqPitch, nullptr, 1, ni, ni, channel, 1, s);
+  stageFreqDem(e, blk, s);
+  carryHalos(e, HALO_X2 | HALO_Y, blk.n, channel, 1, s);
   if (mpx_out) {
     cudaMemcpyAsync(mpx_out, e->dMpx + static_cast<size_t>(channel) * e->mpxPitch + H_MPX,
                     n * sizeof(float), cudaMemcpyDeviceToHost, s);
   }
   size_t produced = 0;
   if (mono_out) {
-    stageMono(e, ni, 0, 0, channel, 1, s);
-    launchCommit(e->dAudioSt, e->dRds, channel, 1, 0, 1, 0, RdsRsRef{e->dRdsRs, 0}, s);
+    stageMono(e, blk, engineOut(e), true, 0, 0, s);
     AudioState a{};
     cudaMemcpyAsync(&a, e->dAudioSt + channel, sizeof(a), cudaMemcpyDeviceToHost, s);
     cudaStreamSynchronize(s);
@@ -2354,11 +2285,7 @@ size_t fmgpu_downsample_mono(fmgpu_engine *e, int channel, const float *mpx, flo
   const int ni = static_cast<int>(n);
   cudaMemcpyAsync(e->dMpx + static_cast<size_t>(channel) * e->mpxPitch + H_MPX, mpx,
                   n * sizeof(float), cudaMemcpyHostToDevice, s);
-  launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, 1, ni, ni, channel, 1, e->k.aud_step,
-                e->k.rds_step, 0, 1, 0, 1, RdsRsRef{e->dRdsRs, 0}, s);
-  stageMono(e, ni, 0, 0, channel, 1, s);
-  launchCommit(e->dAudioSt, e->dRds, channel, 1, 0, 1, 0, RdsRsRef{e->dRdsRs, 0}, s);
-  e->launches += 2;
+  stageMono(e, stageBlock(channel, ni), engineOut(e), true, 0, 0, s);
   AudioState a{};
   cudaMemcpyAsync(&a, e->dAudioSt + channel, sizeof(a), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
@@ -2379,7 +2306,11 @@ size_t fmgpu_stereo(fmgpu_engine *e, int channel, const float *mpx, float *left,
   const int ni = static_cast<int>(n);
   cudaMemcpyAsync(e->dMpx + static_cast<size_t>(channel) * e->mpxPitch + H_MPX, mpx,
                   n * sizeof(float), cudaMemcpyHostToDevice, s);
-  stageStereo(e, nullptr, 1, ni, ni, channel, 1, s);
+  const BlockRef blk = stageBlock(channel, ni);
+  stagePilot(e, blk, s);
+  stageStereo(e, blk, s);
+  stageLpf(e, blk, s);
+  carryHalos(e, HALO_MPX | HALO_LR, blk.n, channel, 1, s);
   cudaMemcpyAsync(left, e->dLf + static_cast<size_t>(channel) * e->lfPitch + H_LF, n * sizeof(float),
                   cudaMemcpyDeviceToHost, s);
   cudaMemcpyAsync(right, e->dRf + static_cast<size_t>(channel) * e->lfPitch + H_LF,
@@ -2421,10 +2352,8 @@ size_t fmgpu_afpost(fmgpu_engine *e, int channel, const float *in_left, const fl
                   n_eff * sizeof(float), cudaMemcpyHostToDevice, s);
   cudaMemcpyAsync(e->dRf + static_cast<size_t>(channel) * e->lfPitch + H_LF, in_right,
                   n_eff * sizeof(float), cudaMemcpyHostToDevice, s);
-  launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, 1, ni, ni, channel, 1, e->k.aud_step,
-                e->k.rds_step, 1, 0, 0, 1, RdsRsRef{e->dRdsRs, 0}, s);
-  stageAfPost(e, ni, 0, channel, 1, s);
-  launchCommit(e->dAudioSt, e->dRds, channel, 1, 1, 0, 0, RdsRsRef{e->dRdsRs, 0}, s);
+  stageAfPost(e, stageBlock(channel, ni), engineOut(e), true, false, 0, s);
+  carryHalos(e, HALO_LF, ni, channel, 1, s);
   cudaMemcpyAsync(&a, e->dAudioSt + channel, sizeof(a), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
   const size_t produced = std::min<size_t>({a.n_out, out_capacity, e->acap});
@@ -2433,7 +2362,6 @@ size_t fmgpu_afpost(fmgpu_engine *e, int channel, const float *in_left, const fl
   cudaMemcpyAsync(out_right, e->dAudio + (static_cast<size_t>(channel) * 2 + 1) * e->acap,
                   produced * sizeof(float), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
-  e->launches += 2;
   return stageFail(e, "afpost") ? 0 : produced;
 }
 
@@ -2447,11 +2375,10 @@ size_t fmgpu_rds(fmgpu_engine *e, int channel, const float *mpx, size_t n, fmgpu
   const int ni = static_cast<int>(n);
   cudaMemcpyAsync(e->dMpx + static_cast<size_t>(channel) * e->mpxPitch + H_MPX, mpx,
                   n * sizeof(float), cudaMemcpyHostToDevice, s);
-  launchPrepare(e->dAudioSt, e->dRds, nullptr, 1, 1, ni, ni, channel, 1, e->k.aud_step,
-                e->k.rds_step, 0, 0, 1, 1, RdsRsRef{e->dRdsRs, 0}, s);
-  stageRds(e, e->dGroups, static_cast<uint32_t>(e->gcap), nullptr, 1, ni, ni, channel, 1, s);
-  launchCommit(e->dAudioSt, e->dRds, channel, 1, 0, 0, 1, RdsRsRef{e->dRdsRs, 0}, s);
-  e->launches += 2;
+  // the block pipeline's two RDS stages, as the first block of a call (parity 0)
+  const BlockRef blk = stageBlock(channel, ni);
+  stageRdsResample(e, blk, 0, s);
+  stageRdsDemod(e, blk, 0, engineOut(e), 0, true, false, s);
   RdsState r{};
   cudaMemcpyAsync(&r, e->dRds + channel, sizeof(r), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);

@@ -611,8 +611,7 @@ __global__ void k_requant_u8(const float2 *__restrict__ x1, size_t x1_pitch, uin
 __global__ void __launch_bounds__(32)
 k_dcblock(const float2 *__restrict__ x1, size_t x1_pitch, const uint8_t *__restrict__ iq_u8,
           size_t iq_stride, float2 *__restrict__ x2, size_t x2_pitch, DemodState *st,
-          fmgpu_block_status *status, int status_pitch, int nblk, int blk_len, int n_total, int ch0,
-          int nch, float a1) {
+          fmgpu_block_status *status, int status_pitch, int n_total, int ch0, int nch, float a1) {
   // ONE warp per 32 channels, one lane per channel: the warp prefetches its next input tile
   // (cp.async), runs the recursions on the current one and writes the finished tile back itself.
   // (A separate mover warp doubles the registers and warp slots this kernel keeps from the FIR
@@ -640,8 +639,7 @@ k_dcblock(const float2 *__restrict__ x1, size_t x1_pitch, const uint8_t *__restr
     tileLoadAsync<TP, 2 * LT>(tin(0), x1f, 2 * x1_pitch, c0, nrows, 0, 2 * min(LT, n_total), lane);
     cpAsyncCommit();
   }
-  int b = 0, in_blk = 0, clip = 0;
-  int cur_len = min(blk_len, n_total);
+  int clip = 0;
   for (int ck = 0; ck < nchunks; ck++) {
     const int n0 = ck * LT;
     const int len = min(LT, n_total - n0);
@@ -656,63 +654,45 @@ k_dcblock(const float2 *__restrict__ x1, size_t x1_pitch, const uint8_t *__restr
       const float *ti = tin(ck) + lane * TP;
       float *to = tout + lane * TP;
       int i = 0;
-      while (i < len) {
-        const int run = min(len - i, cur_len - in_blk);
-        if (inb) {
-          for (int j = 0; j < run; j++, i++) {
-            const uchar2 v = inb[n0 + i];
-            if (v.x == 0 || v.x == 255 || v.y == 0 || v.y == 255) {
-              clip++;
-            }
-            const float ir = ((float)v.x - 127.0f) / 127.5f;
-            const float qr = ((float)v.y - 127.0f) / 127.5f;
-            const float v0i = ir - (a1 * vi);
-            to[2 * i] = v0i - vi;
-            vi = v0i;
-            const float v0q = qr - (a1 * vq);
-            to[2 * i + 1] = v0q - vq;
-            vq = v0q;
+      if (inb) {
+        for (; i < len; i++) {
+          const uchar2 v = inb[n0 + i];
+          if (v.x == 0 || v.x == 255 || v.y == 0 || v.y == 255) {
+            clip++;
           }
-        } else {
-          auto sample = [&](float ir, float qr, float &o_i, float &o_q) {
-            if (fabsf(ir) >= 0.995f || fabsf(qr) >= 0.995f) {
-              clip++;
-            }
-            const float v0i = ir - (a1 * vi);
-            o_i = v0i - vi;
-            vi = v0i;
-            const float v0q = qr - (a1 * vq);
-            o_q = v0q - vq;
-            vq = v0q;
-          };
-          int j = 0;
-          if ((i & 1) == 0) {
-            // two complex samples per 128-bit shared-memory access (conflict-free; the 32-bit
-            // form hits 8 banks)
-#pragma unroll 2
-            for (; j + 2 <= run; j += 2, i += 2) {
-              const float4 v = *reinterpret_cast<const float4 *>(ti + 2 * i);
-              float4 o;
-              sample(v.x, v.y, o.x, o.y);
-              sample(v.z, v.w, o.z, o.w);
-              *reinterpret_cast<float4 *>(to + 2 * i) = o;
-            }
-          }
-          for (; j < run; j++, i++) {
-            sample(ti[2 * i], ti[2 * i + 1], to[2 * i], to[2 * i + 1]);
-          }
+          const float ir = ((float)v.x - 127.0f) / 127.5f;
+          const float qr = ((float)v.y - 127.0f) / 127.5f;
+          const float v0i = ir - (a1 * vi);
+          to[2 * i] = v0i - vi;
+          vi = v0i;
+          const float v0q = qr - (a1 * vq);
+          to[2 * i + 1] = v0q - vq;
+          vq = v0q;
         }
-        in_blk += run;
-        if (in_blk == cur_len) {
-          s.clipping = (clip > 0) ? 1 : 0;
-          s.clip_ratio = (float)clip / (float)cur_len;
-          if (status) {
-            status[(size_t)c * status_pitch + b].clip_ratio = s.clip_ratio;
+      } else {
+        auto sample = [&](float ir, float qr, float &o_i, float &o_q) {
+          if (fabsf(ir) >= 0.995f || fabsf(qr) >= 0.995f) {
+            clip++;
           }
-          b++;
-          in_blk = 0;
-          clip = 0;
-          cur_len = min(blk_len, n_total - b * blk_len);
+          const float v0i = ir - (a1 * vi);
+          o_i = v0i - vi;
+          vi = v0i;
+          const float v0q = qr - (a1 * vq);
+          o_q = v0q - vq;
+          vq = v0q;
+        };
+        // two complex samples per 128-bit shared-memory access (conflict-free; the 32-bit
+        // form hits 8 banks)
+#pragma unroll 2
+        for (; i + 2 <= len; i += 2) {
+          const float4 v = *reinterpret_cast<const float4 *>(ti + 2 * i);
+          float4 o;
+          sample(v.x, v.y, o.x, o.y);
+          sample(v.z, v.w, o.z, o.w);
+          *reinterpret_cast<float4 *>(to + 2 * i) = o;
+        }
+        for (; i < len; i++) {
+          sample(ti[2 * i], ti[2 * i + 1], to[2 * i], to[2 * i + 1]);
         }
       }
     }
@@ -720,11 +700,15 @@ k_dcblock(const float2 *__restrict__ x1, size_t x1_pitch, const uint8_t *__restr
     tileStore<TP, 2 * LT>(tout, x2f, 2 * x2_pitch, c0, nrows, 2L * (H_X2 + n0), 2 * len, lane);
   }
   if (active) {
+    const float clip_ratio = (float)clip / (float)n_total;
+    if (status) {
+      status[(size_t)c * status_pitch].clip_ratio = clip_ratio;
+    }
     // only this stage's fields: the AGC stage of the previous block may be running beside it
     st[c].dc_i = vi;
     st[c].dc_q = vq;
-    st[c].clipping = s.clipping;
-    st[c].clip_ratio = s.clip_ratio;
+    st[c].clipping = (clip > 0) ? 1 : 0;
+    st[c].clip_ratio = clip_ratio;
   }
 }
 
@@ -1004,8 +988,8 @@ k_freqdem(const float2 *__restrict__ ybuf, size_t y_pitch, float *__restrict__ m
 //              copies the blend recursion and the L-R matrix
 //   warp 1     PLL + envelopes: pilot -> phase error -> NCO update -> sin/cos of the new phase is
 //              the one truly serial chain (~264 cycles per sample on B200, tools/microbench/
-//              lat_bench.cu); the four one-pole envelopes and the per-block stereo-lock logic ride
-//              in its idle issue slots
+//              lat_bench.cu); the four one-pole envelopes ride in its idle issue slots, and the
+//              stereo-lock logic runs once, after the block's last sample
 //   warps 2,3  blend target from the envelopes (up to six IEEE divisions and two square roots per
 //              sample, but element-wise): each takes half of the tile's samples
 // Round 1 ran everything behind the PLL in ONE warp; with weak signals (no clean-pilot shortcut)
@@ -1025,7 +1009,7 @@ __global__ void __launch_bounds__(STEREO_THREADS, STEREO_MINB)
 k_stereo(const float *__restrict__ mpx, size_t mpx_pitch, const float *__restrict__ pilot,
          size_t pilot_pitch, float *__restrict__ lraw, float *__restrict__ rraw, size_t lr_pitch,
          StereoState *st, const ChanParams *cp, fmgpu_block_status *status, int status_pitch,
-         int nblk, int blk_len, int n_total, int ch0, int nch, EngineConst k) {
+         int n_total, int ch0, int nch, EngineConst k) {
   constexpr int ST = STEREO_ST;  // samples per tile row
   // 16-byte aligned rows, read and written by their lane four samples at a time; a pitch of ST + 4
   // floats is odd in 16-byte units, so the 8 lanes of a quarter-warp hit 8 different bank groups
@@ -1091,9 +1075,7 @@ k_stereo(const float *__restrict__ mpx, size_t mpx_pitch, const float *__restric
     cpAsyncWait<0>();
   }
   __syncthreads();
-  int b = 0, in_blk = 0;
-  int cur_len = min(blk_len, n_total);
-  bool stereoDetected = s.stereo != 0;
+  const bool stereoDetected = s.stereo != 0;  // the lock logic runs once, after the last sample
 
   // step kk: PLL + envelopes on chunk kk, target on chunk kk-1, blend + matrix on chunk kk-2; the
   // mover loads pilot[kk+1], mpx[kk+1], delayed mpx[kk-1] and stores L/R of chunk kk-3
@@ -1200,76 +1182,24 @@ k_stereo(const float *__restrict__ mpx, size_t mpx_pitch, const float *__restric
           vcoI = cs;
         };
         int i = 0;
-        while (i < len) {
-          const int run = min(len - i, cur_len - in_blk);
-          int q = 0;
-          if ((i & 3) == 0) {
-            // four samples per 128-bit shared-memory access: a lane's row is 16-byte aligned, so a
-            // warp's access is conflict-free (the 32-bit form hits 8 banks: 4-way conflicts)
-            for (; q + 4 <= run; q += 4, i += 4) {
-              const float4 pv = ldsF4(a_tp + 4u * i);
-              const float4 xv = ldsF4(a_tm + 4u * i);
-              float4 of, ob, om, os, oc;
-              sample(pv.x, xv.x, of.x, ob.x, om.x, os.x, oc.x);
-              sample(pv.y, xv.y, of.y, ob.y, om.y, os.y, oc.y);
-              sample(pv.z, xv.z, of.z, ob.z, om.z, os.z, oc.z);
-              sample(pv.w, xv.w, of.w, ob.w, om.w, os.w, oc.w);
-              stsF4(a_tf + 4u * i, of);
-              stsF4(a_tpb + 4u * i, ob);
-              stsF4(a_tmm + 4u * i, om);
-              stsF4(a_ts2 + 4u * i, os);
-              stsF4(a_tc2 + 4u * i, oc);
-            }
-          }
-          for (; q < run; q++, i++) {  // ragged ends (a logical block ending inside the tile)
-            sample(tp[i], tm[i], tf[i], tpb[i], tmm[i], ts2[i], tc2[i]);
-          }
-          in_blk += run;
-          if (in_blk == cur_len) {
-            // per-block tail (stereo_decoder.cpp:243-286)
-            const float pilotMag = FM_SQRT((pilotI * pilotI) + (pilotQ * pilotQ));
-            s.pilot_mag = (s.pilot_mag * 0.9f) + (pilotMag * 0.1f);
-            const bool det = s.stereo != 0;
-            const float mpxThreshold = det ? kMpxMinHold : kMpxMinAcquire;
-            const float pilotRatio = pbm / fmaxf(mm, 1e-3f);
-            const float pilotCoherence = s.pilot_mag / fmaxf(pbm, 1e-4f);
-            const float ratioThreshold = det ? kPilotRatioHold : kPilotRatioAcquire;
-            const float coherenceThreshold = det ? kPilotCoherenceHold : kPilotCoherenceAcquire;
-            const float pllErrHz = fabsf(pllFreq - k.nominal_pll) * k.fsf / (2.0f * kPi);
-            const float pllThreshold = det ? kPllLockHoldHz : kPllLockAcquireHz;
-            const bool pilotPresent = (mm > mpxThreshold) && (pilotRatio > ratioThreshold) &&
-                                      (pilotCoherence > coherenceThreshold) && (pllErrHz < pllThreshold);
-            if (!p.force_stereo) {
-              if (!det) {
-                if (pilotPresent) {
-                  s.pilot_count++;
-                  s.loss_count = 0;
-                  if (s.pilot_count >= 6) {
-                    s.stereo = 1;
-                  }
-                } else {
-                  s.pilot_count = 0;
-                }
-              } else if (pilotPresent) {
-                s.loss_count = 0;
-              } else if (++s.loss_count >= 24) {
-                s.stereo = 0;
-                s.pilot_count = 0;
-                s.loss_count = 0;
-              }
-            }
-            const float calibrated = s.pilot_mag * 8.0f;
-            s.pilot_tenths = min(750, max(0, (int)fm_roundf(calibrated * 750.0f)));
-            if (status) {
-              fmgpu_block_status *o = &status[(size_t)c * status_pitch + b];
-              o->stereo = s.stereo;
-              o->pilot_tenths = s.pilot_tenths;
-            }
-            b++;
-            in_blk = 0;
-            cur_len = min(blk_len, n_total - b * blk_len);
-            stereoDetected = s.stereo != 0;
-          }
+        // four samples per 128-bit shared-memory access: a lane's row is 16-byte aligned, so a
+        // warp's access is conflict-free (the 32-bit form hits 8 banks: 4-way conflicts)
+        for (; i + 4 <= len; i += 4) {
+          const float4 pv = ldsF4(a_tp + 4u * i);
+          const float4 xv = ldsF4(a_tm + 4u * i);
+          float4 of, ob, om, os, oc;
+          sample(pv.x, xv.x, of.x, ob.x, om.x, os.x, oc.x);
+          sample(pv.y, xv.y, of.y, ob.y, om.y, os.y, oc.y);
+          sample(pv.z, xv.z, of.z, ob.z, om.z, os.z, oc.z);
+          sample(pv.w, xv.w, of.w, ob.w, om.w, os.w, oc.w);
+          stsF4(a_tf + 4u * i, of);
+          stsF4(a_tpb + 4u * i, ob);
+          stsF4(a_tmm + 4u * i, om);
+          stsF4(a_ts2 + 4u * i, os);
+          stsF4(a_tc2 + 4u * i, oc);
+        }
+        for (; i < len; i++) {  // ragged end of the block
+          sample(tp[i], tm[i], tf[i], tpb[i], tmm[i], ts2[i], tc2[i]);
         }
       }
     } else if (role == 2 || role == 3) {
@@ -1349,6 +1279,45 @@ k_stereo(const float *__restrict__ mpx, size_t mpx_pitch, const float *__restric
     __syncthreads();
   }
   if (active && role == 1) {
+    // per-block tail (stereo_decoder.cpp:243-286)
+    const float pilotMag = FM_SQRT((pilotI * pilotI) + (pilotQ * pilotQ));
+    s.pilot_mag = (s.pilot_mag * 0.9f) + (pilotMag * 0.1f);
+    const bool det = s.stereo != 0;
+    const float mpxThreshold = det ? kMpxMinHold : kMpxMinAcquire;
+    const float pilotRatio = pbm / fmaxf(mm, 1e-3f);
+    const float pilotCoherence = s.pilot_mag / fmaxf(pbm, 1e-4f);
+    const float ratioThreshold = det ? kPilotRatioHold : kPilotRatioAcquire;
+    const float coherenceThreshold = det ? kPilotCoherenceHold : kPilotCoherenceAcquire;
+    const float pllErrHz = fabsf(pllFreq - k.nominal_pll) * k.fsf / (2.0f * kPi);
+    const float pllThreshold = det ? kPllLockHoldHz : kPllLockAcquireHz;
+    const bool pilotPresent = (mm > mpxThreshold) && (pilotRatio > ratioThreshold) &&
+                              (pilotCoherence > coherenceThreshold) && (pllErrHz < pllThreshold);
+    if (!p.force_stereo) {
+      if (!det) {
+        if (pilotPresent) {
+          s.pilot_count++;
+          s.loss_count = 0;
+          if (s.pilot_count >= 6) {
+            s.stereo = 1;
+          }
+        } else {
+          s.pilot_count = 0;
+        }
+      } else if (pilotPresent) {
+        s.loss_count = 0;
+      } else if (++s.loss_count >= 24) {
+        s.stereo = 0;
+        s.pilot_count = 0;
+        s.loss_count = 0;
+      }
+    }
+    const float calibrated = s.pilot_mag * 8.0f;
+    s.pilot_tenths = min(750, max(0, (int)fm_roundf(calibrated * 750.0f)));
+    if (status) {
+      fmgpu_block_status *ob = &status[(size_t)c * status_pitch];
+      ob->stereo = s.stereo;
+      ob->pilot_tenths = s.pilot_tenths;
+    }
     StereoState *o = &st[c];
     o->theta = theta;
     o->dtheta = dtheta;
@@ -1383,11 +1352,9 @@ __device__ __forceinline__ uint32_t resampCount(uint32_t phase0, uint32_t step, 
 }
 
 __global__ void k_prepare(AudioState *au, RdsState *rds, fmgpu_block_status *status,
-                          int status_pitch, int nblk, int blk_len, int n_total, int ch0, int nch,
-                          uint32_t aud_step, uint32_t rds_step, int do_audio, int do_mono,
-                          int do_rds, int first, RdsRsRef rr) {
-  // do_rds: 1 = resampler bookkeeping + (first block of a call) the call's counters; 2 = the
-  // bookkeeping only (resampler stage of the block pipeline); 3 = the counters only (its demodulator stage)
+                          int status_pitch, int n_total, int ch0, int nch, uint32_t aud_step,
+                          uint32_t rds_step, int do_audio, int do_mono, int do_rds, int first,
+                          RdsRsRef rr) {
   const int lane = blockIdx.x * blockDim.x + threadIdx.x;
   if (lane >= nch) {
     return;
@@ -1409,23 +1376,16 @@ __global__ void k_prepare(AudioState *au, RdsState *rds, fmgpu_block_status *sta
       a->rs_phase_next = nx;
     }
     if (status) {
-      uint32_t prev = 0;
-      for (int b = 0; b < nblk; b++) {
-        const long upto = min((long)(b + 1) * blk_len, (long)n_total);
-        uint32_t dummy;
-        const uint32_t cum = resampCount(p0, aud_step, upto, &dummy);
-        status[(size_t)c * status_pitch + b].n_audio = (int)(cum - prev);
-        prev = cum;
-      }
+      status[(size_t)c * status_pitch].n_audio = (int)total;
     }
   }
-  if (do_rds == 1 || do_rds == 2) {
+  if (do_rds == PREPARE_RDS_RESAMPLER) {
     RdsRsState *q = &rr.st[c];
     uint32_t nx;
     q->n171[rr.par] = resampCount(q->rs_phase, rds_step, n_total, &nx);
     q->rs_phase_next = nx;
   }
-  if (do_rds == 1 || do_rds == 3) {
+  if (do_rds == PREPARE_RDS_COUNTERS) {
     RdsState *r = &rds[c];
     if (first) {
       r->n_groups = 0;  // groups and bits accumulate over the logical blocks of one call
@@ -1458,18 +1418,18 @@ __global__ void k_commit(AudioState *au, RdsState *rds, int ch0, int nch, int do
 // ---------------------------------------------------------------------------
 // K5b: arbitrary-rate polyphase resampler to 32 kHz (one thread per output frame)
 // ---------------------------------------------------------------------------
-// SUB > 0: the branch length known at compile time (24 for the audio resampler): the dot products
-// are fully unrolled, the taps of the thread's branch are read once (128-bit) and serve both rows.
-// The run-time form (SUB = 0) spent ~8 instructions per tap and row on loop bookkeeping.
-template <int SUB>
+// The branch length is known at compile time: the dot products are fully unrolled, the taps of the
+// thread's branch are read once (128-bit) and serve both rows. (A run-time length spent ~8
+// instructions per tap and row on loop bookkeeping.)
 __global__ void k_resample(const float *__restrict__ in0, const float *__restrict__ in1,
                            size_t in_pitch, int in_off, const float *__restrict__ hist,
                            int hist_pitch, float *__restrict__ out, size_t acap,
-                           const float *__restrict__ bank, int sub_len_rt, uint32_t step,
-                           const AudioState *au, int mono, int ch0) {
-  const int sub_len = (SUB > 0) ? SUB : sub_len_rt;
+                           const float *__restrict__ bank, uint32_t step, const AudioState *au,
+                           int mono, int ch0) {
+  constexpr int SUB = AUD_RS_LEN;
+  static_assert(SUB % 4 == 0, "the taps of a branch are read four at a time");
   extern __shared__ __align__(16) float bk[];
-  for (int i = threadIdx.x; i < 32 * sub_len; i += blockDim.x) {
+  for (int i = threadIdx.x; i < 32 * SUB; i += blockDim.x) {
     bk[i] = bank[i];
   }
   __syncthreads();
@@ -1484,10 +1444,10 @@ __global__ void k_resample(const float *__restrict__ in0, const float *__restric
   const unsigned long long P = (unsigned long long)phase0 + (unsigned long long)j * step;
   const long i = (long)(P >> 24);
   const int br = (int)((P & 0xffffffull) >> 19);
-  const float *h = bk + br * sub_len;
-  const float *a = in0 + (size_t)c * in_pitch + in_off + i - (sub_len - 1);
-  if (SUB > 0 && SUB % 4 == 0 && !(hist && i < sub_len - 1)) {
-    float hq[SUB > 0 ? SUB : 4];
+  const float *h = bk + br * SUB;
+  const float *a = in0 + (size_t)c * in_pitch + in_off + i - (SUB - 1);
+  if (!(hist && i < SUB - 1)) {
+    float hq[SUB];
 #pragma unroll
     for (int q = 0; q < SUB; q += 4) {
       const float4 v = *reinterpret_cast<const float4 *>(h + q);
@@ -1503,7 +1463,7 @@ __global__ void k_resample(const float *__restrict__ in0, const float *__restric
     }
     out[((size_t)c * 2 + 0) * acap + ob + j] = acc0;
     if (in1) {
-      const float *b = in1 + (size_t)c * in_pitch + in_off + i - (sub_len - 1);
+      const float *b = in1 + (size_t)c * in_pitch + in_off + i - (SUB - 1);
       float acc1 = 0.0f;
 #pragma unroll
       for (int q = 0; q < SUB; q++) {
@@ -1513,26 +1473,20 @@ __global__ void k_resample(const float *__restrict__ in0, const float *__restric
     }
     return;
   }
+  // window reaches before this call: those samples live in the stage's own history
+  const float *hc = hist + (size_t)c * hist_pitch;
+  constexpr int H = SUB - 1;
   float acc0 = 0.0f;
-  if (hist && i < sub_len - 1) {
-    // window reaches before this call: those samples live in the stage's own history
-    const float *hc = hist + (size_t)c * hist_pitch;
-    const int H = sub_len - 1;
-    for (int q = 0; q < sub_len; q++) {
-      const long si = i - (sub_len - 1) + q;
-      const float x = (si >= 0) ? a[q] : hc[H + si];
-      acc0 = fmaf(h[q], x, acc0);
-    }
-  } else {
-    for (int q = 0; q < sub_len; q++) {
-      acc0 = fmaf(h[q], a[q], acc0);
-    }
+  for (int q = 0; q < SUB; q++) {
+    const long si = i - (SUB - 1) + q;
+    const float x = (si >= 0) ? a[q] : hc[H + si];
+    acc0 = fmaf(h[q], x, acc0);
   }
   out[((size_t)c * 2 + 0) * acap + ob + j] = acc0;
   if (in1) {
-    const float *b = in1 + (size_t)c * in_pitch + in_off + i - (sub_len - 1);
+    const float *b = in1 + (size_t)c * in_pitch + in_off + i - (SUB - 1);
     float acc1 = 0.0f;
-    for (int q = 0; q < sub_len; q++) {
+    for (int q = 0; q < SUB; q++) {
       acc1 = fmaf(h[q], b[q], acc1);
     }
     out[((size_t)c * 2 + 1) * acap + ob + j] = acc1;
@@ -1974,8 +1928,8 @@ k_rds_resample(const float *__restrict__ mpx, size_t mpx_pitch, const float *__r
 __global__ void __maxnreg__(255)
 k_rds(const float *__restrict__ r171, size_t r_pitch, RdsState *st, float2 *ring,
       const float *__restrict__ g_lpf, const float *__restrict__ g_mf,
-      const float *__restrict__ g_dmf, uint8_t *bits_out, uint32_t bits_cap, uint32_t *bit_end,
-      int ch0, int nch, EngineConst k, RdsRsRef rr) {
+      const float *__restrict__ g_dmf, uint8_t *bits_out, uint32_t bits_cap, int ch0, int nch,
+      EngineConst k, RdsRsRef rr) {
   __shared__ float s_lpf[RDS_LPF_LEN + 1];
   __shared__ float s_mf[32 * SS_LEN];
   __shared__ float s_dmf[32 * SS_LEN];
@@ -2254,7 +2208,6 @@ k_rds(const float *__restrict__ r171, size_t r_pitch, RdsState *st, float2 *ring
   if (!active) {
     return;
   }
-  bit_end[c] = min(s.n_bits, bits_cap);  // bits demodulated so far in this call
 #pragma unroll
   for (int j = 0; j < RDS_NACC; j++) {
     s.acc[j] = acc[j];
@@ -2274,9 +2227,9 @@ k_rds(const float *__restrict__ r171, size_t r_pitch, RdsState *st, float2 *ring
 // (every bit while searching for sync, every 26th once locked).
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(128)
-k_blocksync(const uint8_t *__restrict__ bits, uint32_t bits_cap, const uint32_t *__restrict__ bit_end,
-            RdsState *st, unsigned long long *words, fmgpu_rds_group *groups, uint32_t gcap,
-            fmgpu_block_status *status, int status_pitch, int nblk, int blk0, int ch0, int nch) {
+k_blocksync(const uint8_t *__restrict__ bits, uint32_t bits_cap, RdsState *st, unsigned long long *words,
+            fmgpu_rds_group *groups, uint32_t gcap, fmgpu_block_status *status, int status_pitch, int blk,
+            int ch0, int nch) {
   __shared__ uint32_t s_reg[32], s_nb[32], s_b0[32];
   const int c0 = ch0 + blockIdx.x * 32;
   const int nrows = min(32, ch0 + nch - c0);
@@ -2315,27 +2268,14 @@ k_blocksync(const uint8_t *__restrict__ bits, uint32_t bits_cap, const uint32_t 
   const uint32_t nb = s_nb[threadIdx.x];
   const uint32_t bit0 = s_b0[threadIdx.x];
   const unsigned long long *wrow = words + (size_t)c * bits_cap;
-  const uint32_t *bend = bit_end + (size_t)c * nblk;
   fmgpu_rds_group *gout = groups ? groups + (size_t)c * gcap : nullptr;
-  int blk = 0;
-  uint32_t before = s.n_groups;
+  const uint32_t before = s.n_groups;
   for (uint32_t i = bit0; i < nb; i++) {
-    while (blk < nblk - 1 && i >= bend[blk]) {
-      if (status) {
-        status[(size_t)c * status_pitch + blk].n_groups = (int)(s.n_groups - before);
-      }
-      before = s.n_groups;
-      blk++;
-    }
     const unsigned long long w = wrow[i];
-    rdsPushWord(s, (uint32_t)w & 0x3ffffffu, (uint32_t)(w >> 32), gout, gcap,
-                (uint32_t)(blk0 + blk));
+    rdsPushWord(s, (uint32_t)w & 0x3ffffffu, (uint32_t)(w >> 32), gout, gcap, (uint32_t)blk);
   }
   if (status) {
-    for (; blk < nblk; blk++) {
-      status[(size_t)c * status_pitch + blk].n_groups = (int)(s.n_groups - before);
-      before = s.n_groups;
-    }
+    status[(size_t)c * status_pitch].n_groups = (int)(s.n_groups - before);
   }
   // only the block-synchroniser fields changed
   RdsState *o = &st[c];
@@ -2536,14 +2476,12 @@ void launchCarryF2(float2 *buf, size_t pitch, int H, size_t n, int ch0, int nch,
 
 void launchDcBlock(const float2 *x1, size_t x1_pitch, const uint8_t *iq_u8, size_t iq_stride,
                    float2 *x2, size_t x2_pitch, DemodState *st, fmgpu_block_status *status,
-                   int status_pitch, int nblk, int blk_len, int n_total, int ch0, int nch, float a1,
-                   cudaStream_t stream) {
+                   int status_pitch, int n_total, int ch0, int nch, float a1, cudaStream_t stream) {
   constexpr size_t smem = 3 * 32 * (2 * LT + 4) * sizeof(float);
   static DeviceOnce attrs;  // per device: device_once.h
   attrs.run([] { return cudaFuncSetAttribute(k_dcblock, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); });
   k_dcblock<<<(nch + 31) / 32, 32, smem, stream>>>(x1, x1_pitch, iq_u8, iq_stride, x2, x2_pitch, st,
-                                               status, status_pitch, nblk, blk_len, n_total, ch0,
-                                               nch, a1);
+                                               status, status_pitch, n_total, ch0, nch, a1);
 }
 
 void launchDcBlockScan(const float2 *x1, size_t x1_pitch, float2 *x2, size_t x2_pitch, DemodState *st,
@@ -2659,23 +2597,22 @@ void launchFirReal(const FirRealJob &job, int nsig, int nch, const TapsParam &ta
 
 void launchStereo(const float *mpx, size_t mpx_pitch, const float *pilot, size_t pilot_pitch,
                   float *lraw, float *rraw, size_t lr_pitch, StereoState *st, const ChanParams *cp,
-                  fmgpu_block_status *status, int status_pitch, int nblk, int blk_len, int n_total,
-                  int ch0, int nch, const EngineConst &k, cudaStream_t stream) {
+                  fmgpu_block_status *status, int status_pitch, int n_total, int ch0, int nch,
+                  const EngineConst &k, cudaStream_t stream) {
   constexpr size_t smem = STEREO_TILES * STEREO_CPC * (STEREO_ST + 4) * sizeof(float);  // tiles of [CPC][ST + 4]
   static DeviceOnce attrs;  // per device: device_once.h
   attrs.run([] { return cudaFuncSetAttribute(k_stereo, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); });
   k_stereo<<<(nch + STEREO_CPC - 1) / STEREO_CPC, STEREO_THREADS, smem, stream>>>(mpx, mpx_pitch, pilot, pilot_pitch, lraw, rraw,
-                                                 lr_pitch, st, cp, status, status_pitch, nblk,
-                                                 blk_len, n_total, ch0, nch, k);
+                                                 lr_pitch, st, cp, status, status_pitch, n_total,
+                                                 ch0, nch, k);
 }
 
 void launchPrepare(AudioState *au, RdsState *rds, fmgpu_block_status *status, int status_pitch,
-                   int nblk, int blk_len, int n_total, int ch0, int nch, uint32_t aud_step,
-                   uint32_t rds_step, int do_audio, int do_mono, int do_rds, int first,
-                   RdsRsRef rr, cudaStream_t stream) {
-  k_prepare<<<(nch + 127) / 128, 128, 0, stream>>>(au, rds, status, status_pitch, nblk, blk_len,
-                                                  n_total, ch0, nch, aud_step, rds_step, do_audio,
-                                                  do_mono, do_rds, first, rr);
+                   int n_total, int ch0, int nch, uint32_t aud_step, uint32_t rds_step, int do_audio,
+                   int do_mono, int do_rds, int first, RdsRsRef rr, cudaStream_t stream) {
+  k_prepare<<<(nch + 127) / 128, 128, 0, stream>>>(au, rds, status, status_pitch, n_total, ch0, nch,
+                                                  aud_step, rds_step, do_audio, do_mono, do_rds, first,
+                                                  rr);
 }
 
 void launchCommit(AudioState *au, RdsState *rds, int ch0, int nch, int do_audio, int do_mono,
@@ -2685,19 +2622,14 @@ void launchCommit(AudioState *au, RdsState *rds, int ch0, int nch, int do_audio,
 
 void launchResample(const float *in0, const float *in1, size_t in_pitch, int in_off,
                     const float *hist, int hist_pitch, float *out, size_t acap, const float *bank,
-                    int sub_len, uint32_t step, const AudioState *au, int mono, int max_out,
-                    int ch0, int nch, cudaStream_t stream) {
+                    uint32_t step, const AudioState *au, int mono, int max_out, int ch0, int nch,
+                    cudaStream_t stream) {
   if (max_out <= 0) {
     return;
   }
   dim3 grid((max_out + 127) / 128, nch);
-  if (sub_len == AUD_RS_LEN) {
-    k_resample<AUD_RS_LEN><<<grid, 128, 32 * sub_len * sizeof(float), stream>>>(
-        in0, in1, in_pitch, in_off, hist, hist_pitch, out, acap, bank, sub_len, step, au, mono, ch0);
-  } else {
-    k_resample<0><<<grid, 128, 32 * sub_len * sizeof(float), stream>>>(
-        in0, in1, in_pitch, in_off, hist, hist_pitch, out, acap, bank, sub_len, step, au, mono, ch0);
-  }
+  k_resample<<<grid, 128, 32 * AUD_RS_LEN * sizeof(float), stream>>>(
+      in0, in1, in_pitch, in_off, hist, hist_pitch, out, acap, bank, step, au, mono, ch0);
 }
 
 void launchSaveTail(const float *src, size_t src_pitch, int src_off, float *hist, int hist_pitch,
@@ -2733,31 +2665,18 @@ void launchRdsResample(const float *mpx, size_t mpx_pitch, const float *hist, in
 }
 
 void launchRdsDemod(RdsState *st, float2 *ring, const float *lpf, const float *mf, const float *dmf,
-                    const float *r171, size_t r_pitch, uint8_t *bits_out, uint32_t bits_cap,
-                    uint32_t *bit_end, int ch0, int nch, const EngineConst &k, RdsRsRef rr,
-                    cudaStream_t stream) {
+                    const float *r171, size_t r_pitch, uint8_t *bits_out, uint32_t bits_cap, int ch0,
+                    int nch, const EngineConst &k, RdsRsRef rr, cudaStream_t stream) {
   constexpr size_t smem = 2 * 32 * (LT + 4) * sizeof(float);
   k_rds<<<(nch + RDS_CPC - 1) / RDS_CPC, 32, smem, stream>>>(r171, r_pitch, st, ring, lpf, mf, dmf, bits_out,
-                                              bits_cap, bit_end, ch0, nch, k, rr);
+                                              bits_cap, ch0, nch, k, rr);
 }
 
-void launchRds(const float *mpx, size_t mpx_pitch, const float *hist, int hist_pitch, RdsState *st,
-               float2 *ring, const float *bank, const float *lpf, const float *mf, const float *dmf,
-               float *r171, size_t r_pitch, int max_171, uint8_t *bits_out, uint32_t bits_cap,
-               uint32_t *bit_end, int ch0, int nch, const EngineConst &k, RdsRsRef rr,
-               cudaStream_t stream) {
-  launchRdsResample(mpx, mpx_pitch, hist, hist_pitch, rr, bank, r171, r_pitch, max_171, ch0, nch, k,
-                    stream);
-  launchRdsDemod(st, ring, lpf, mf, dmf, r171, r_pitch, bits_out, bits_cap, bit_end, ch0, nch, k, rr,
-                 stream);
-}
-
-void launchBlockSync(const uint8_t *bits, uint32_t bits_cap, const uint32_t *bit_end, RdsState *st,
-                     unsigned long long *words, fmgpu_rds_group *groups, uint32_t gcap,
-                     fmgpu_block_status *status, int status_pitch, int nblk, int blk0, int ch0,
-                     int nch, cudaStream_t stream) {
-  k_blocksync<<<(nch + 31) / 32, 128, 0, stream>>>(bits, bits_cap, bit_end, st, words, groups, gcap,
-                                                  status, status_pitch, nblk, blk0, ch0, nch);
+void launchBlockSync(const uint8_t *bits, uint32_t bits_cap, RdsState *st, unsigned long long *words,
+                     fmgpu_rds_group *groups, uint32_t gcap, fmgpu_block_status *status,
+                     int status_pitch, int blk, int ch0, int nch, cudaStream_t stream) {
+  k_blocksync<<<(nch + 31) / 32, 128, 0, stream>>>(bits, bits_cap, st, words, groups, gcap, status,
+                                                  status_pitch, blk, ch0, nch);
 }
 
 void launchSigLevel(const uint8_t *iq, size_t iq_stride, fmgpu_level_sums *sums, int nblk,

@@ -77,8 +77,7 @@ void launchSaveTail(const float *src, size_t src_pitch, int src_off, float *hist
                     int H, long n, int ch0, int nch, cudaStream_t stream);
 void launchDcBlock(const float2 *x1, size_t x1_pitch, const uint8_t *iq_u8, size_t iq_stride,
                    float2 *x2, size_t x2_pitch, DemodState *st, fmgpu_block_status *status,
-                   int status_pitch, int nblk, int blk_len, int n_total, int ch0, int nch, float a1,
-                   cudaStream_t stream);
+                   int status_pitch, int n_total, int ch0, int nch, float a1, cudaStream_t stream);
 // the I/Q DC blockers of one logical block as a warp-shuffle scan (float input; fast arithmetic)
 void launchDcBlockScan(const float2 *x1, size_t x1_pitch, float2 *x2, size_t x2_pitch, DemodState *st,
                        fmgpu_block_status *status, int status_pitch, int n_total, int ch0, int nch,
@@ -94,18 +93,20 @@ void launchFirReal(const FirRealJob &job, int nsig, int nch, const TapsParam &ta
                    cudaStream_t stream);
 void launchStereo(const float *mpx, size_t mpx_pitch, const float *pilot, size_t pilot_pitch,
                   float *lraw, float *rraw, size_t lr_pitch, StereoState *st, const ChanParams *cp,
-                  fmgpu_block_status *status, int status_pitch, int nblk, int blk_len, int n_total,
-                  int ch0, int nch, const EngineConst &k, cudaStream_t stream);
+                  fmgpu_block_status *status, int status_pitch, int n_total, int ch0, int nch,
+                  const EngineConst &k, cudaStream_t stream);
+// k_prepare's RDS work (do_rds): the 171 kHz resampler's bookkeeping (the resampler stage), or, on the
+// first block of a call, zeroing the call's group / bit counters (the demodulator stage)
+enum { PREPARE_RDS_NONE = 0, PREPARE_RDS_RESAMPLER = 1, PREPARE_RDS_COUNTERS = 2 };
 void launchPrepare(AudioState *au, RdsState *rds, fmgpu_block_status *status, int status_pitch,
-                   int nblk, int blk_len, int n_total, int ch0, int nch, uint32_t aud_step,
-                   uint32_t rds_step, int do_audio, int do_mono, int do_rds, int first,
-                   RdsRsRef rr, cudaStream_t stream);
+                   int n_total, int ch0, int nch, uint32_t aud_step, uint32_t rds_step, int do_audio,
+                   int do_mono, int do_rds, int first, RdsRsRef rr, cudaStream_t stream);
 void launchCommit(AudioState *au, RdsState *rds, int ch0, int nch, int do_audio, int do_mono,
                   int do_rds, RdsRsRef rr, cudaStream_t stream);
 void launchResample(const float *in0, const float *in1, size_t in_pitch, int in_off,
                     const float *hist, int hist_pitch, float *out, size_t acap, const float *bank,
-                    int sub_len, uint32_t step, const AudioState *au, int mono, int max_out,
-                    int ch0, int nch, cudaStream_t stream);
+                    uint32_t step, const AudioState *au, int mono, int max_out, int ch0, int nch,
+                    cudaStream_t stream);
 void launchAudioIir(float *audio, size_t acap, AudioState *au, const ChanParams *cp, int ch0,
                     int nch, float dc_a1, int mono, int clamp, int mono_dup, cudaStream_t stream);
 // de-emphasis + DC blocker of the stereo rows as a warp-shuffle affine scan (fast arithmetic)
@@ -120,18 +121,12 @@ void launchRdsResample(const float *mpx, size_t mpx_pitch, const float *hist, in
                        RdsRsRef rr, const float *bank, float *r171, size_t r_pitch,
                        int max_171, int ch0, int nch, const EngineConst &k, cudaStream_t stream);
 void launchRdsDemod(RdsState *st, float2 *ring, const float *lpf, const float *mf, const float *dmf,
-                    const float *r171, size_t r_pitch, uint8_t *bits_out, uint32_t bits_cap,
-                    uint32_t *bit_end, int ch0, int nch, const EngineConst &k, RdsRsRef rr,
-                    cudaStream_t stream);
-void launchRds(const float *mpx, size_t mpx_pitch, const float *hist, int hist_pitch, RdsState *st,
-               float2 *ring, const float *bank, const float *lpf, const float *mf, const float *dmf,
-               float *r171, size_t r_pitch, int max_171, uint8_t *bits_out, uint32_t bits_cap,
-               uint32_t *bit_end, int ch0, int nch, const EngineConst &k, RdsRsRef rr,
-               cudaStream_t stream);
-void launchBlockSync(const uint8_t *bits, uint32_t bits_cap, const uint32_t *bit_end, RdsState *st,
-                     unsigned long long *words, fmgpu_rds_group *groups, uint32_t gcap,
-                     fmgpu_block_status *status, int status_pitch, int nblk, int blk0, int ch0,
-                     int nch, cudaStream_t stream);
+                    const float *r171, size_t r_pitch, uint8_t *bits_out, uint32_t bits_cap, int ch0,
+                    int nch, const EngineConst &k, RdsRsRef rr, cudaStream_t stream);
+// blk: the block number the groups found are tagged with
+void launchBlockSync(const uint8_t *bits, uint32_t bits_cap, RdsState *st, unsigned long long *words,
+                     fmgpu_rds_group *groups, uint32_t gcap, fmgpu_block_status *status,
+                     int status_pitch, int blk, int ch0, int nch, cudaStream_t stream);
 
 void launchSigLevel(const uint8_t *iq, size_t iq_stride, fmgpu_level_sums *sums, int nblk,
                     long samples_per_block, int ch0, int nch, cudaStream_t stream);

@@ -210,6 +210,39 @@ def test_rds_decoder_chunks_and_reset(orc_fm):
     eng.close()
 
 
+def test_stage_calls_chained_on_one_engine():
+    """Every stage-level call carries only its own stage's halos and state: the five calls chained block
+    after block on ONE engine channel give, bit for bit, what each gives on an engine of its own."""
+    sizes = RAGGED + [16384, 12001, 16384, 9000] * 6
+    iq = orc.config1_signal(fs_iq=2_048_000, seed=5).generate(sum(sizes) * 8)
+    cfg = fm.make_config(iq_rate=2_048_000, decimation=8, block_samples=16384, max_blocks=1)
+    shared = fm.Engine(cfg, 1, 0)
+    own = [fm.Engine(cfg, 1, 0) for _ in range(5)]
+
+    def chain(dec, dem, ste, afp, rds, chunk, n, cap):
+        x = dec.executeComplex(chunk, n)
+        mpx, mono = dem.processSplitComplex(x, want_mono=True)
+        left, right = ste.processAudio(mpx)
+        al, ar = afp.afpost(left, right, cap)
+        return (x, mpx, mono, left, right, al, ar), rds.rds(mpx, cap=64)
+
+    pos = n_groups = 0
+    for i, n in enumerate(sizes):
+        chunk = iq[2 * 8 * pos:2 * 8 * (pos + n)]
+        cap = n if i % 4 else max(2, n // 10)   # a short capacity leaves part of the L/R input unused
+        got, g_got = chain(*[shared] * 5, chunk, n, cap)
+        ref, g_ref = chain(*own, chunk, n, cap)
+        assert got[0].size == n and got[1].size == n
+        for k, (a, b) in enumerate(zip(got, ref)):
+            assert a.size == b.size and np.array_equal(a, b), (i, n, k)
+        assert groups_equal(g_got, g_ref), i
+        n_groups += len(g_ref)
+        pos += n
+    assert n_groups >= 3
+    for e in (shared, *own):
+        e.close()
+
+
 def test_null_and_empty_arguments_return_zero():
     eng = fm.Engine(fm.make_config(iq_rate=256000, decimation=1, max_blocks=1), 1, 0)
     L = eng.L
