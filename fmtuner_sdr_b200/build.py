@@ -10,7 +10,7 @@ LIB = os.path.join(HERE, "libfmgpu.so")
 DROPIN_LIB = os.path.join(HERE, "libfmgpu_dropin.so")
 SOURCES = ["kernels.cu", "engine.cu", "decim_tc.cu", "fir_tc.cu", "channelizer.cu", "synth.cu", "probe.cu", "design.cpp",
            "xdr_format.cpp"]
-HEADERS = ["engine.h", "kernels.h", "tc_common.cuh", "device_once.h", "design.h", "fm_math.h", os.path.join("..", "..", "include", "fmgpu.h")]
+HEADERS = ["engine.h", "kernels.h", "tc_common.cuh", "device_once.h", "cuda_handle.h", "design.h", "fm_math.h", os.path.join("..", "..", "include", "fmgpu.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

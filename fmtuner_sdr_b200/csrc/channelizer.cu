@@ -46,6 +46,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/fmgpu.h"
+#include "cuda_handle.h"
 #include "design.h"
 #include "device_once.h"
 
@@ -55,15 +56,15 @@ struct fmgpu_channelizer {
   double firstHz = 0.0, spacingHz = 0.0;
   std::vector<float> taps;         // prototype h[n]
   std::vector<double> nuD;         // frac(nu_k * D): phase advance per output, in turns
-  float2 *dW = nullptr;            // [L][Cpad]
-  double *dNuD = nullptr;          // [Cpad]
-  uint8_t *dHist = nullptr;        // last L-1 input samples (u8 pairs) of the previous call
+  fmgpu::DeviceArray<float2> dW;      // [L][Cpad]
+  fmgpu::DeviceArray<double> dNuD;    // [Cpad]
+  fmgpu::DeviceArray<uint8_t> dHist;  // last L-1 input samples (u8 pairs) of the previous call
   // polyphase form (uniform grid): nu_k = (k + c0) / P
   bool polyphase = false;
   int P = 0, rotPeriod = 0;        // rotation table period (P * T, c0 * T integer)
-  float *dTaps = nullptr;          // [L]
-  float2 *dRot = nullptr;          // [rotPeriod] exp(-j 2 pi c0 s / P)
-  float2 *dTw = nullptr;           // [P] exp(-j 2 pi i / P)
+  fmgpu::DeviceArray<float> dTaps;    // [L]
+  fmgpu::DeviceArray<float2> dRot;    // [rotPeriod] exp(-j 2 pi c0 s / P)
+  fmgpu::DeviceArray<float2> dTw;     // [P] exp(-j 2 pi i / P)
   unsigned long long outCount = 0; // outputs produced so far (m of the next output)
   long histValid = 0;              // how many of the carried samples are real input (rest = 0)
   std::string lastError;
@@ -331,23 +332,22 @@ int fmgpu_channelizer_create(int device, int wide_rate, int decimation, int n_ch
   }
   bool ok = cudaSetDevice(device) == cudaSuccess;
   if (z->polyphase) {
-    ok = ok && cudaMalloc(&z->dTaps, z->taps.size() * sizeof(float)) == cudaSuccess;
-    ok = ok && cudaMalloc(&z->dRot, rotTab.size() * sizeof(float2)) == cudaSuccess;
-    ok = ok && cudaMalloc(&z->dTw, twTab.size() * sizeof(float2)) == cudaSuccess;
+    ok = ok && fmgpu::devAlloc(&z->dTaps, z->taps.size()) == cudaSuccess;
+    ok = ok && fmgpu::devAlloc(&z->dRot, rotTab.size()) == cudaSuccess;
+    ok = ok && fmgpu::devAlloc(&z->dTw, twTab.size()) == cudaSuccess;
     ok = ok && cudaMemcpy(z->dTaps, z->taps.data(), z->taps.size() * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
     ok = ok && cudaMemcpy(z->dRot, rotTab.data(), rotTab.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
     ok = ok && cudaMemcpy(z->dTw, twTab.data(), twTab.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
   }
-  ok = ok && cudaMalloc(&z->dW, W.size() * sizeof(float2)) == cudaSuccess;
-  ok = ok && cudaMalloc(&z->dNuD, z->Cpad * sizeof(double)) == cudaSuccess;
-  ok = ok && cudaMalloc(&z->dHist, static_cast<size_t>(z->L) * 2) == cudaSuccess;
+  ok = ok && fmgpu::devAlloc(&z->dW, W.size()) == cudaSuccess;
+  ok = ok && fmgpu::devAlloc(&z->dNuD, z->Cpad) == cudaSuccess;
+  // the input before the first call is ZERO: no byte maps to 0.0, so the kernel clears the
+  // part of the window older than histValid samples
+  ok = ok && fmgpu::devAlloc(&z->dHist, static_cast<size_t>(z->L) * 2) == cudaSuccess;
   ok = ok && cudaMemcpy(z->dW, W.data(), W.size() * sizeof(float2), cudaMemcpyHostToDevice) ==
                  cudaSuccess;
   ok = ok && cudaMemcpy(z->dNuD, z->nuD.data(), z->Cpad * sizeof(double), cudaMemcpyHostToDevice) ==
                  cudaSuccess;
-  // the input before the first call is ZERO: no byte maps to 0.0, so the kernel clears the
-  // part of the window older than histValid samples
-  ok = ok && cudaMemset(z->dHist, 0, static_cast<size_t>(z->L) * 2) == cudaSuccess;
   if (!ok) {
     cudaGetLastError();
     fmgpu_channelizer_destroy(z);
@@ -363,13 +363,7 @@ void fmgpu_channelizer_destroy(fmgpu_channelizer *z) {
   }
   cudaSetDevice(z->device);
   cudaDeviceSynchronize();
-  cudaFree(z->dW);
-  cudaFree(z->dNuD);
-  cudaFree(z->dHist);
-  cudaFree(z->dTaps);
-  cudaFree(z->dRot);
-  cudaFree(z->dTw);
-  delete z;
+  delete z;  // the handles free the device buffers
 }
 
 int fmgpu_channelizer_output_rate(const fmgpu_channelizer *z) { return z ? z->wideRate / z->D : 0; }

@@ -16,6 +16,7 @@
 #include <tuple>
 #include <vector>
 
+#include "cuda_handle.h"
 #include "design.h"
 #include "kernels.h"
 
@@ -62,10 +63,10 @@ struct fmgpu_engine {
   int demodMode = 0;
   bool decimTcOk = false, pilTcOk = false, audTcOk = false;
   FirTcTables pilTc{}, audTc{};
-  uint8_t *dPilB = nullptr, *dAudB = nullptr;
+  DeviceArray<uint8_t> dPilB, dAudB;
   int smCount = 148;
-  uint8_t *dDecB = nullptr;
-  int32_t *dDecOffs = nullptr;
+  DeviceArray<uint8_t> dDecB;
+  DeviceArray<int32_t> dDecOffs;
   std::vector<float> pilTaps, audTaps, rdsLpf;
   fmdesign::ResamplerDesign audRs, rdsRs;
   fmdesign::SymSyncDesign ss;
@@ -77,7 +78,7 @@ struct fmgpu_engine {
     int lp;
     // tensor-core form (fir_tc.cu): integer taps' digits as a B image on the device
     FirTcTables tc{};
-    uint8_t *dB = nullptr;
+    DeviceArray<uint8_t> dB;
     bool tcOk = false;
   };
   std::vector<ChanFilter> filters;
@@ -86,29 +87,32 @@ struct fmgpu_engine {
   bool paramsDirty = true;
 
   // device memory
-  uint8_t *dIq = nullptr, *dHistIq = nullptr;
-  int *dHistValid = nullptr;
-  float2 *dX1 = nullptr, *dX2 = nullptr, *dY = nullptr, *dRing = nullptr;
-  float *dR171 = nullptr;  // MPX resampled to 171 kHz (RDS branch): two buffers, by block parity
+  DeviceArray<uint8_t> dIq, dHistIq;
+  DeviceArray<int> dHistValid;
+  DeviceArray<float2> dX1, dX2, dY, dRing;
+  DeviceArray<float> dR171;  // MPX resampled to 171 kHz (RDS branch): two buffers, by block parity
   size_t r171Pitch = 0;
-  float *dMpx = nullptr, *dPilot = nullptr, *dLraw = nullptr, *dRraw = nullptr, *dLf = nullptr,
-        *dRf = nullptr, *dAudio = nullptr, *dRdsHist = nullptr, *dMonoHist = nullptr;
-  float *dChanTaps = nullptr, *dChanScale = nullptr, *dAudBank = nullptr, *dRdsBank = nullptr,
-        *dRdsLpf = nullptr, *dMf = nullptr, *dDmf = nullptr;
-  int *dChanLp = nullptr;
-  ChanParams *dParams = nullptr;
-  DemodState *dDemod = nullptr;
-  StereoState *dStereo = nullptr;
-  AudioState *dAudioSt = nullptr;
-  RdsState *dRds = nullptr;
-  RdsRsState *dRdsRs = nullptr;  // 171 kHz resampler bookkeeping (apart from RdsState, see engine.h)
-  fmgpu_rds_group *dGroups = nullptr;
-  fmgpu_block_status *dStatus = nullptr;
-  uint32_t *dNAudio = nullptr, *dNGroups = nullptr;
-  uint8_t *dBits = nullptr;
-  unsigned long long *dWords = nullptr;
+  DeviceArray<float> dMpx, dPilot, dLraw, dRraw, dLf, dRf, dRdsHist, dMonoHist;
+  DeviceArray<float> dChanTaps, dChanScale, dAudBank, dRdsBank, dRdsLpf, dMf, dDmf;
+  DeviceArray<int> dChanLp;
+  DeviceArray<ChanParams> dParams;
+  DeviceArray<DemodState> dDemod;
+  DeviceArray<StereoState> dStereo;
+  DeviceArray<AudioState> dAudioSt;
+  DeviceArray<RdsState> dRds;
+  DeviceArray<RdsRsState> dRdsRs;  // 171 kHz resampler bookkeeping (apart from RdsState, see engine.h)
+  // device result buffers, two sets: consecutive host submissions alternate between them; the
+  // batched and stage-level calls use set 0 when the caller gives no buffers of its own
+  struct Results {
+    DeviceArray<float> audio;               // [C][2][acap]
+    DeviceArray<fmgpu_rds_group> groups;    // [C][gcap]
+    DeviceArray<fmgpu_block_status> status; // [C][maxBlocks]
+    DeviceArray<uint32_t> nAudio, nGroups;  // [C]
+  } res[2];
+  DeviceArray<uint8_t> dBits;
+  DeviceArray<unsigned long long> dWords;
   size_t x2Pitch = 0, yPitch = 0, mpxPitch = 0, lrPitch = 0, lfPitch = 0;
-  cudaStream_t stream = nullptr;  // stage-level (single-channel) entry points, resets, reads
+  Stream stream;  // stage-level (single-channel) entry points, resets, reads
 
   // ---- block pipeline ---------------------------------------------------------------------
   // The batched path runs ONE LOGICAL BLOCK AT A TIME through per-stage streams: every stage
@@ -128,11 +132,11 @@ struct fmgpu_engine {
     ST_D2H, ST_RDSRS /* MPX -> 171 kHz, one block ahead of the RDS demodulator */, ST_COUNT
   };
   struct Pipe {
-    cudaStream_t st[ST_COUNT] = {};   // the streams as created
+    Stream st[ST_COUNT];              // the streams as created
     cudaStream_t run[ST_COUNT] = {};  // the streams in use (all the same one when serialStages)
-    std::vector<cudaEvent_t> done[ST_COUNT];  // ring of ER events per stage
-    cudaEvent_t callDone = nullptr;           // everything of the last batch call of this pipe
-    cudaEvent_t hostDone[2] = {};             // per host ticket: results are in the host buffers
+    std::vector<Event> done[ST_COUNT];  // ring of ER events per stage
+    Event callDone;                     // everything of the last batch call of this pipe
+    Event hostDone[2];                  // per host ticket: results are in the host buffers
   };
   static constexpr int kMaxGroups = 2;        // channel ranges with their own pipe (streams)
   int nGroups = 1;
@@ -143,7 +147,7 @@ struct fmgpu_engine {
   bool headFresh = true; // the halo in front of slot 0 is already in place (start, reset, realign)
   bool asyncPending = false;
   bool serialStages = false;  // measurement aid: every stage on ONE stream, no overlap
-  cudaEvent_t evStart = nullptr;
+  Event evStart;
   // streaming host path: two tickets in flight (submit k+1 before waiting for k)
   struct HostTicket {
     bool pending = false;
@@ -152,11 +156,6 @@ struct fmgpu_engine {
     bool clampGroups = false;
   } tickets[2];
   int nextTicket = 0;
-  // second set of device result buffers: consecutive host submissions alternate between the sets
-  float *dAudio2 = nullptr;
-  fmgpu_rds_group *dGroups2 = nullptr;
-  fmgpu_block_status *dStatus2 = nullptr;
-  uint32_t *dNAudio2 = nullptr, *dNGroups2 = nullptr;
   uint64_t lastSeq0 = 0;  // first block of the last batch call (debug reads)
   int lastBlocks = 0;
 
@@ -165,8 +164,12 @@ struct fmgpu_engine {
   std::string lastError;
 
   bool timing = false;
-  std::vector<std::tuple<const char *, cudaEvent_t, cudaEvent_t>> spans;
-  std::vector<int> spanGroup;   // pipeline group of each span
+  struct SpanRecord {
+    const char *name;
+    int group;  // pipeline group
+    Event start, end;
+  };
+  std::vector<SpanRecord> spans;
   int curGroup = 0;
   bool timeline = false;        // keep the raw spans (fmgpu_debug_timeline) instead of merging
   std::vector<std::pair<const char *, float>> lastTimes;
@@ -178,18 +181,11 @@ namespace {
   do {                                                                                   \
     cudaError_t err__ = (expr);                                                          \
     if (err__ != cudaSuccess) {                                                          \
+      cudaGetLastError(); /* reported here: not left for the next call to find */       \
       e->lastError = std::string(#expr) + ": " + cudaGetErrorString(err__);              \
       return (err__ == cudaErrorMemoryAllocation) ? FMGPU_ENOMEM : FMGPU_ENODEV;         \
     }                                                                                    \
   } while (0)
-
-template <typename T> cudaError_t devAlloc(T **p, size_t count) {
-  cudaError_t err = cudaMalloc(reinterpret_cast<void **>(p), std::max<size_t>(1, count) * sizeof(T));
-  if (err == cudaSuccess) {
-    err = cudaMemset(*p, 0, std::max<size_t>(1, count) * sizeof(T));
-  }
-  return err;
-}
 
 TapsParam padFront(const std::vector<float> &hrev, int lp) {
   TapsParam t{};
@@ -260,6 +256,8 @@ RdsState defaultRds(const EngineConst &k) {
   return s;
 }
 
+// The channel filter table's slot of a filter design (added on first use), or a negative FMGPU_E*
+// code with lastError set.
 int filterSlot(fmgpu_engine *e, unsigned len, float cutoff, float atten) {
   const auto key = std::make_tuple(len, cutoff, atten);
   auto it = e->filterIndex.find(key);
@@ -267,7 +265,8 @@ int filterSlot(fmgpu_engine *e, unsigned len, float cutoff, float atten) {
     return it->second;
   }
   if (static_cast<int>(e->filters.size()) >= MAX_CHAN_FILTERS) {
-    return -1;
+    e->lastError = "channel filter table full";
+    return FMGPU_ENOMEM;
   }
   fmgpu_engine::ChanFilter f;
   f.taps = fmdesign::kaiserLowpass(len, cutoff, atten, 0.0f);
@@ -279,19 +278,19 @@ int filterSlot(fmgpu_engine *e, unsigned len, float cutoff, float atten) {
   for (unsigned i = 0; i < len; i++) {
     row[CHAN_TAPS_PITCH - len + i] = hrev[i];
   }
-  cudaMemcpy(e->dChanTaps + static_cast<size_t>(slot) * CHAN_TAPS_PITCH, row.data(),
-             CHAN_TAPS_PITCH * sizeof(float), cudaMemcpyHostToDevice);
-  cudaMemcpy(e->dChanLp + slot, &f.lp, sizeof(int), cudaMemcpyHostToDevice);
-  cudaMemcpy(e->dChanScale + slot, &f.scale, sizeof(float), cudaMemcpyHostToDevice);
+  CK(cudaMemcpy(e->dChanTaps + static_cast<size_t>(slot) * CHAN_TAPS_PITCH, row.data(),
+                CHAN_TAPS_PITCH * sizeof(float), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(e->dChanLp + slot, &f.lp, sizeof(int), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(e->dChanScale + slot, &f.scale, sizeof(float), cudaMemcpyHostToDevice));
   {
     const float *h = row.data() + (CHAN_TAPS_PITCH - f.lp);   // the padded taps as k_chanfir reads them
     if (chanTcSupported(h, f.lp, H_X2)) {
       firTcBuildTables(h, f.lp, &f.tc);
-      void *d = nullptr;
-      if (cudaMalloc(&d, f.tc.b_image.size()) == cudaSuccess &&
-          cudaMemcpy(d, f.tc.b_image.data(), f.tc.b_image.size(), cudaMemcpyHostToDevice) == cudaSuccess) {
-        f.dB = static_cast<uint8_t *>(d);
+      if (devAlloc(&f.dB, f.tc.b_image.size()) == cudaSuccess &&
+          cudaMemcpy(f.dB, f.tc.b_image.data(), f.tc.b_image.size(), cudaMemcpyHostToDevice) == cudaSuccess) {
         f.tcOk = true;
+      } else {
+        cudaGetLastError();  // no tensor-core image: the three-kernel path runs this filter
       }
     }
   }
@@ -346,14 +345,15 @@ template <typename F> int forChannels(fmgpu_engine *e, int channel, F &&f) {
 struct Span {
   fmgpu_engine *e;
   cudaStream_t s;
-  cudaEvent_t a = nullptr, b = nullptr;
+  cudaEvent_t b = nullptr;
   Span(fmgpu_engine *e_, const char *name, cudaStream_t s_) : e(e_), s(s_) {
     if (e->timing) {
-      cudaEventCreate(&a);
-      cudaEventCreate(&b);
-      cudaEventRecord(a, s);
-      e->spans.emplace_back(name, a, b);
-      e->spanGroup.push_back(e->curGroup);
+      e->spans.push_back({name, e->curGroup, {}, {}});
+      fmgpu_engine::SpanRecord &r = e->spans.back();
+      cudaEventCreate(r.start.out());
+      cudaEventCreate(r.end.out());
+      cudaEventRecord(r.start, s);
+      b = r.end;
     }
   }
   ~Span() {
@@ -365,14 +365,14 @@ struct Span {
 
 // zero a [C][pitch] region [0, count) of channel c (or all)
 template <typename T>
-void zeroPrefix(T *buf, size_t pitch, size_t count, int lo, int hi, cudaStream_t s) {
+void zeroPrefix(const DeviceArray<T> &buf, size_t pitch, size_t count, int lo, int hi, cudaStream_t s) {
   cudaMemset2DAsync(buf + static_cast<size_t>(lo) * pitch, pitch * sizeof(T), 0, count * sizeof(T),
                     static_cast<size_t>(hi - lo), s);
 }
 
 // One strided copy of the same `bytes` to `field` of every state struct of channels [lo, hi).
 template <typename S>
-int fillStateField(fmgpu_engine *e, S *base, size_t fieldOffset, const void *value,
+int fillStateField(fmgpu_engine *e, const DeviceArray<S> &base, size_t fieldOffset, const void *value,
                           size_t bytes, int lo, int hi) {
   const size_t cnt = static_cast<size_t>(hi - lo);
   std::vector<uint8_t> rows(cnt * bytes);
@@ -442,13 +442,17 @@ struct BatchOut {
   fmgpu_block_status *status = nullptr;  // [C][n_blocks]
 };
 
-// the engine's own result buffers (the stage-level entry points copy from them)
-BatchOut engineOut(const fmgpu_engine *e) {
+// the engine's own result buffers of set `set` (the stage-level entry points copy from set 0)
+BatchOut engineOut(const fmgpu_engine *e, int set = 0) {
+  const fmgpu_engine::Results &r = e->res[set];
   BatchOut out;
-  out.audio = e->dAudio;
+  out.audio = r.audio;
   out.acap = e->acap;
-  out.groups = e->dGroups;
+  out.nAudio = r.nAudio;
+  out.groups = r.groups;
   out.gcap = static_cast<uint32_t>(e->gcap);
+  out.nGroups = r.nGroups;
+  out.status = r.status;
   return out;
 }
 
@@ -742,23 +746,20 @@ void collectTimes(fmgpu_engine *e) {
   e->lastTimes.clear();
   for (auto &sp : e->spans) {
     float ms = 0.0f;
-    cudaEventSynchronize(std::get<2>(sp));
-    cudaEventElapsedTime(&ms, std::get<1>(sp), std::get<2>(sp));
+    cudaEventSynchronize(sp.end);
+    cudaEventElapsedTime(&ms, sp.start, sp.end);
     bool merged = false;
     for (auto &t : e->lastTimes) {
-      if (std::strcmp(t.first, std::get<0>(sp)) == 0) {
+      if (std::strcmp(t.first, sp.name) == 0) {
         t.second += ms;
         merged = true;
       }
     }
     if (!merged) {
-      e->lastTimes.emplace_back(std::get<0>(sp), ms);
+      e->lastTimes.emplace_back(sp.name, ms);
     }
-    cudaEventDestroy(std::get<1>(sp));
-    cudaEventDestroy(std::get<2>(sp));
   }
   e->spans.clear();
-  e->spanGroup.clear();
 }
 
 // ---------------------------------------------------------------------------
@@ -814,7 +815,7 @@ void launchBlock(fmgpu_engine *e, fmgpu_engine::Pipe &P, int ch0, int nch, uint6
   // slot 0 brings the tail of slot K-1 in front of it
   const BlockRef blk{ch0, nch, static_cast<size_t>(slot) * N, N, out.status ? out.status + b : nullptr, nb,
                      (slot == 0) && !e->headFresh};
-  auto ev = [&](int st, uint64_t qq) { return P.done[st][qq % static_cast<uint64_t>(e->ER)]; };
+  auto ev = [&](int st, uint64_t qq) -> cudaEvent_t { return P.done[st][qq % static_cast<uint64_t>(e->ER)]; };
   // producers: stages of THIS block whose output the stage reads; overwritten: consumer stages
   // of the buffers it writes, which must have finished block q - K (same ring slot)
   auto need = [&](int st, std::initializer_list<int> producers, std::initializer_list<int> readers) {
@@ -1064,15 +1065,16 @@ int runBatch(fmgpu_engine *e, const uint8_t *iq_dev, size_t stride, int n_blocks
   if (rc != FMGPU_OK) {
     return rc;
   }
+  const BatchOut own = engineOut(e);
   BatchOut out;
-  out.status = status_dev ? status_dev : e->dStatus;
-  out.groups = groups_dev ? groups_dev : e->dGroups;
-  out.gcap = static_cast<uint32_t>(groups_dev ? group_cap : e->gcap);
-  out.nAudio = n_audio_dev ? n_audio_dev : e->dNAudio;
-  out.nGroups = n_groups_dev ? n_groups_dev : e->dNGroups;
+  out.status = status_dev ? status_dev : own.status;
+  out.groups = groups_dev ? groups_dev : own.groups;
+  out.gcap = groups_dev ? static_cast<uint32_t>(group_cap) : own.gcap;
+  out.nAudio = n_audio_dev ? n_audio_dev : own.nAudio;
+  out.nGroups = n_groups_dev ? n_groups_dev : own.nGroups;
   // audio is produced straight into the caller's buffer when one is given
-  out.audio = audio_dev ? audio_dev : e->dAudio;
-  out.acap = audio_dev ? audio_cap : e->acap;
+  out.audio = audio_dev ? audio_dev : own.audio;
+  out.acap = audio_dev ? audio_cap : own.acap;
   if (cf32) {
     return queueBlocks(e, nullptr, nullptr, 0, n_blocks, out, s, join, reinterpret_cast<const float2 *>(iq_dev),
                        stride / sizeof(float2));
@@ -1230,6 +1232,7 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
   do {                                                                             \
     cudaError_t err__ = (expr);                                                    \
     if (err__ != cudaSuccess) {                                                    \
+      cudaGetLastError();                                                          \
       e->lastError = std::string(#expr) + ": " + cudaGetErrorString(err__);        \
       return fail(err__ == cudaErrorMemoryAllocation ? FMGPU_ENOMEM : FMGPU_ENODEV); \
     }                                                                              \
@@ -1278,10 +1281,10 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
   e->acap = static_cast<size_t>((static_cast<double>(e->nmax) * 16777216.0) / e->k.aud_step) + 8;
   e->gcap = e->nmax * 12 / static_cast<size_t>(std::max(1, e->fs)) + 8;  // 11.4 groups/s
   e->bitsCap = e->nmax / 100 + 64;
-  CKC(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
+  CKC(cudaStreamCreateWithFlags(e->stream.out(), cudaStreamNonBlocking));
   int prLo = 0, prHi = 0;
   CKC(cudaDeviceGetStreamPriorityRange(&prLo, &prHi));  // prHi = numerically smallest = highest
-  CKC(cudaEventCreateWithFlags(&e->evStart, cudaEventDisableTiming));
+  CKC(cudaEventCreateWithFlags(e->evStart.out(), cudaEventDisableTiming));
   for (auto &P : e->pipes) {
     for (int st = 0; st < fmgpu_engine::ST_COUNT; st++) {
       // The serial one-lane-per-channel stages are the slowest per block: they get the high
@@ -1291,16 +1294,16 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
                         st == fmgpu_engine::ST_STEREO || st == fmgpu_engine::ST_RDS ||
                         st == fmgpu_engine::ST_AF;
       const int prio = lane ? prHi : prLo;
-      CKC(cudaStreamCreateWithPriority(&P.st[st], cudaStreamNonBlocking, prio));
+      CKC(cudaStreamCreateWithPriority(P.st[st].out(), cudaStreamNonBlocking, prio));
       P.run[st] = P.st[st];
       P.done[st].resize(static_cast<size_t>(e->ER));
       for (auto &ev : P.done[st]) {
-        CKC(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        CKC(cudaEventCreateWithFlags(ev.out(), cudaEventDisableTiming));
       }
     }
-    CKC(cudaEventCreateWithFlags(&P.callDone, cudaEventDisableTiming));
-    CKC(cudaEventCreateWithFlags(&P.hostDone[0], cudaEventDisableTiming));
-    CKC(cudaEventCreateWithFlags(&P.hostDone[1], cudaEventDisableTiming));
+    CKC(cudaEventCreateWithFlags(P.callDone.out(), cudaEventDisableTiming));
+    CKC(cudaEventCreateWithFlags(P.hostDone[0].out(), cudaEventDisableTiming));
+    CKC(cudaEventCreateWithFlags(P.hostDone[1].out(), cudaEventDisableTiming));
   }
   CKC(initRdsTables());
   CKC(devAlloc(&e->dIq, C * e->iqPitch));
@@ -1356,11 +1359,9 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
   CKC(devAlloc(&e->dRraw, C * e->lrPitch));
   CKC(devAlloc(&e->dLf, C * e->lfPitch));
   CKC(devAlloc(&e->dRf, C * e->lfPitch));
-  CKC(devAlloc(&e->dAudio, C * 2 * e->acap));
   e->r171Pitch = roundUp(static_cast<size_t>(max171(e, static_cast<int>(e->nmax))) + 32, 32);
   CKC(devAlloc(&e->dR171, 2 * C * e->r171Pitch));
   CKC(devAlloc(&e->dRdsRs, C));
-  CKC(cudaMemset(e->dRdsRs, 0, C * sizeof(RdsRsState)));
   CKC(devAlloc(&e->dRing, C * RDS_RING));
   CKC(devAlloc(&e->dRdsHist, C * 32));
   CKC(devAlloc(&e->dMonoHist, C * 32));
@@ -1377,15 +1378,13 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
   CKC(devAlloc(&e->dStereo, C));
   CKC(devAlloc(&e->dAudioSt, C));
   CKC(devAlloc(&e->dRds, C));
-  CKC(devAlloc(&e->dGroups, C * e->gcap));
-  CKC(devAlloc(&e->dStatus, C * static_cast<size_t>(e->maxBlocks)));
-  CKC(devAlloc(&e->dNAudio, C));
-  CKC(devAlloc(&e->dNGroups, C));
-  CKC(devAlloc(&e->dAudio2, C * 2 * e->acap));
-  CKC(devAlloc(&e->dGroups2, C * e->gcap));
-  CKC(devAlloc(&e->dStatus2, C * static_cast<size_t>(e->maxBlocks)));
-  CKC(devAlloc(&e->dNAudio2, C));
-  CKC(devAlloc(&e->dNGroups2, C));
+  for (auto &r : e->res) {
+    CKC(devAlloc(&r.audio, C * 2 * e->acap));
+    CKC(devAlloc(&r.groups, C * e->gcap));
+    CKC(devAlloc(&r.status, C * static_cast<size_t>(e->maxBlocks)));
+    CKC(devAlloc(&r.nAudio, C));
+    CKC(devAlloc(&r.nGroups, C));
+  }
   CKC(devAlloc(&e->dBits, C * e->bitsCap));
   CKC(devAlloc(&e->dWords, C * e->bitsCap));
   CKC(cudaMemcpy(e->dAudBank, e->audRs.bank.data(), e->audRs.bank.size() * sizeof(float),
@@ -1403,6 +1402,9 @@ int fmgpu_engine_create(const fmgpu_config *cfg, int n_channels, int device, fmg
   // per-channel defaults: FMDemod ctor filter (fm_demod.cpp:36-37), then the calls main.cpp makes
   const float ctorCut = std::clamp(110000.0f / static_cast<float>(e->fs), 0.01f, 0.45f);
   const int slot0 = filterSlot(e, 81, ctorCut, 60.0f);
+  if (slot0 < 0) {
+    return fail(slot0);
+  }
   ChanParams p{};
   p.filt = slot0;
   p.bandwidth_mode = 0;
@@ -1441,48 +1443,7 @@ void fmgpu_engine_destroy(fmgpu_engine *e) {
   }
   cudaSetDevice(e->device);
   cudaDeviceSynchronize();
-  void *ptrs[] = {e->dIq,      e->dHistIq, e->dX1,     e->dX2,      e->dY,       e->dMpx,
-                  e->dPilot,   e->dLraw,   e->dRraw,   e->dLf,      e->dRf,      e->dAudio,
-                  e->dRing,    e->dRdsHist, e->dMonoHist, e->dChanTaps, e->dChanScale, e->dChanLp,
-                  e->dAudBank, e->dRdsBank, e->dRdsLpf, e->dMf,     e->dDmf,     e->dParams,
-                  e->dDemod,   e->dStereo, e->dAudioSt, e->dRds,    e->dGroups,  e->dStatus,
-                  e->dNAudio,  e->dNGroups, e->dBits, e->dHistValid, e->dWords,
-                  e->dAudio2,  e->dGroups2, e->dStatus2, e->dNAudio2, e->dNGroups2, e->dR171,
-                  e->dDecB,    e->dDecOffs, e->dPilB, e->dAudB, e->dRdsRs};
-  for (auto &f : e->filters) {
-    if (f.dB) {
-      cudaFree(f.dB);
-    }
-  }
-  for (void *p : ptrs) {
-    if (p) {
-      cudaFree(p);
-    }
-  }
-  if (e->stream) {
-    cudaStreamDestroy(e->stream);
-  }
-  if (e->evStart) {
-    cudaEventDestroy(e->evStart);
-  }
-  for (auto &P : e->pipes) {
-    for (int st = 0; st < fmgpu_engine::ST_COUNT; st++) {
-      if (P.st[st]) {
-        cudaStreamDestroy(P.st[st]);
-      }
-      for (cudaEvent_t ev : P.done[st]) {
-        if (ev) {
-          cudaEventDestroy(ev);
-        }
-      }
-    }
-    for (cudaEvent_t ev : {P.callDone, P.hostDone[0], P.hostDone[1]}) {
-      if (ev) {
-        cudaEventDestroy(ev);
-      }
-    }
-  }
-  delete e;
+  delete e;  // the handles free every buffer, stream and event
 }
 
 const char *fmgpu_last_error(const fmgpu_engine *e) {
@@ -1520,8 +1481,7 @@ int fmgpu_set_bandwidth_hz(fmgpu_engine *e, int channel, int bw_hz) {
     }
     const int slot = filterSlot(e, spec.length, spec.cutoff, spec.atten);
     if (slot < 0) {
-      e->lastError = "channel filter table full";
-      return FMGPU_ENOMEM;
+      return slot;
     }
     p.bandwidth_mode = spec.index;
     p.filt = slot;
@@ -1988,19 +1948,7 @@ int fmgpu_submit_host(fmgpu_engine *e, const uint8_t *iq_host, size_t iq_stride_
   // submission queued behind, its copies overlap this call's kernels.
   // device-side result buffers alternate with the ticket, so the next submission's kernels never
   // wait for this one's device-to-host copies
-  float *dAud = ticket ? e->dAudio2 : e->dAudio;
-  fmgpu_rds_group *dGrp = ticket ? e->dGroups2 : e->dGroups;
-  fmgpu_block_status *dSt = ticket ? e->dStatus2 : e->dStatus;
-  uint32_t *dNA = ticket ? e->dNAudio2 : e->dNAudio;
-  uint32_t *dNG = ticket ? e->dNGroups2 : e->dNGroups;
-  BatchOut out;
-  out.audio = dAud;
-  out.acap = e->acap;
-  out.nAudio = dNA;
-  out.groups = dGrp;
-  out.gcap = static_cast<uint32_t>(e->gcap);
-  out.nGroups = dNG;
-  out.status = dSt;
+  const BatchOut out = engineOut(e, ticket);
   rc = queueBlocks(e, nullptr, iq_host, iq_stride_bytes, n_blocks, out, nullptr, false);
   if (rc != FMGPU_OK) {
     return rc;
@@ -2017,26 +1965,24 @@ int fmgpu_submit_host(fmgpu_engine *e, const uint8_t *iq_host, size_t iq_stride_
     const size_t c0 = static_cast<size_t>(ch0), cn = static_cast<size_t>(nch);
     if (audio_host) {
       CK(cudaMemcpy2DAsync(audio_host + c0 * 2 * audio_cap, audio_cap * sizeof(float),
-                           dAud + c0 * 2 * e->acap, e->acap * sizeof(float), frames * sizeof(float),
+                           out.audio + c0 * 2 * e->acap, e->acap * sizeof(float), frames * sizeof(float),
                            cn * 2, cudaMemcpyDeviceToHost, s));
     }
     if (n_audio_host) {
-      CK(cudaMemcpyAsync(n_audio_host + c0, dNA + c0, cn * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                         s));
+      CK(cudaMemcpyAsync(n_audio_host + c0, out.nAudio + c0, cn * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     }
     if (groups_host) {
       const size_t gw = std::min(group_cap, e->gcap);
       CK(cudaMemcpy2DAsync(groups_host + c0 * group_cap, group_cap * sizeof(fmgpu_rds_group),
-                           dGrp + c0 * e->gcap, e->gcap * sizeof(fmgpu_rds_group),
+                           out.groups + c0 * e->gcap, e->gcap * sizeof(fmgpu_rds_group),
                            gw * sizeof(fmgpu_rds_group), cn, cudaMemcpyDeviceToHost, s));
     }
     if (n_groups_host) {
-      CK(cudaMemcpyAsync(n_groups_host + c0, dNG + c0, cn * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                         s));
+      CK(cudaMemcpyAsync(n_groups_host + c0, out.nGroups + c0, cn * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     }
     if (status_host) {
       // the status rows of this call are [C][n_blocks] (pitch = n_blocks)
-      CK(cudaMemcpyAsync(status_host + c0 * n_blocks, dSt + c0 * n_blocks,
+      CK(cudaMemcpyAsync(status_host + c0 * n_blocks, out.status + c0 * n_blocks,
                          cn * n_blocks * sizeof(fmgpu_block_status), cudaMemcpyDeviceToHost, s));
     }
     CK(cudaEventRecord(P.hostDone[ticket], s));
@@ -2237,7 +2183,8 @@ static size_t demodCommon(fmgpu_engine *e, int channel, const uint8_t *iq_u8, co
   // the serial chain whatever the scan and demodulator modes: DC blocker -> channel FIR -> [AGC] ->
   // discriminator
   const BlockRef blk = stageBlock(channel, ni);
-  stageDcBlock(e, blk, iq_u8 ? nullptr : e->dX1, e->pitch, iq_u8 ? e->dIq : nullptr, e->iqPitch, false, s);
+  stageDcBlock(e, blk, iq_u8 ? nullptr : e->dX1.get(), e->pitch, iq_u8 ? e->dIq.get() : nullptr, e->iqPitch,
+               false, s);
   stageChanFir(e, blk, s);
   if (anyAgc(e, channel, 1)) {
     stageAgc(e, blk, s);
@@ -2255,7 +2202,7 @@ static size_t demodCommon(fmgpu_engine *e, int channel, const uint8_t *iq_u8, co
     cudaMemcpyAsync(&a, e->dAudioSt + channel, sizeof(a), cudaMemcpyDeviceToHost, s);
     cudaStreamSynchronize(s);
     produced = std::min<size_t>(a.mono_n_out, e->acap);
-    cudaMemcpyAsync(mono_out, e->dAudio + static_cast<size_t>(channel) * 2 * e->acap,
+    cudaMemcpyAsync(mono_out, e->res[0].audio + static_cast<size_t>(channel) * 2 * e->acap,
                     produced * sizeof(float), cudaMemcpyDeviceToHost, s);
   }
   cudaStreamSynchronize(s);
@@ -2290,7 +2237,7 @@ size_t fmgpu_downsample_mono(fmgpu_engine *e, int channel, const float *mpx, flo
   cudaMemcpyAsync(&a, e->dAudioSt + channel, sizeof(a), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
   const size_t produced = std::min<size_t>(a.mono_n_out, e->acap);
-  cudaMemcpyAsync(audio_out, e->dAudio + static_cast<size_t>(channel) * 2 * e->acap,
+  cudaMemcpyAsync(audio_out, e->res[0].audio + static_cast<size_t>(channel) * 2 * e->acap,
                   produced * sizeof(float), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
   return stageFail(e, "downsample") ? 0 : produced;
@@ -2357,9 +2304,9 @@ size_t fmgpu_afpost(fmgpu_engine *e, int channel, const float *in_left, const fl
   cudaMemcpyAsync(&a, e->dAudioSt + channel, sizeof(a), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
   const size_t produced = std::min<size_t>({a.n_out, out_capacity, e->acap});
-  cudaMemcpyAsync(out_left, e->dAudio + (static_cast<size_t>(channel) * 2 + 0) * e->acap,
+  cudaMemcpyAsync(out_left, e->res[0].audio + (static_cast<size_t>(channel) * 2 + 0) * e->acap,
                   produced * sizeof(float), cudaMemcpyDeviceToHost, s);
-  cudaMemcpyAsync(out_right, e->dAudio + (static_cast<size_t>(channel) * 2 + 1) * e->acap,
+  cudaMemcpyAsync(out_right, e->res[0].audio + (static_cast<size_t>(channel) * 2 + 1) * e->acap,
                   produced * sizeof(float), cudaMemcpyDeviceToHost, s);
   cudaStreamSynchronize(s);
   return stageFail(e, "afpost") ? 0 : produced;
@@ -2385,7 +2332,7 @@ size_t fmgpu_rds(fmgpu_engine *e, int channel, const float *mpx, size_t n, fmgpu
   const size_t ng = r.n_groups;
   const size_t copy = std::min({ng, cap, e->gcap});
   if (out && copy > 0) {
-    cudaMemcpyAsync(out, e->dGroups + static_cast<size_t>(channel) * e->gcap,
+    cudaMemcpyAsync(out, e->res[0].groups + static_cast<size_t>(channel) * e->gcap,
                     copy * sizeof(fmgpu_rds_group), cudaMemcpyDeviceToHost, s);
     cudaStreamSynchronize(s);
   }
@@ -2513,23 +2460,17 @@ int fmgpu_debug_timeline(fmgpu_engine *e, const char **names, int *groups, float
   int first = 0;
   for (int i = 1; i < n; i++) {
     float d = 0.0f;
-    if (cudaEventElapsedTime(&d, std::get<1>(e->spans[first]), std::get<1>(e->spans[i])) ==
-            cudaSuccess && d < 0.0f) {
+    if (cudaEventElapsedTime(&d, e->spans[first].start, e->spans[i].start) == cudaSuccess && d < 0.0f) {
       first = i;
     }
   }
   for (int i = 0; i < n && i < cap; i++) {
-    names[i] = std::get<0>(e->spans[i]);
-    groups[i] = e->spanGroup[i];
-    cudaEventElapsedTime(&t0_ms[i], std::get<1>(e->spans[first]), std::get<1>(e->spans[i]));
-    cudaEventElapsedTime(&t1_ms[i], std::get<1>(e->spans[first]), std::get<2>(e->spans[i]));
-  }
-  for (auto &sp : e->spans) {
-    cudaEventDestroy(std::get<1>(sp));
-    cudaEventDestroy(std::get<2>(sp));
+    names[i] = e->spans[i].name;
+    groups[i] = e->spans[i].group;
+    cudaEventElapsedTime(&t0_ms[i], e->spans[first].start, e->spans[i].start);
+    cudaEventElapsedTime(&t1_ms[i], e->spans[first].start, e->spans[i].end);
   }
   e->spans.clear();
-  e->spanGroup.clear();
   return n;
 }
 
