@@ -50,20 +50,27 @@
 #include "design.h"
 #include "device_once.h"
 
+// Captures. One object may serve n_captures captures that advance together (same rate, decimation,
+// spacing and filter; capture w's carrier k sits first_center_hz[w] + k * spacing from ITS centre).
+// Every kernel takes the capture from one grid dimension (k_chan_carry: one CTA per capture); each
+// capture has its own input row, history row and carrier frequencies (direct form: tap table and
+// phase steps; polyphase form: rotation table). The prototype taps and the DFT twiddles are shared.
+// One capture is the single-capture channelizer, with the same arithmetic.
 struct fmgpu_channelizer {
   int device = 0;
+  int nCap = 1;                    // captures
   int wideRate = 0, D = 0, C = 0, Cpad = 0, L = 0;
-  double firstHz = 0.0, spacingHz = 0.0;
+  double spacingHz = 0.0;
   std::vector<float> taps;         // prototype h[n]
-  std::vector<double> nuD;         // frac(nu_k * D): phase advance per output, in turns
-  fmgpu::DeviceArray<float2> dW;      // [L][Cpad]
-  fmgpu::DeviceArray<double> dNuD;    // [Cpad]
-  fmgpu::DeviceArray<uint8_t> dHist;  // last L-1 input samples (u8 pairs) of the previous call
-  // polyphase form (uniform grid): nu_k = (k + c0) / P
+  fmgpu::DeviceArray<float2> dW;      // [nCap][L][Cpad]
+  fmgpu::DeviceArray<double> dNuD;    // [nCap][Cpad] frac(nu_k * D): phase advance per output, in turns
+  fmgpu::DeviceArray<uint8_t> dHist;  // [nCap][2 (L-1)]: last L-1 input samples (u8 pairs) of the previous call
+  // polyphase form (uniform grid): nu_k = (k + c0_w) / P
   bool polyphase = false;
-  int P = 0, rotPeriod = 0;        // rotation table period (P * T, c0 * T integer)
+  int P = 0;
   fmgpu::DeviceArray<float> dTaps;    // [L]
-  fmgpu::DeviceArray<float2> dRot;    // [rotPeriod] exp(-j 2 pi c0 s / P)
+  fmgpu::DeviceArray<float2> dRot;    // capture w: [rotOff[w], rotOff[w+1]) exp(-j 2 pi c0_w s / P)
+  fmgpu::DeviceArray<int> dRotOff;    // [nCap + 1]; the period of capture w's table is P * T_w
   fmgpu::DeviceArray<float2> dTw;     // [P] exp(-j 2 pi i / P)
   unsigned long long outCount = 0; // outputs produced so far (m of the next output)
   long histValid = 0;              // how many of the carried samples are real input (rest = 0)
@@ -77,12 +84,18 @@ constexpr int WARPS = 4;          // warps per CTA: 4 groups of TMW instants
 constexpr int TM = TMW * WARPS;   // output instants per CTA
 
 __global__ void __launch_bounds__(32 * WARPS)
-k_channelize(const uint8_t *__restrict__ iq, const uint8_t *__restrict__ hist, long hist_valid,
-             long n_in,
+k_channelize(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restrict__ hist,
+             long hist_valid, long n_in,
              const float2 *__restrict__ W, const double *__restrict__ nuD, int L, int D, int Cpad,
              int ch_first, int ch_count, unsigned long long m_base, long n_out,
              float2 *__restrict__ out, size_t out_stride) {
   extern __shared__ float2 cx[];  // tile element a <-> input sample m0*D - (L-1) + a
+  const unsigned cap = blockIdx.z;  // capture: its input, history, taps, phase steps and output rows
+  iq += cap * iq_stride;
+  hist += (size_t)cap * 2 * (L - 1);
+  W += (size_t)cap * L * Cpad;
+  nuD += (size_t)cap * Cpad;
+  out += (size_t)cap * ch_count * out_stride;
   const long m0 = (long)blockIdx.x * TM;
   const int tile_len = (TM - 1) * D + L;
   const long s0 = m0 * D - (L - 1);
@@ -152,12 +165,19 @@ constexpr int PP_TM = 32;         // output instants per CTA of the polyphase ke
 constexpr int PP_THREADS = 256;
 
 __global__ void __launch_bounds__(PP_THREADS)
-k_channelize_pp(const uint8_t *__restrict__ iq, const uint8_t *__restrict__ hist, long hist_valid,
-                long n_in, const float *__restrict__ taps, const float2 *__restrict__ rot,
-                const float2 *__restrict__ tw, int L, int D, int P, int rot_period, int ch_first,
+k_channelize_pp(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restrict__ hist,
+                long hist_valid, long n_in, const float *__restrict__ taps,
+                const float2 *__restrict__ rot, const int *__restrict__ rot_off,
+                const float2 *__restrict__ tw, int L, int D, int P, int ch_first,
                 int ch_count, unsigned long long m_base, long n_out, float2 *__restrict__ out,
                 size_t out_stride) {
   extern __shared__ float2 pp_smem[];
+  const unsigned cap = blockIdx.y;  // capture: its input, history, rotation table and output rows
+  iq += cap * iq_stride;
+  hist += (size_t)cap * 2 * (L - 1);
+  rot += rot_off[cap];
+  const int rot_period = rot_off[cap + 1] - rot_off[cap];
+  out += (size_t)cap * ch_count * out_stride;
   const int tile_len = (PP_TM - 1) * D + L;
   float2 *xs = pp_smem;                       // [tile_len] rotated input, element a <-> sample m0*D-(L-1)+a
   float2 *u = xs + tile_len;                  // [P][PP_TM + 1]
@@ -234,11 +254,11 @@ k_channelize_pp(const uint8_t *__restrict__ iq, const uint8_t *__restrict__ hist
   }
 }
 
-// hist <- last H samples of (hist ++ in[0..n_in))
-__global__ void k_chan_carry(uint8_t *hist, const uint8_t *iq, long n_in, int H) {
-  uchar2 *h = reinterpret_cast<uchar2 *>(hist);
-  const uchar2 *in = reinterpret_cast<const uchar2 *>(iq);
-  // single CTA, two phases so the shift is safe when n_in < H
+// hist <- last H samples of (hist ++ in[0..n_in)), one CTA per capture
+__global__ void k_chan_carry(uint8_t *hist, const uint8_t *iq, size_t iq_stride, long n_in, int H) {
+  uchar2 *h = reinterpret_cast<uchar2 *>(hist) + (size_t)blockIdx.x * H;
+  const uchar2 *in = reinterpret_cast<const uchar2 *>(iq + blockIdx.x * iq_stride);
+  // two phases so the shift is safe when n_in < H
   extern __shared__ uchar2 tmp[];
   for (int e = threadIdx.x; e < H; e += blockDim.x) {
     const long src = n_in - H + e;
@@ -257,8 +277,18 @@ extern "C" {
 int fmgpu_channelizer_create(int device, int wide_rate, int decimation, int n_channels,
                              double first_center_hz, double spacing_hz, int taps_per_phase,
                              double cutoff_hz, float atten_db, fmgpu_channelizer **out) {
-  if (!out || wide_rate < 1 || decimation < 1 || n_channels < 1 || taps_per_phase < 1 ||
-      !(cutoff_hz > 0.0) || cutoff_hz * 2.0 > static_cast<double>(wide_rate)) {
+  return fmgpu_channelizer_create_multi(device, 1, wide_rate, decimation, n_channels, &first_center_hz,
+                                        spacing_hz, taps_per_phase, cutoff_hz, atten_db, out);
+}
+
+int fmgpu_channelizer_create_multi(int device, int n_captures, int wide_rate, int decimation,
+                                   int n_channels, const double *first_center_hz, double spacing_hz,
+                                   int taps_per_phase, double cutoff_hz, float atten_db,
+                                   fmgpu_channelizer **out) {
+  // the capture is a grid dimension: y of k_channelize_pp, z of k_channelize (at most 65535 each)
+  if (!out || !first_center_hz || n_captures < 1 || n_captures > 65535 || wide_rate < 1 ||
+      decimation < 1 || n_channels < 1 || taps_per_phase < 1 || !(cutoff_hz > 0.0) ||
+      cutoff_hz * 2.0 > static_cast<double>(wide_rate)) {
     return FMGPU_EINVAL;
   }
   *out = nullptr;
@@ -272,56 +302,74 @@ int fmgpu_channelizer_create(int device, int wide_rate, int decimation, int n_ch
     return FMGPU_ENOMEM;
   }
   z->device = device;
+  z->nCap = n_captures;
   z->wideRate = wide_rate;
   z->D = decimation;
   z->C = n_channels;
   z->Cpad = (n_channels + 31) / 32 * 32;
   z->L = decimation * taps_per_phase;
-  z->firstHz = first_center_hz;
   z->spacingHz = spacing_hz;
-  const float fc = static_cast<float>(cutoff_hz / static_cast<double>(wide_rate));
-  z->taps = fmdesign::kaiserLowpass(static_cast<unsigned>(z->L), fc, atten_db, 0.0f);
-  for (float &t : z->taps) {
-    t *= 2.0f * fc;  // unity gain in the pass band
-  }
-  std::vector<float2> W(static_cast<size_t>(z->L) * z->Cpad, make_float2(0.0f, 0.0f));
-  z->nuD.assign(z->Cpad, 0.0);
-  for (int k = 0; k < z->C; k++) {
-    const double nu = (first_center_hz + spacing_hz * k) / static_cast<double>(wide_rate);
-    const double adv = nu * static_cast<double>(decimation);
-    z->nuD[k] = adv - std::floor(adv);
-    for (int n = 0; n < z->L; n++) {
-      const double turns = nu * static_cast<double>(n);
-      const double ph = 2.0 * M_PI * (turns - std::floor(turns));
-      W[static_cast<size_t>(n) * z->Cpad + k] =
-          make_float2(static_cast<float>(z->taps[n] * std::cos(ph)),
-                      static_cast<float>(z->taps[n] * std::sin(ph)));
+  const size_t nCap = static_cast<size_t>(n_captures);
+  std::vector<float2> W, rotTab, twTab;
+  std::vector<double> nuD;
+  std::vector<int> rotOff;
+  try {
+    const float fc = static_cast<float>(cutoff_hz / static_cast<double>(wide_rate));
+    z->taps = fmdesign::kaiserLowpass(static_cast<unsigned>(z->L), fc, atten_db, 0.0f);
+    for (float &t : z->taps) {
+      t *= 2.0f * fc;  // unity gain in the pass band
     }
-  }
-  // uniform grid? P = Fs / spacing integer, c0 = first / spacing with c0 * T integer for a small T
-  std::vector<float2> rotTab, twTab;
-  {
-    const double pd = static_cast<double>(wide_rate) / spacing_hz;
-    const double c0 = first_center_hz / spacing_hz;
-    const int P = static_cast<int>(std::llround(pd));
-    int T = 0;
-    for (int t = 1; t <= 8 && T == 0; t++) {
-      if (std::fabs(c0 * t - std::round(c0 * t)) < 1e-9) {
-        T = t;
+    const size_t wRow = static_cast<size_t>(z->L) * z->Cpad;
+    W.assign(nCap * wRow, make_float2(0.0f, 0.0f));
+    nuD.assign(nCap * z->Cpad, 0.0);
+    for (size_t w = 0; w < nCap; w++) {
+      for (int k = 0; k < z->C; k++) {
+        const double nu = (first_center_hz[w] + spacing_hz * k) / static_cast<double>(wide_rate);
+        const double adv = nu * static_cast<double>(decimation);
+        nuD[w * z->Cpad + k] = adv - std::floor(adv);
+        for (int n = 0; n < z->L; n++) {
+          const double turns = nu * static_cast<double>(n);
+          const double ph = 2.0 * M_PI * (turns - std::floor(turns));
+          W[w * wRow + static_cast<size_t>(n) * z->Cpad + k] =
+              make_float2(static_cast<float>(z->taps[n] * std::cos(ph)),
+                          static_cast<float>(z->taps[n] * std::sin(ph)));
+        }
       }
     }
-    if (spacing_hz > 0.0 && P >= 2 && P <= 1024 && std::fabs(pd - P) < 1e-9 && T > 0 && n_channels <= P &&
-        getenv("FMGPU_CHANNELIZER_DIRECT") == nullptr) {
+    // uniform grid? P = Fs / spacing integer, and for every capture c0 = first / spacing with
+    // c0 * T integer for a small T; otherwise every capture takes the direct form
+    const double pd = static_cast<double>(wide_rate) / spacing_hz;
+    const int P = static_cast<int>(std::llround(pd));
+    bool uniform = spacing_hz > 0.0 && P >= 2 && P <= 1024 && std::fabs(pd - P) < 1e-9 && n_channels <= P &&
+                   getenv("FMGPU_CHANNELIZER_DIRECT") == nullptr;
+    std::vector<int> T(nCap, 0);
+    for (size_t w = 0; w < nCap && uniform; w++) {
+      const double c0 = first_center_hz[w] / spacing_hz;
+      for (int t = 1; t <= 8 && T[w] == 0; t++) {
+        if (std::fabs(c0 * t - std::round(c0 * t)) < 1e-9) {
+          T[w] = t;
+        }
+      }
+      uniform = T[w] > 0;
+    }
+    if (uniform) {
       z->polyphase = true;
       z->P = P;
-      z->rotPeriod = P * T;
-      rotTab.resize(z->rotPeriod);
-      for (int i = 0; i < z->rotPeriod; i++) {
-        // exp(-j 2 pi c0 i / P), the turn count reduced exactly: c0 * T is an integer
-        const long long num = std::llround(c0 * T) * static_cast<long long>(i);   // turns * (P T)
-        const long long red = ((num % z->rotPeriod) + z->rotPeriod) % z->rotPeriod;
-        const double ph = -2.0 * M_PI * static_cast<double>(red) / static_cast<double>(z->rotPeriod);
-        rotTab[i] = make_float2(static_cast<float>(std::cos(ph)), static_cast<float>(std::sin(ph)));
+      rotOff.assign(nCap + 1, 0);
+      for (size_t w = 0; w < nCap; w++) {
+        rotOff[w + 1] = rotOff[w] + P * T[w];
+      }
+      rotTab.resize(rotOff[nCap]);
+      for (size_t w = 0; w < nCap; w++) {
+        const double c0 = first_center_hz[w] / spacing_hz;
+        const int rotPeriod = P * T[w];
+        for (int i = 0; i < rotPeriod; i++) {
+          // exp(-j 2 pi c0 i / P), the turn count reduced exactly: c0 * T is an integer
+          const long long num = std::llround(c0 * T[w]) * static_cast<long long>(i);   // turns * (P T)
+          const long long red = ((num % rotPeriod) + rotPeriod) % rotPeriod;
+          const double ph = -2.0 * M_PI * static_cast<double>(red) / static_cast<double>(rotPeriod);
+          rotTab[rotOff[w] + i] = make_float2(static_cast<float>(std::cos(ph)), static_cast<float>(std::sin(ph)));
+        }
       }
       twTab.resize(P);
       for (int i = 0; i < P; i++) {
@@ -329,24 +377,29 @@ int fmgpu_channelizer_create(int device, int wide_rate, int decimation, int n_ch
         twTab[i] = make_float2(static_cast<float>(std::cos(ph)), static_cast<float>(std::sin(ph)));
       }
     }
+  } catch (const std::bad_alloc &) {
+    delete z;
+    return FMGPU_ENOMEM;
   }
   bool ok = cudaSetDevice(device) == cudaSuccess;
   if (z->polyphase) {
     ok = ok && fmgpu::devAlloc(&z->dTaps, z->taps.size()) == cudaSuccess;
     ok = ok && fmgpu::devAlloc(&z->dRot, rotTab.size()) == cudaSuccess;
+    ok = ok && fmgpu::devAlloc(&z->dRotOff, rotOff.size()) == cudaSuccess;
     ok = ok && fmgpu::devAlloc(&z->dTw, twTab.size()) == cudaSuccess;
     ok = ok && cudaMemcpy(z->dTaps, z->taps.data(), z->taps.size() * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
     ok = ok && cudaMemcpy(z->dRot, rotTab.data(), rotTab.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
+    ok = ok && cudaMemcpy(z->dRotOff, rotOff.data(), rotOff.size() * sizeof(int), cudaMemcpyHostToDevice) == cudaSuccess;
     ok = ok && cudaMemcpy(z->dTw, twTab.data(), twTab.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
   }
   ok = ok && fmgpu::devAlloc(&z->dW, W.size()) == cudaSuccess;
-  ok = ok && fmgpu::devAlloc(&z->dNuD, z->Cpad) == cudaSuccess;
+  ok = ok && fmgpu::devAlloc(&z->dNuD, nuD.size()) == cudaSuccess;
   // the input before the first call is ZERO: no byte maps to 0.0, so the kernel clears the
   // part of the window older than histValid samples
-  ok = ok && fmgpu::devAlloc(&z->dHist, static_cast<size_t>(z->L) * 2) == cudaSuccess;
+  ok = ok && fmgpu::devAlloc(&z->dHist, nCap * 2 * static_cast<size_t>(z->L - 1)) == cudaSuccess;
   ok = ok && cudaMemcpy(z->dW, W.data(), W.size() * sizeof(float2), cudaMemcpyHostToDevice) ==
                  cudaSuccess;
-  ok = ok && cudaMemcpy(z->dNuD, z->nuD.data(), z->Cpad * sizeof(double), cudaMemcpyHostToDevice) ==
+  ok = ok && cudaMemcpy(z->dNuD, nuD.data(), nuD.size() * sizeof(double), cudaMemcpyHostToDevice) ==
                  cudaSuccess;
   if (!ok) {
     cudaGetLastError();
@@ -368,6 +421,8 @@ void fmgpu_channelizer_destroy(fmgpu_channelizer *z) {
 
 int fmgpu_channelizer_output_rate(const fmgpu_channelizer *z) { return z ? z->wideRate / z->D : 0; }
 
+int fmgpu_channelizer_n_captures(const fmgpu_channelizer *z) { return z ? z->nCap : 0; }
+
 size_t fmgpu_channelizer_taps(const fmgpu_channelizer *z, float *out, size_t cap) {
   if (!z) {
     return 0;
@@ -383,7 +438,19 @@ size_t fmgpu_channelizer_taps(const fmgpu_channelizer *z, float *out, size_t cap
 int fmgpu_channelizer_process(fmgpu_channelizer *z, const uint8_t *iq_dev, size_t n_in,
                               int ch_first, int ch_count, float *out_cf32_dev,
                               size_t out_stride_samples, void *stream) {
+  if (z && z->nCap != 1) {
+    return FMGPU_EINVAL;
+  }
+  return fmgpu_channelizer_process_multi(z, iq_dev, 2 * n_in, n_in, ch_first, ch_count, out_cf32_dev,
+                                         out_stride_samples, stream);
+}
+
+int fmgpu_channelizer_process_multi(fmgpu_channelizer *z, const uint8_t *iq_dev,
+                                    size_t iq_stride_bytes, size_t n_in, int ch_first,
+                                    int ch_count, float *out_cf32_dev, size_t out_stride_samples,
+                                    void *stream) {
   if (!z || !iq_dev || !out_cf32_dev || n_in == 0 || n_in % static_cast<size_t>(z->D) != 0 ||
+      iq_stride_bytes % 2 != 0 || iq_stride_bytes < 2 * n_in ||
       ch_first < 0 || ch_count < 1 || ch_first + ch_count > z->C ||
       out_stride_samples < n_in / static_cast<size_t>(z->D)) {
     return FMGPU_EINVAL;
@@ -392,6 +459,7 @@ int fmgpu_channelizer_process(fmgpu_channelizer *z, const uint8_t *iq_dev, size_
     return FMGPU_ENODEV;
   }
   cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const unsigned nCap = static_cast<unsigned>(z->nCap);
   const long n_out = static_cast<long>(n_in / static_cast<size_t>(z->D));
   const size_t smem = static_cast<size_t>((TM - 1) * z->D + z->L) * sizeof(float2);
   static fmgpu::DeviceOnce attrs;  // per device: device_once.h
@@ -405,19 +473,21 @@ int fmgpu_channelizer_process(fmgpu_channelizer *z, const uint8_t *iq_dev, size_
   if (z->polyphase && pp_smem <= 200 * 1024) {
     static fmgpu::DeviceOnce pp_attrs;
     pp_attrs.run([] { return cudaFuncSetAttribute(k_channelize_pp, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
-    k_channelize_pp<<<static_cast<unsigned>((n_out + PP_TM - 1) / PP_TM), PP_THREADS, pp_smem, s>>>(
-        iq_dev, z->dHist, z->histValid, static_cast<long>(n_in), z->dTaps, z->dRot, z->dTw, z->L, z->D, z->P,
-        z->rotPeriod, ch_first, ch_count, z->outCount, n_out, reinterpret_cast<float2 *>(out_cf32_dev),
-        out_stride_samples);
+    dim3 grid(static_cast<unsigned>((n_out + PP_TM - 1) / PP_TM), nCap);
+    k_channelize_pp<<<grid, PP_THREADS, pp_smem, s>>>(
+        iq_dev, iq_stride_bytes, z->dHist, z->histValid, static_cast<long>(n_in), z->dTaps, z->dRot, z->dRotOff,
+        z->dTw, z->L, z->D, z->P, ch_first, ch_count, z->outCount, n_out,
+        reinterpret_cast<float2 *>(out_cf32_dev), out_stride_samples);
   } else {
-    dim3 grid(static_cast<unsigned>((n_out + TM - 1) / TM), static_cast<unsigned>((ch_count + 31) / 32));
+    dim3 grid(static_cast<unsigned>((n_out + TM - 1) / TM), static_cast<unsigned>((ch_count + 31) / 32), nCap);
     k_channelize<<<grid, 32 * WARPS, smem, s>>>(
-        iq_dev, z->dHist, z->histValid, static_cast<long>(n_in), z->dW, z->dNuD, z->L, z->D, z->Cpad, ch_first,
-        ch_count, z->outCount, n_out, reinterpret_cast<float2 *>(out_cf32_dev), out_stride_samples);
+        iq_dev, iq_stride_bytes, z->dHist, z->histValid, static_cast<long>(n_in), z->dW, z->dNuD, z->L, z->D,
+        z->Cpad, ch_first, ch_count, z->outCount, n_out, reinterpret_cast<float2 *>(out_cf32_dev),
+        out_stride_samples);
   }
   const int H = z->L - 1;
-  k_chan_carry<<<1, 512, static_cast<size_t>(H) * sizeof(uchar2), s>>>(z->dHist, iq_dev,
-                                                                      static_cast<long>(n_in), H);
+  k_chan_carry<<<nCap, 512, static_cast<size_t>(H) * sizeof(uchar2), s>>>(z->dHist, iq_dev, iq_stride_bytes,
+                                                                         static_cast<long>(n_in), H);
   z->outCount += static_cast<unsigned long long>(n_out);
   z->histValid = std::min<long>(H, z->histValid + static_cast<long>(n_in));
   return cudaGetLastError() == cudaSuccess ? FMGPU_OK : FMGPU_ENODEV;

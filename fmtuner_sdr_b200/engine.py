@@ -119,6 +119,10 @@ def load_library(build: bool = True):
     L.fmgpu_channelizer_taps.argtypes = [vp, f32p, sz]
     L.fmgpu_channelizer_taps.restype = sz
     L.fmgpu_channelizer_process.argtypes = [vp, u8p, sz, i32, i32, f32p, sz, vp]
+    L.fmgpu_channelizer_create_multi.argtypes = [i32, i32, i32, i32, i32, C.POINTER(C.c_double),
+                                                 C.c_double, i32, C.c_double, C.c_float, C.POINTER(vp)]
+    L.fmgpu_channelizer_n_captures.argtypes = [vp]
+    L.fmgpu_channelizer_process_multi.argtypes = [vp, u8p, sz, sz, i32, i32, f32p, sz, vp]
     L.fmgpu_submit_host.argtypes = [vp, u8p, sz, i32, f32p, sz, vp, vp, sz, vp, vp]
     L.fmgpu_wait_host.argtypes = [vp, i32]
     L.fmgpu_decimate.restype = sz
@@ -508,16 +512,28 @@ class XdrRdsFormatter:
 
 class Channelizer:
     """Wideband front end for BASELINE config 4 (include/fmgpu.h: fmgpu_channelizer_*): one uint8
-    IQ capture -> n_channels complex-float streams at wide_rate / decimation."""
+    IQ capture -> n_channels complex-float streams at wide_rate / decimation.
+
+    first_center_hz may be a sequence: one capture per entry, all advancing together, capture w's
+    carrier k at first_center_hz[w] + k * spacing_hz from its own centre (fmgpu_channelizer_create_multi);
+    its outputs are n_captures * ch_count rows, capture-major."""
 
     def __init__(self, wide_rate=24_000_000, decimation=100, n_channels=100,
                  first_center_hz=-9_900_000.0, spacing_hz=200_000.0, taps_per_phase=16,
                  cutoff_hz=100_000.0, atten_db=60.0, device=0):
         self.L = load_library()
         h = C.c_void_p()
-        rc = self.L.fmgpu_channelizer_create(device, wide_rate, decimation, n_channels,
-                                             first_center_hz, spacing_hz, taps_per_phase, cutoff_hz,
-                                             atten_db, C.byref(h))
+        if np.ndim(first_center_hz) == 0:
+            rc = self.L.fmgpu_channelizer_create(device, wide_rate, decimation, n_channels,
+                                                 first_center_hz, spacing_hz, taps_per_phase,
+                                                 cutoff_hz, atten_db, C.byref(h))
+        else:
+            first_center_hz = [float(f) for f in first_center_hz]
+            arr = (C.c_double * len(first_center_hz))(*first_center_hz)
+            rc = self.L.fmgpu_channelizer_create_multi(device, len(first_center_hz), wide_rate,
+                                                       decimation, n_channels, arr, spacing_hz,
+                                                       taps_per_phase, cutoff_hz, atten_db,
+                                                       C.byref(h))
         if rc != 0:
             raise EngineError(f"fmgpu_channelizer_create failed ({rc}); no CPU fallback")
         self.h = h
@@ -528,6 +544,10 @@ class Channelizer:
     def output_rate(self) -> int:
         return self.L.fmgpu_channelizer_output_rate(self.h)
 
+    @property
+    def n_captures(self) -> int:
+        return self.L.fmgpu_channelizer_n_captures(self.h)
+
     def taps(self) -> np.ndarray:
         n = self.L.fmgpu_channelizer_taps(self.h, None, 0)
         out = np.zeros(n, np.float32)
@@ -535,12 +555,22 @@ class Channelizer:
         return out
 
     def process(self, iq_dev_ptr, n_in, out_dev_ptr, out_stride_samples, ch_first=0, ch_count=None,
-                stream=None):
+                stream=None, iq_stride_bytes=None):
+        """With more than one capture: iq [n_captures][iq_stride_bytes] (default 2 * n_in) and
+        out [n_captures][ch_count][out_stride_samples]."""
         ch_count = self.n_channels - ch_first if ch_count is None else ch_count
-        rc = self.L.fmgpu_channelizer_process(self.h, iq_dev_ptr, n_in, ch_first, ch_count,
-                                              out_dev_ptr, out_stride_samples, stream)
+        if self.n_captures > 1:
+            stride = 2 * n_in if iq_stride_bytes is None else iq_stride_bytes
+            rc = self.L.fmgpu_channelizer_process_multi(self.h, iq_dev_ptr, stride, n_in, ch_first,
+                                                        ch_count, out_dev_ptr, out_stride_samples,
+                                                        stream)
+            what = "fmgpu_channelizer_process_multi"
+        else:
+            rc = self.L.fmgpu_channelizer_process(self.h, iq_dev_ptr, n_in, ch_first, ch_count,
+                                                  out_dev_ptr, out_stride_samples, stream)
+            what = "fmgpu_channelizer_process"
         if rc != 0:
-            raise EngineError(f"fmgpu_channelizer_process failed ({rc})")
+            raise EngineError(f"{what} failed ({rc})")
 
     def close(self):
         if self.h:

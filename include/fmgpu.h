@@ -248,21 +248,50 @@ int fmgpu_xdr_rds_lines(fmgpu_xdr_rds_state *s, const fmgpu_rds_group *g, char l
  * fmgpu_process_batch_cf32 (the FMDemod::processSplitComplex path, fm_demod.cpp:258-274).
  * Definition (what tests/test_gpu_channelizer.py evaluates in float64):
  *   y_k[m] = sum_n h[n] x[m*D - n] exp(-j 2 pi f_k (m*D - n) / wide_rate),  x = (u8 - 127.5)/127.5,
- * m counted from creation, input before the first call = 0. */
+ * m counted from creation, input before the first call = 0.
+ * Two evaluations of it: a polyphase bank when the carriers sit on a uniform grid (wide_rate /
+ * spacing_hz an integer P <= 1024, n_channels <= P, and first_center_hz / spacing_hz * T an
+ * integer for some T <= 8), otherwise the direct form (one complex tap table per carrier, several
+ * times slower). FMGPU_CHANNELIZER_DIRECT set in the environment at creation selects the direct form.
+ *
+ * Many captures: one object may serve n_captures captures that advance together (same wide_rate,
+ * decimation, carrier spacing and filter), each with its own centre offset: capture w's carrier k
+ * sits first_center_hz[w] + k * spacing_hz from ITS centre. The definition holds per capture, with
+ * capture w's input, its own history and its own f_k; m is shared. The polyphase bank is used only
+ * when every capture passes the grid test above, so one off-grid offset (e.g. a ppm-corrected
+ * centre) selects the slower direct form for all captures. At most 65535 captures.
+ * fmgpu_channelizer_create is fmgpu_channelizer_create_multi with one capture. */
 typedef struct fmgpu_channelizer fmgpu_channelizer;
 int fmgpu_channelizer_create(int device, int wide_rate, int decimation, int n_channels,
                              double first_center_hz, double spacing_hz, int taps_per_phase,
                              double cutoff_hz, float atten_db, fmgpu_channelizer **out);
+/* first_center_hz [n_captures] */
+int fmgpu_channelizer_create_multi(int device, int n_captures, int wide_rate, int decimation,
+                                   int n_channels, const double *first_center_hz, double spacing_hz,
+                                   int taps_per_phase, double cutoff_hz, float atten_db,
+                                   fmgpu_channelizer **out);
 void fmgpu_channelizer_destroy(fmgpu_channelizer *z);
 int fmgpu_channelizer_output_rate(const fmgpu_channelizer *z);
+int fmgpu_channelizer_n_captures(const fmgpu_channelizer *z);
 size_t fmgpu_channelizer_taps(const fmgpu_channelizer *z, float *out, size_t cap);
 /* iq_dev: n_in uint8 I,Q pairs (n_in a multiple of the decimation) continuing the stream of the
  * previous call; out_cf32_dev [ch_count][out_stride_samples] complex float for channels
  * ch_first .. ch_first + ch_count - 1 (a rank of a sharded job extracts only its own channels from
- * the capture every rank reads). Asynchronous on `stream`. */
+ * the capture every rank reads). Asynchronous on `stream`. FMGPU_EINVAL on an object with more
+ * than one capture. */
 int fmgpu_channelizer_process(fmgpu_channelizer *z, const uint8_t *iq_dev, size_t n_in,
                               int ch_first, int ch_count, float *out_cf32_dev,
                               size_t out_stride_samples, void *stream);
+/* iq_dev [n_captures][iq_stride_bytes] (stride even, >= 2 * n_in): n_in pairs per capture,
+ * continuing each capture's stream. out_cf32_dev [n_captures][ch_count][out_stride_samples]: row
+ * w * ch_count + kk is carrier ch_first + kk of capture w, so the buffer is an
+ * fmgpu_process_batch_cf32 input of n_captures * ch_count channels as it stands. A rank of a
+ * sharded job channelizes either its own captures (its own object) or its ch_first / ch_count share
+ * of every capture. Asynchronous on `stream`. */
+int fmgpu_channelizer_process_multi(fmgpu_channelizer *z, const uint8_t *iq_dev,
+                                    size_t iq_stride_bytes, size_t n_in, int ch_first,
+                                    int ch_count, float *out_cf32_dev, size_t out_stride_samples,
+                                    void *stream);
 
 /* fmgpu_process_batch with complex-float input at the DSP rate (engine created with
  * decimation = 1): x_cf32_dev [C][stride_samples] interleaved re,im; base and stride 16-byte
