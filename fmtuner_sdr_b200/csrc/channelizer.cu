@@ -1,4 +1,4 @@
-// channelizer.cu — wideband front end for BASELINE config 4: one uint8 IQ capture (24 MS/s) ->
+// channelizer.cu — wideband front end for BASELINE config 4: one IQ capture (24 MS/s) ->
 // C carriers at a fixed spacing, each mixed to baseband, low-pass filtered and decimated to the
 // engine's DSP rate (240 kS/s), ready for fmgpu_process_batch_cf32.
 //
@@ -9,9 +9,9 @@
 //   y_k[m] = sum_{n=0}^{L-1} h[n] * x[m*D - n] * exp(-j 2 pi nu_k (m*D - n)),   nu_k = f_k / Fs
 //          = exp(-j 2 pi nu_k m D) * sum_n W[n][k] * x[m*D - n],   W[n][k] = h[n] exp(+j 2 pi nu_k n)
 //
-// with x[s] = (u8 - 127.5) / 127.5 (the convention of ComplexDecimator, liquid_primitives.cpp:
-// 461-499), h a Kaiser-windowed sinc of L = D * taps_per_phase taps scaled to unity pass-band gain,
-// and the input before the first call equal to zero. m counts outputs since creation, so
+// with x[s] the input pair converted by the object's sample format (toX below; for uint8,
+// (u8 - 127.5) / 127.5, the convention of ComplexDecimator, liquid_primitives.cpp:461-499), h a
+// Kaiser-windowed sinc of L = D * taps_per_phase taps scaled to unity pass-band gain, and the input before the first call equal to zero. m counts outputs since creation, so
 // consecutive calls continue the same stream (the last L-1 inputs are carried).
 //
 // Two evaluations of that definition:
@@ -37,6 +37,7 @@
 //   every thread keeps 8 output instants so a tap is reused 8 times.
 #include <algorithm>
 #include <cmath>
+#include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <new>
@@ -64,7 +65,9 @@ struct fmgpu_channelizer {
   std::vector<float> taps;         // prototype h[n]
   fmgpu::DeviceArray<float2> dW;      // [nCap][L][Cpad]
   fmgpu::DeviceArray<double> dNuD;    // [nCap][Cpad] frac(nu_k * D): phase advance per output, in turns
-  fmgpu::DeviceArray<uint8_t> dHist;  // [nCap][2 (L-1)]: last L-1 input samples (u8 pairs) of the previous call
+  int format = FMGPU_IQ_CU8;       // sample format, shared by every capture
+  int pairBytes = 2;               // bytes of one I,Q pair of that format
+  fmgpu::DeviceArray<uint8_t> dHist;  // [nCap][pairBytes (L-1)]: last L-1 input pairs of the previous call
   // polyphase form (uniform grid): nu_k = (k + c0_w) / P
   bool polyphase = false;
   int P = 0;
@@ -79,10 +82,24 @@ struct fmgpu_channelizer {
 
 namespace {
 
+// Sample formats (include/fmgpu.h FMGPU_IQ_*): the pair type a kernel is instantiated on decides only
+// how a pair becomes x; everything after the load is the same for every format.
+__device__ __forceinline__ float2 toX(uchar2 b) {  // FMGPU_IQ_CU8: offset binary
+  constexpr float kScale = 1.0f / 127.5f;
+  return make_float2(((float)b.x - 127.5f) * kScale, ((float)b.y - 127.5f) * kScale);
+}
+__device__ __forceinline__ float2 toX(char2 b) {   // FMGPU_IQ_CS8: exact
+  return make_float2((float)b.x * (1.0f / 128.0f), (float)b.y * (1.0f / 128.0f));
+}
+__device__ __forceinline__ float2 toX(short2 b) {  // FMGPU_IQ_CS16: exact
+  return make_float2((float)b.x * (1.0f / 32768.0f), (float)b.y * (1.0f / 32768.0f));
+}
+
 constexpr int TMW = 8;            // output instants per thread
 constexpr int WARPS = 4;          // warps per CTA: 4 groups of TMW instants
 constexpr int TM = TMW * WARPS;   // output instants per CTA
 
+template <typename Pair>
 __global__ void __launch_bounds__(32 * WARPS)
 k_channelize(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restrict__ hist,
              long hist_valid, long n_in,
@@ -92,16 +109,15 @@ k_channelize(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__
   extern __shared__ float2 cx[];  // tile element a <-> input sample m0*D - (L-1) + a
   const unsigned cap = blockIdx.z;  // capture: its input, history, taps, phase steps and output rows
   iq += cap * iq_stride;
-  hist += (size_t)cap * 2 * (L - 1);
+  hist += (size_t)cap * sizeof(Pair) * (L - 1);
   W += (size_t)cap * L * Cpad;
   nuD += (size_t)cap * Cpad;
   out += (size_t)cap * ch_count * out_stride;
   const long m0 = (long)blockIdx.x * TM;
   const int tile_len = (TM - 1) * D + L;
   const long s0 = m0 * D - (L - 1);
-  constexpr float kScale = 1.0f / 127.5f;
-  const uchar2 *in2 = reinterpret_cast<const uchar2 *>(iq);
-  const uchar2 *hist2 = reinterpret_cast<const uchar2 *>(hist);
+  const Pair *in2 = reinterpret_cast<const Pair *>(iq);
+  const Pair *hist2 = reinterpret_cast<const Pair *>(hist);
   for (int a = threadIdx.x; a < tile_len; a += blockDim.x) {
     const long s = s0 + a;
     float2 v = make_float2(0.0f, 0.0f);
@@ -109,8 +125,7 @@ k_channelize(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__
       // beyond this call (only outputs past n_out would use it) or before the first input ever
       v = make_float2(0.0f, 0.0f);
     } else {
-      const uchar2 b = (s >= 0) ? in2[s] : hist2[(L - 1) + s];
-      v = make_float2(((float)b.x - 127.5f) * kScale, ((float)b.y - 127.5f) * kScale);
+      v = toX((s >= 0) ? in2[s] : hist2[(L - 1) + s]);
     }
     cx[a] = v;
   }
@@ -164,6 +179,7 @@ k_channelize(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__
 constexpr int PP_TM = 32;         // output instants per CTA of the polyphase kernel
 constexpr int PP_THREADS = 256;
 
+template <typename Pair>
 __global__ void __launch_bounds__(PP_THREADS)
 k_channelize_pp(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t *__restrict__ hist,
                 long hist_valid, long n_in, const float *__restrict__ taps,
@@ -174,7 +190,7 @@ k_channelize_pp(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t 
   extern __shared__ float2 pp_smem[];
   const unsigned cap = blockIdx.y;  // capture: its input, history, rotation table and output rows
   iq += cap * iq_stride;
-  hist += (size_t)cap * 2 * (L - 1);
+  hist += (size_t)cap * sizeof(Pair) * (L - 1);
   rot += rot_off[cap];
   const int rot_period = rot_off[cap + 1] - rot_off[cap];
   out += (size_t)cap * ch_count * out_stride;
@@ -185,17 +201,16 @@ k_channelize_pp(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t 
   float *hs = reinterpret_cast<float *>(tws + P);   // [L]
   const long m0 = (long)blockIdx.x * PP_TM;
   const long s0 = m0 * D - (L - 1);           // call-relative sample index of tile element 0
-  constexpr float kScale = 1.0f / 127.5f;
-  const uchar2 *in2 = reinterpret_cast<const uchar2 *>(iq);
-  const uchar2 *hist2 = reinterpret_cast<const uchar2 *>(hist);
+  const Pair *in2 = reinterpret_cast<const Pair *>(iq);
+  const Pair *hist2 = reinterpret_cast<const Pair *>(hist);
   // absolute sample index of call-relative sample 0, modulo the rotation period
   const unsigned long long abs0 = (m_base % (unsigned long long)rot_period) * (unsigned long long)D;
   for (int a = threadIdx.x; a < tile_len; a += PP_THREADS) {
     const long s = s0 + a;
     float2 v = make_float2(0.0f, 0.0f);
     if (s < n_in && s >= -hist_valid) {
-      const uchar2 b = (s >= 0) ? in2[s] : hist2[(L - 1) + s];
-      const float xr = ((float)b.x - 127.5f) * kScale, xi = ((float)b.y - 127.5f) * kScale;
+      const float2 x = toX((s >= 0) ? in2[s] : hist2[(L - 1) + s]);
+      const float xr = x.x, xi = x.y;
       // (abs0 + s) mod period, s may be negative: add a multiple of the period first
       const unsigned long long ai = abs0 + (unsigned long long)(s + (long)rot_period * (long)(L / rot_period + 2));
       const float2 w = rot[ai % (unsigned long long)rot_period];
@@ -254,12 +269,15 @@ k_channelize_pp(const uint8_t *__restrict__ iq, size_t iq_stride, const uint8_t 
   }
 }
 
-// hist <- last H samples of (hist ++ in[0..n_in)), one CTA per capture
+// hist <- last H pairs of (hist ++ in[0..n_in)), one CTA per capture. It only moves pairs, so it
+// is instantiated per pair size (uchar2: cu8 and cs8; short2: cs16), not per format.
+template <typename Pair>
 __global__ void k_chan_carry(uint8_t *hist, const uint8_t *iq, size_t iq_stride, long n_in, int H) {
-  uchar2 *h = reinterpret_cast<uchar2 *>(hist) + (size_t)blockIdx.x * H;
-  const uchar2 *in = reinterpret_cast<const uchar2 *>(iq + blockIdx.x * iq_stride);
+  Pair *h = reinterpret_cast<Pair *>(hist) + (size_t)blockIdx.x * H;
+  const Pair *in = reinterpret_cast<const Pair *>(iq + blockIdx.x * iq_stride);
   // two phases so the shift is safe when n_in < H
-  extern __shared__ uchar2 tmp[];
+  extern __shared__ __align__(4) unsigned char carry_smem[];
+  Pair *tmp = reinterpret_cast<Pair *>(carry_smem);
   for (int e = threadIdx.x; e < H; e += blockDim.x) {
     const long src = n_in - H + e;
     tmp[e] = (src >= 0) ? in[src] : h[e + n_in];
@@ -268,6 +286,47 @@ __global__ void k_chan_carry(uint8_t *hist, const uint8_t *iq, size_t iq_stride,
   for (int e = threadIdx.x; e < H; e += blockDim.x) {
     h[e] = tmp[e];
   }
+}
+
+// bytes of one I,Q pair of a sample format; 0 for an unknown format
+int formatPairBytes(int format) {
+  switch (format) {
+    case FMGPU_IQ_CU8:
+    case FMGPU_IQ_CS8:
+      return 2;
+    case FMGPU_IQ_CS16:
+      return 4;
+    default:
+      return 0;
+  }
+}
+
+// The one launch sequence of a call, instantiated on the format's pair type (Carry: the pair type
+// of the same size that k_chan_carry moves).
+template <typename Pair, typename Carry>
+void launchChannelize(fmgpu_channelizer *z, const uint8_t *iq_dev, size_t iq_stride_bytes, size_t n_in,
+                      int ch_first, int ch_count, float2 *out, size_t out_stride_samples,
+                      size_t smem, size_t pp_smem, cudaStream_t s) {
+  const unsigned nCap = static_cast<unsigned>(z->nCap);
+  const long n_out = static_cast<long>(n_in / static_cast<size_t>(z->D));
+  if (z->polyphase && pp_smem <= 200 * 1024) {
+    static fmgpu::DeviceOnce pp_attrs;  // per device and instantiation: device_once.h
+    pp_attrs.run([] { return cudaFuncSetAttribute(k_channelize_pp<Pair>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
+    dim3 grid(static_cast<unsigned>((n_out + PP_TM - 1) / PP_TM), nCap);
+    k_channelize_pp<Pair><<<grid, PP_THREADS, pp_smem, s>>>(
+        iq_dev, iq_stride_bytes, z->dHist, z->histValid, static_cast<long>(n_in), z->dTaps, z->dRot, z->dRotOff,
+        z->dTw, z->L, z->D, z->P, ch_first, ch_count, z->outCount, n_out, out, out_stride_samples);
+  } else {
+    static fmgpu::DeviceOnce attrs;
+    attrs.run([] { return cudaFuncSetAttribute(k_channelize<Pair>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
+    dim3 grid(static_cast<unsigned>((n_out + TM - 1) / TM), static_cast<unsigned>((ch_count + 31) / 32), nCap);
+    k_channelize<Pair><<<grid, 32 * WARPS, smem, s>>>(
+        iq_dev, iq_stride_bytes, z->dHist, z->histValid, static_cast<long>(n_in), z->dW, z->dNuD, z->L, z->D,
+        z->Cpad, ch_first, ch_count, z->outCount, n_out, out, out_stride_samples);
+  }
+  const int H = z->L - 1;
+  k_chan_carry<Carry><<<nCap, 512, static_cast<size_t>(H) * sizeof(Carry), s>>>(z->dHist, iq_dev, iq_stride_bytes,
+                                                                               static_cast<long>(n_in), H);
 }
 
 }  // namespace
@@ -285,8 +344,16 @@ int fmgpu_channelizer_create_multi(int device, int n_captures, int wide_rate, in
                                    int n_channels, const double *first_center_hz, double spacing_hz,
                                    int taps_per_phase, double cutoff_hz, float atten_db,
                                    fmgpu_channelizer **out) {
+  return fmgpu_channelizer_create_format(device, FMGPU_IQ_CU8, n_captures, wide_rate, decimation, n_channels,
+                                         first_center_hz, spacing_hz, taps_per_phase, cutoff_hz, atten_db, out);
+}
+
+int fmgpu_channelizer_create_format(int device, int sample_format, int n_captures, int wide_rate,
+                                    int decimation, int n_channels, const double *first_center_hz,
+                                    double spacing_hz, int taps_per_phase, double cutoff_hz,
+                                    float atten_db, fmgpu_channelizer **out) {
   // the capture is a grid dimension: y of k_channelize_pp, z of k_channelize (at most 65535 each)
-  if (!out || !first_center_hz || n_captures < 1 || n_captures > 65535 || wide_rate < 1 ||
+  if (!out || formatPairBytes(sample_format) == 0 || !first_center_hz || n_captures < 1 || n_captures > 65535 || wide_rate < 1 ||
       decimation < 1 || n_channels < 1 || taps_per_phase < 1 || !(cutoff_hz > 0.0) ||
       cutoff_hz * 2.0 > static_cast<double>(wide_rate)) {
     return FMGPU_EINVAL;
@@ -303,6 +370,8 @@ int fmgpu_channelizer_create_multi(int device, int n_captures, int wide_rate, in
   }
   z->device = device;
   z->nCap = n_captures;
+  z->format = sample_format;
+  z->pairBytes = formatPairBytes(sample_format);
   z->wideRate = wide_rate;
   z->D = decimation;
   z->C = n_channels;
@@ -394,9 +463,9 @@ int fmgpu_channelizer_create_multi(int device, int n_captures, int wide_rate, in
   }
   ok = ok && fmgpu::devAlloc(&z->dW, W.size()) == cudaSuccess;
   ok = ok && fmgpu::devAlloc(&z->dNuD, nuD.size()) == cudaSuccess;
-  // the input before the first call is ZERO: no byte maps to 0.0, so the kernel clears the
-  // part of the window older than histValid samples
-  ok = ok && fmgpu::devAlloc(&z->dHist, nCap * 2 * static_cast<size_t>(z->L - 1)) == cudaSuccess;
+  // the input before the first call is ZERO: no uint8 pair maps to 0.0, so for every format the
+  // kernel clears the part of the window older than histValid samples
+  ok = ok && fmgpu::devAlloc(&z->dHist, nCap * z->pairBytes * static_cast<size_t>(z->L - 1)) == cudaSuccess;
   ok = ok && cudaMemcpy(z->dW, W.data(), W.size() * sizeof(float2), cudaMemcpyHostToDevice) ==
                  cudaSuccess;
   ok = ok && cudaMemcpy(z->dNuD, nuD.data(), nuD.size() * sizeof(double), cudaMemcpyHostToDevice) ==
@@ -422,6 +491,8 @@ void fmgpu_channelizer_destroy(fmgpu_channelizer *z) {
 int fmgpu_channelizer_output_rate(const fmgpu_channelizer *z) { return z ? z->wideRate / z->D : 0; }
 
 int fmgpu_channelizer_n_captures(const fmgpu_channelizer *z) { return z ? z->nCap : 0; }
+
+int fmgpu_channelizer_sample_format(const fmgpu_channelizer *z) { return z ? z->format : FMGPU_EINVAL; }
 
 size_t fmgpu_channelizer_taps(const fmgpu_channelizer *z, float *out, size_t cap) {
   if (!z) {
@@ -449,8 +520,22 @@ int fmgpu_channelizer_process_multi(fmgpu_channelizer *z, const uint8_t *iq_dev,
                                     size_t iq_stride_bytes, size_t n_in, int ch_first,
                                     int ch_count, float *out_cf32_dev, size_t out_stride_samples,
                                     void *stream) {
-  if (!z || !iq_dev || !out_cf32_dev || n_in == 0 || n_in % static_cast<size_t>(z->D) != 0 ||
-      iq_stride_bytes % 2 != 0 || iq_stride_bytes < 2 * n_in ||
+  if (z && z->format != FMGPU_IQ_CU8) {
+    return FMGPU_EINVAL;
+  }
+  return fmgpu_channelizer_process_iq(z, iq_dev, iq_stride_bytes, n_in, ch_first, ch_count, out_cf32_dev,
+                                      out_stride_samples, stream);
+}
+
+int fmgpu_channelizer_process_iq(fmgpu_channelizer *z, const void *iq_dev, size_t iq_stride_bytes,
+                                 size_t n_in, int ch_first, int ch_count, float *out_cf32_dev,
+                                 size_t out_stride_samples, void *stream) {
+  if (!z || !iq_dev || !out_cf32_dev || n_in == 0 || n_in % static_cast<size_t>(z->D) != 0) {
+    return FMGPU_EINVAL;
+  }
+  const size_t pb = static_cast<size_t>(z->pairBytes);
+  if (iq_stride_bytes % pb != 0 || iq_stride_bytes < pb * n_in ||
+      reinterpret_cast<uintptr_t>(iq_dev) % pb != 0 ||
       ch_first < 0 || ch_count < 1 || ch_first + ch_count > z->C ||
       out_stride_samples < n_in / static_cast<size_t>(z->D)) {
     return FMGPU_EINVAL;
@@ -459,37 +544,32 @@ int fmgpu_channelizer_process_multi(fmgpu_channelizer *z, const uint8_t *iq_dev,
     return FMGPU_ENODEV;
   }
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const unsigned nCap = static_cast<unsigned>(z->nCap);
-  const long n_out = static_cast<long>(n_in / static_cast<size_t>(z->D));
   const size_t smem = static_cast<size_t>((TM - 1) * z->D + z->L) * sizeof(float2);
-  static fmgpu::DeviceOnce attrs;  // per device: device_once.h
-  attrs.run([] { return cudaFuncSetAttribute(k_channelize, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
   if (smem > 200 * 1024) {
     z->lastError = "channelizer: filter too long for the shared-memory tile";
     return FMGPU_ERANGE;
   }
   const size_t pp_smem = (static_cast<size_t>((PP_TM - 1) * z->D + z->L) + static_cast<size_t>(z->P) * (PP_TM + 1) +
                           static_cast<size_t>(z->P)) * sizeof(float2) + static_cast<size_t>(z->L) * sizeof(float);
-  if (z->polyphase && pp_smem <= 200 * 1024) {
-    static fmgpu::DeviceOnce pp_attrs;
-    pp_attrs.run([] { return cudaFuncSetAttribute(k_channelize_pp, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
-    dim3 grid(static_cast<unsigned>((n_out + PP_TM - 1) / PP_TM), nCap);
-    k_channelize_pp<<<grid, PP_THREADS, pp_smem, s>>>(
-        iq_dev, iq_stride_bytes, z->dHist, z->histValid, static_cast<long>(n_in), z->dTaps, z->dRot, z->dRotOff,
-        z->dTw, z->L, z->D, z->P, ch_first, ch_count, z->outCount, n_out,
-        reinterpret_cast<float2 *>(out_cf32_dev), out_stride_samples);
-  } else {
-    dim3 grid(static_cast<unsigned>((n_out + TM - 1) / TM), static_cast<unsigned>((ch_count + 31) / 32), nCap);
-    k_channelize<<<grid, 32 * WARPS, smem, s>>>(
-        iq_dev, iq_stride_bytes, z->dHist, z->histValid, static_cast<long>(n_in), z->dW, z->dNuD, z->L, z->D,
-        z->Cpad, ch_first, ch_count, z->outCount, n_out, reinterpret_cast<float2 *>(out_cf32_dev),
-        out_stride_samples);
+  const uint8_t *iq = static_cast<const uint8_t *>(iq_dev);
+  float2 *out = reinterpret_cast<float2 *>(out_cf32_dev);
+  switch (z->format) {
+    case FMGPU_IQ_CU8:
+      launchChannelize<uchar2, uchar2>(z, iq, iq_stride_bytes, n_in, ch_first, ch_count, out, out_stride_samples,
+                                       smem, pp_smem, s);
+      break;
+    case FMGPU_IQ_CS8:
+      launchChannelize<char2, uchar2>(z, iq, iq_stride_bytes, n_in, ch_first, ch_count, out, out_stride_samples,
+                                      smem, pp_smem, s);
+      break;
+    default:  // FMGPU_IQ_CS16: create accepts no other format
+      launchChannelize<short2, short2>(z, iq, iq_stride_bytes, n_in, ch_first, ch_count, out, out_stride_samples,
+                                       smem, pp_smem, s);
+      break;
   }
-  const int H = z->L - 1;
-  k_chan_carry<<<nCap, 512, static_cast<size_t>(H) * sizeof(uchar2), s>>>(z->dHist, iq_dev, iq_stride_bytes,
-                                                                         static_cast<long>(n_in), H);
+  const long n_out = static_cast<long>(n_in / static_cast<size_t>(z->D));
   z->outCount += static_cast<unsigned long long>(n_out);
-  z->histValid = std::min<long>(H, z->histValid + static_cast<long>(n_in));
+  z->histValid = std::min<long>(z->L - 1, z->histValid + static_cast<long>(n_in));
   return cudaGetLastError() == cudaSuccess ? FMGPU_OK : FMGPU_ENODEV;
 }
 

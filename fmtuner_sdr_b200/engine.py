@@ -123,6 +123,10 @@ def load_library(build: bool = True):
                                                  C.c_double, i32, C.c_double, C.c_float, C.POINTER(vp)]
     L.fmgpu_channelizer_n_captures.argtypes = [vp]
     L.fmgpu_channelizer_process_multi.argtypes = [vp, u8p, sz, sz, i32, i32, f32p, sz, vp]
+    L.fmgpu_channelizer_create_format.argtypes = [i32, i32, i32, i32, i32, i32, C.POINTER(C.c_double),
+                                                  C.c_double, i32, C.c_double, C.c_float, C.POINTER(vp)]
+    L.fmgpu_channelizer_sample_format.argtypes = [vp]
+    L.fmgpu_channelizer_process_iq.argtypes = [vp, vp, sz, sz, i32, i32, f32p, sz, vp]
     L.fmgpu_submit_host.argtypes = [vp, u8p, sz, i32, f32p, sz, vp, vp, sz, vp, vp]
     L.fmgpu_wait_host.argtypes = [vp, i32]
     L.fmgpu_decimate.restype = sz
@@ -510,33 +514,41 @@ class XdrRdsFormatter:
         return [buf.raw[32 * i:32 * i + 32].split(b"\0")[0].decode() for i in range(n)]
 
 
+SAMPLE_FORMATS = {"cu8": 0, "cs8": 1, "cs16": 2}     # include/fmgpu.h FMGPU_IQ_*
+PAIR_BYTES = {"cu8": 2, "cs8": 2, "cs16": 4}
+
+
 class Channelizer:
-    """Wideband front end for BASELINE config 4 (include/fmgpu.h: fmgpu_channelizer_*): one uint8
-    IQ capture -> n_channels complex-float streams at wide_rate / decimation.
+    """Wideband front end for BASELINE config 4 (include/fmgpu.h: fmgpu_channelizer_*): one IQ
+    capture -> n_channels complex-float streams at wide_rate / decimation.
+
+    sample_format is the captures' I,Q pair format: "cu8" (uint8 offset binary, RTL-SDR), "cs8"
+    (int8, HackRF) or "cs16" (int16, USRP / bladeRF / LimeSDR / SDRplay, SoapySDR CS16).
 
     first_center_hz may be a sequence: one capture per entry, all advancing together, capture w's
-    carrier k at first_center_hz[w] + k * spacing_hz from its own centre (fmgpu_channelizer_create_multi);
-    its outputs are n_captures * ch_count rows, capture-major."""
+    carrier k at first_center_hz[w] + k * spacing_hz from its own centre; its outputs are
+    n_captures * ch_count rows, capture-major."""
 
     def __init__(self, wide_rate=24_000_000, decimation=100, n_channels=100,
                  first_center_hz=-9_900_000.0, spacing_hz=200_000.0, taps_per_phase=16,
-                 cutoff_hz=100_000.0, atten_db=60.0, device=0):
+                 cutoff_hz=100_000.0, atten_db=60.0, device=0, sample_format="cu8"):
+        if sample_format not in SAMPLE_FORMATS:
+            raise ValueError(f"sample_format must be one of {sorted(SAMPLE_FORMATS)}, not {sample_format!r}")
         self.L = load_library()
+        self.h = None
         h = C.c_void_p()
-        if np.ndim(first_center_hz) == 0:
-            rc = self.L.fmgpu_channelizer_create(device, wide_rate, decimation, n_channels,
-                                                 first_center_hz, spacing_hz, taps_per_phase,
-                                                 cutoff_hz, atten_db, C.byref(h))
-        else:
-            first_center_hz = [float(f) for f in first_center_hz]
-            arr = (C.c_double * len(first_center_hz))(*first_center_hz)
-            rc = self.L.fmgpu_channelizer_create_multi(device, len(first_center_hz), wide_rate,
-                                                       decimation, n_channels, arr, spacing_hz,
-                                                       taps_per_phase, cutoff_hz, atten_db,
-                                                       C.byref(h))
+        firsts = [float(first_center_hz)] if np.ndim(first_center_hz) == 0 else \
+            [float(f) for f in first_center_hz]
+        arr = (C.c_double * len(firsts))(*firsts)
+        rc = self.L.fmgpu_channelizer_create_format(device, SAMPLE_FORMATS[sample_format], len(firsts),
+                                                    wide_rate, decimation, n_channels, arr, spacing_hz,
+                                                    taps_per_phase, cutoff_hz, atten_db, C.byref(h))
         if rc != 0:
-            raise EngineError(f"fmgpu_channelizer_create failed ({rc}); no CPU fallback")
+            raise EngineError(f"fmgpu_channelizer_create_format failed ({rc}); no CPU fallback")
+        if np.ndim(first_center_hz) != 0:
+            first_center_hz = firsts
         self.h = h
+        self._format = sample_format
         self.wide_rate, self.decimation, self.n_channels = wide_rate, decimation, n_channels
         self.first_center_hz, self.spacing_hz = first_center_hz, spacing_hz
 
@@ -548,6 +560,15 @@ class Channelizer:
     def n_captures(self) -> int:
         return self.L.fmgpu_channelizer_n_captures(self.h)
 
+    @property
+    def sample_format(self) -> str:
+        return self._format
+
+    @property
+    def pair_bytes(self) -> int:
+        """Bytes of one I,Q pair of the input."""
+        return PAIR_BYTES[self._format]
+
     def taps(self) -> np.ndarray:
         n = self.L.fmgpu_channelizer_taps(self.h, None, 0)
         out = np.zeros(n, np.float32)
@@ -556,21 +577,14 @@ class Channelizer:
 
     def process(self, iq_dev_ptr, n_in, out_dev_ptr, out_stride_samples, ch_first=0, ch_count=None,
                 stream=None, iq_stride_bytes=None):
-        """With more than one capture: iq [n_captures][iq_stride_bytes] (default 2 * n_in) and
-        out [n_captures][ch_count][out_stride_samples]."""
+        """iq [n_captures][iq_stride_bytes] (default pair_bytes * n_in): n_in pairs per capture;
+        out [n_captures][ch_count][out_stride_samples] (fmgpu_channelizer_process_iq)."""
         ch_count = self.n_channels - ch_first if ch_count is None else ch_count
-        if self.n_captures > 1:
-            stride = 2 * n_in if iq_stride_bytes is None else iq_stride_bytes
-            rc = self.L.fmgpu_channelizer_process_multi(self.h, iq_dev_ptr, stride, n_in, ch_first,
-                                                        ch_count, out_dev_ptr, out_stride_samples,
-                                                        stream)
-            what = "fmgpu_channelizer_process_multi"
-        else:
-            rc = self.L.fmgpu_channelizer_process(self.h, iq_dev_ptr, n_in, ch_first, ch_count,
-                                                  out_dev_ptr, out_stride_samples, stream)
-            what = "fmgpu_channelizer_process"
+        stride = self.pair_bytes * n_in if iq_stride_bytes is None else iq_stride_bytes
+        rc = self.L.fmgpu_channelizer_process_iq(self.h, iq_dev_ptr, stride, n_in, ch_first, ch_count,
+                                                 out_dev_ptr, out_stride_samples, stream)
         if rc != 0:
-            raise EngineError(f"{what} failed ({rc})")
+            raise EngineError(f"fmgpu_channelizer_process_iq failed ({rc})")
 
     def close(self):
         if self.h:

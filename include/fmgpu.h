@@ -240,15 +240,16 @@ void fmgpu_xdr_rds_init(fmgpu_xdr_rds_state *s);
 int fmgpu_xdr_rds_lines(fmgpu_xdr_rds_state *s, const fmgpu_rds_group *g, char lines[2][32]);
 
 /* ---- wideband channelizer (BASELINE config 4; SURVEY section 8(f) row 3) --------------------
- * NO reference counterpart: the reference tunes one carrier in the RTL-SDR hardware. One uint8 IQ
- * capture at wide_rate holds n_channels carriers, channel k centred first_center_hz +
+ * NO reference counterpart: the reference tunes one carrier in the RTL-SDR hardware. One IQ
+ * capture at wide_rate (uint8 by default; other sample formats below) holds n_channels carriers, channel k centred first_center_hz +
  * k * spacing_hz away from the capture centre; each is mixed to baseband, low-pass filtered by a
  * Kaiser-windowed sinc of decimation * taps_per_phase taps (cut-off cutoff_hz, atten_db) and
  * decimated to wide_rate / decimation — complex float at the engine's DSP rate, the input of
  * fmgpu_process_batch_cf32 (the FMDemod::processSplitComplex path, fm_demod.cpp:258-274).
  * Definition (what tests/test_gpu_channelizer.py evaluates in float64):
- *   y_k[m] = sum_n h[n] x[m*D - n] exp(-j 2 pi f_k (m*D - n) / wide_rate),  x = (u8 - 127.5)/127.5,
- * m counted from creation, input before the first call = 0.
+ *   y_k[m] = sum_n h[n] x[m*D - n] exp(-j 2 pi f_k (m*D - n) / wide_rate),
+ * x the input pair converted by the object's sample format (FMGPU_IQ_*): cu8 x = (u8 - 127.5)/127.5,
+ * cs8 x = s8 / 128, cs16 x = s16 / 32768; m counted from creation, input before the first call = 0.
  * Two evaluations of it: a polyphase bank when the carriers sit on a uniform grid (wide_rate /
  * spacing_hz an integer P <= 1024, n_channels <= P, and first_center_hz / spacing_hz * T an
  * integer for some T <= 8), otherwise the direct form (one complex tap table per carrier, several
@@ -260,7 +261,16 @@ int fmgpu_xdr_rds_lines(fmgpu_xdr_rds_state *s, const fmgpu_rds_group *g, char l
  * capture w's input, its own history and its own f_k; m is shared. The polyphase bank is used only
  * when every capture passes the grid test above, so one off-grid offset (e.g. a ppm-corrected
  * centre) selects the slower direct form for all captures. At most 65535 captures.
- * fmgpu_channelizer_create is fmgpu_channelizer_create_multi with one capture. */
+ * fmgpu_channelizer_create is fmgpu_channelizer_create_multi with one capture.
+ *
+ * Sample formats: all captures of one object share one format (a mixed fleet uses one object per
+ * format). Only the load of a pair differs; the filter, the bank and the outputs' layout do not.
+ * bladeRF's SC16_Q11 samples are cs16 with full scale 2048, so their outputs come out 16x smaller,
+ * which the scale-invariant discriminator behind the channelizer does not notice. */
+#define FMGPU_IQ_CU8 0   /* uint8 I,Q, offset binary: RTL-SDR */
+#define FMGPU_IQ_CS8 1   /* int8 I,Q: HackRF */
+#define FMGPU_IQ_CS16 2  /* int16 I,Q, native (little-endian) order: USRP, bladeRF, LimeSDR,
+                            SDRplay (SoapySDR CS16) */
 typedef struct fmgpu_channelizer fmgpu_channelizer;
 int fmgpu_channelizer_create(int device, int wide_rate, int decimation, int n_channels,
                              double first_center_hz, double spacing_hz, int taps_per_phase,
@@ -270,15 +280,23 @@ int fmgpu_channelizer_create_multi(int device, int n_captures, int wide_rate, in
                                    int n_channels, const double *first_center_hz, double spacing_hz,
                                    int taps_per_phase, double cutoff_hz, float atten_db,
                                    fmgpu_channelizer **out);
+/* fmgpu_channelizer_create_multi for captures of sample_format (FMGPU_IQ_*; FMGPU_EINVAL for any
+ * other value); create_multi is this with FMGPU_IQ_CU8. */
+int fmgpu_channelizer_create_format(int device, int sample_format, int n_captures, int wide_rate,
+                                    int decimation, int n_channels, const double *first_center_hz,
+                                    double spacing_hz, int taps_per_phase, double cutoff_hz,
+                                    float atten_db, fmgpu_channelizer **out);
 void fmgpu_channelizer_destroy(fmgpu_channelizer *z);
 int fmgpu_channelizer_output_rate(const fmgpu_channelizer *z);
 int fmgpu_channelizer_n_captures(const fmgpu_channelizer *z);
+/* the FMGPU_IQ_* format the object was created for */
+int fmgpu_channelizer_sample_format(const fmgpu_channelizer *z);
 size_t fmgpu_channelizer_taps(const fmgpu_channelizer *z, float *out, size_t cap);
 /* iq_dev: n_in uint8 I,Q pairs (n_in a multiple of the decimation) continuing the stream of the
  * previous call; out_cf32_dev [ch_count][out_stride_samples] complex float for channels
  * ch_first .. ch_first + ch_count - 1 (a rank of a sharded job extracts only its own channels from
  * the capture every rank reads). Asynchronous on `stream`. FMGPU_EINVAL on an object with more
- * than one capture. */
+ * than one capture or another format than FMGPU_IQ_CU8. */
 int fmgpu_channelizer_process(fmgpu_channelizer *z, const uint8_t *iq_dev, size_t n_in,
                               int ch_first, int ch_count, float *out_cf32_dev,
                               size_t out_stride_samples, void *stream);
@@ -287,11 +305,19 @@ int fmgpu_channelizer_process(fmgpu_channelizer *z, const uint8_t *iq_dev, size_
  * w * ch_count + kk is carrier ch_first + kk of capture w, so the buffer is an
  * fmgpu_process_batch_cf32 input of n_captures * ch_count channels as it stands. A rank of a
  * sharded job channelizes either its own captures (its own object) or its ch_first / ch_count share
- * of every capture. Asynchronous on `stream`. */
+ * of every capture. Asynchronous on `stream`. It is fmgpu_channelizer_process_iq for FMGPU_IQ_CU8
+ * objects, and FMGPU_EINVAL on any other format. */
 int fmgpu_channelizer_process_multi(fmgpu_channelizer *z, const uint8_t *iq_dev,
                                     size_t iq_stride_bytes, size_t n_in, int ch_first,
                                     int ch_count, float *out_cf32_dev, size_t out_stride_samples,
                                     void *stream);
+/* Any format, any number of captures: iq_dev [n_captures][iq_stride_bytes] holds n_in pairs of the
+ * object's format per capture (pair size 2 bytes for cu8 and cs8, 4 for cs16). FMGPU_EINVAL when the
+ * stride is not a multiple of the pair size or shorter than pair size * n_in, or iq_dev is not
+ * aligned to the pair size; otherwise as fmgpu_channelizer_process_multi. */
+int fmgpu_channelizer_process_iq(fmgpu_channelizer *z, const void *iq_dev, size_t iq_stride_bytes,
+                                 size_t n_in, int ch_first, int ch_count, float *out_cf32_dev,
+                                 size_t out_stride_samples, void *stream);
 
 /* fmgpu_process_batch with complex-float input at the DSP rate (engine created with
  * decimation = 1): x_cf32_dev [C][stride_samples] interleaved re,im; base and stride 16-byte

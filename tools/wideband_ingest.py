@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """Many wideband captures through one channelizer: what batching the captures buys.
 
-Usage: python tools/wideband_ingest.py OUT_DIR [--steps K] [--reps R] [--only a|b]
+Usage: python tools/wideband_ingest.py OUT_DIR [--steps K] [--reps R] [--only a|b|formats]
 
-Writes OUT_DIR/wideband_ingest.jsonl, one JSON line per workload, each with the card name, power
+Writes OUT_DIR/wideband_ingest.jsonl, one JSON line per workload (the formats workload runs only
+with --only formats and writes OUT_DIR/wideband_formats.jsonl), each with the card name, power
 limit and maximum SM clock read (nvidia-smi, read-only) in the same run. One step is 68 ms of
 signal per capture: two 8192-sample blocks at 240 kS/s.
 
@@ -21,7 +22,12 @@ Per workload:
                 pinned host; ms per step, real-time factor, real-time captures per GPU, and H2D
                 GB/s against a bare copy of the same buffers measured in the same run
 
-Inputs are seeded random bytes generated on the device. Needs a CUDA device: without one it fails.
+  (formats) 32 captures of 24 MS/s, 100 carriers, D = 100, as cu8, cs8 and cs16 objects
+             (fmgpu_channelizer_create_format) on inputs of the same number of pairs (cs16: twice
+             the bytes): the channelizer stage alone, formats alternated rep by rep, and the full
+             step above for each format, reps alternated the same way, through one engine
+
+Inputs are seeded random samples generated on the device. Needs a CUDA device: without one it fails.
 """
 from __future__ import annotations
 
@@ -113,71 +119,152 @@ def run_workload(fm, torch, kind, W, wide, D, Cn, c0s, steps, reps, seed):
             "outputs_equal": same}
     chan["singles_over_multi"] = chan["singles"]["ms_per_step_median"] / chan["multi"]["ms_per_step_median"]
 
-    # full step
-    nch = W * Cn
-    eng = fm.Engine(fm.make_config(iq_rate=240_000, decimation=1, max_blocks=B), nch, 0)
-    acap = eng.audio_capacity(B)
-    audio = torch.empty((nch, 2, acap), dtype=torch.float32, device=dev)
-    n_audio = torch.zeros(nch, dtype=torch.int32, device=dev)
-    status = torch.zeros((nch, B, 20), dtype=torch.uint8, device=dev)
-    iq_host = torch.empty((W, stride), dtype=torch.uint8).pin_memory()
-    iq_host.copy_(iq)
-    audio_host = torch.empty((nch, 2, acap), dtype=torch.float32).pin_memory()
-    n_audio_host = torch.zeros(nch, dtype=torch.int32).pin_memory()
-    bufs = [iq, torch.empty_like(iq)]
-    cs = torch.cuda.Stream()
-    copied = [torch.cuda.Event(), torch.cuda.Event()]
-    consumed = [torch.cuda.Event(), torch.cuda.Event()]
-    h2d = [(ev(), ev()) for _ in range(steps)]
-
-    def full(k, rec=None):
-        i = k & 1
-        with torch.cuda.stream(cs):
-            cs.wait_event(consumed[i])
-            if rec:
-                rec[0].record(cs)
-            bufs[i].copy_(iq_host, non_blocking=True)
-            if rec:
-                rec[1].record(cs)
-            copied[i].record(cs)
-        s.wait_event(copied[i])
-        zm.process(bufs[i].data_ptr(), n_in, out_m.data_ptr(), n_dsp, stream=sp, iq_stride_bytes=stride)
-        consumed[i].record(s)
-        eng.process_batch_cf32(out_m.data_ptr(), n_dsp, B, audio.data_ptr(), acap, n_audio.data_ptr(),
-                               None, B + 8, None, status.data_ptr(), sp)
-        with torch.cuda.stream(s):
-            audio_host.copy_(audio, non_blocking=True)
-            n_audio_host.copy_(n_audio, non_blocking=True)
-
-    for k in range(3):
-        full(k)
-    torch.cuda.synchronize()
-    t0 = time.perf_counter()
-    for k in range(steps):
-        full(k, h2d[k])
-    torch.cuda.synchronize()
-    step_ms = (time.perf_counter() - t0) / steps * 1e3
-    h2d_ms = statistics.median(a.elapsed_time(b) for a, b in h2d)
-    # bare copy of the same buffers, nothing else running
-    e0, e1 = ev(), ev()
-    with torch.cuda.stream(cs):
-        e0.record(cs)
-        for k in range(steps):
-            bufs[k & 1].copy_(iq_host, non_blocking=True)
-        e1.record(cs)
-    torch.cuda.synchronize()
-    bare_ms = e0.elapsed_time(e1) / steps
+    eng = FullStep(fm, torch, W * Cn, s)
+    full_rec = eng.run(zm, iq, n_in, out_m, steps)
     eng.close()
     zm.close()
-    sig_s = n_dsp / 240_000.0
-    nbytes = W * stride
-    rtf = sig_s / (step_ms * 1e-3)
-    full_rec = {"ms_per_step": step_ms, "realtime_factor": rtf, "realtime_captures_per_gpu": W * rtf,
+    return {"workload": kind, "captures": W, "wide_rate": wide, "decimation": D, "carriers_per_capture": Cn,
+            "c0": c0s, "taps": D * 16, "steps": steps, "reps": reps, "signal_ms_per_step": n_dsp / 240.0,
+            "channelizer": chan, "full_step": full_rec}
+
+
+class FullStep:
+    """pinned host [W][stride] -> device (copy stream, double-buffered) -> channelizer -> engine of
+    nch channels -> audio back to pinned host, on stream s."""
+
+    def __init__(self, fm, torch, nch, s):
+        self.torch, self.s, self.nch = torch, s, nch
+        dev = torch.device("cuda", 0)
+        self.eng = fm.Engine(fm.make_config(iq_rate=240_000, decimation=1, max_blocks=B), nch, 0)
+        self.acap = self.eng.audio_capacity(B)
+        self.audio = torch.empty((nch, 2, self.acap), dtype=torch.float32, device=dev)
+        self.n_audio = torch.zeros(nch, dtype=torch.int32, device=dev)
+        self.status = torch.zeros((nch, B, 20), dtype=torch.uint8, device=dev)
+        self.audio_host = torch.empty((nch, 2, self.acap), dtype=torch.float32).pin_memory()
+        self.n_audio_host = torch.zeros(nch, dtype=torch.int32).pin_memory()
+
+    def close(self):
+        self.eng.close()
+
+    def run(self, zm, iq, n_in, out_m, steps):
+        """iq [W][stride] on the device, the input of zm; its copy in pinned host memory is the source."""
+        torch, s, eng = self.torch, self.s, self.eng
+        sp = s.cuda_stream
+        n_dsp = B * BLOCK
+        W = iq.shape[0]
+        stride = iq[0].numel() * iq.element_size()
+        acap, audio, n_audio, status = self.acap, self.audio, self.n_audio, self.status
+        audio_host, n_audio_host = self.audio_host, self.n_audio_host
+        iq_host = torch.empty_like(iq, device="cpu").pin_memory()
+        iq_host.copy_(iq)
+        bufs = [iq, torch.empty_like(iq)]
+        cs = torch.cuda.Stream()
+        copied = [torch.cuda.Event(), torch.cuda.Event()]
+        consumed = [torch.cuda.Event(), torch.cuda.Event()]
+        h2d = [(ev(), ev()) for _ in range(steps)]
+
+        def full(k, rec=None):
+            i = k & 1
+            with torch.cuda.stream(cs):
+                cs.wait_event(consumed[i])
+                if rec:
+                    rec[0].record(cs)
+                bufs[i].copy_(iq_host, non_blocking=True)
+                if rec:
+                    rec[1].record(cs)
+                copied[i].record(cs)
+            s.wait_event(copied[i])
+            zm.process(bufs[i].data_ptr(), n_in, out_m.data_ptr(), n_dsp, stream=sp, iq_stride_bytes=stride)
+            consumed[i].record(s)
+            eng.process_batch_cf32(out_m.data_ptr(), n_dsp, B, audio.data_ptr(), acap, n_audio.data_ptr(),
+                                   None, B + 8, None, status.data_ptr(), sp)
+            with torch.cuda.stream(s):
+                audio_host.copy_(audio, non_blocking=True)
+                n_audio_host.copy_(n_audio, non_blocking=True)
+
+        for k in range(3):
+            full(k)
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        for k in range(steps):
+            full(k, h2d[k])
+        torch.cuda.synchronize()
+        step_ms = (time.perf_counter() - t0) / steps * 1e3
+        h2d_ms = statistics.median(a.elapsed_time(b) for a, b in h2d)
+        # bare copy of the same buffers, nothing else running
+        e0, e1 = ev(), ev()
+        with torch.cuda.stream(cs):
+            e0.record(cs)
+            for k in range(steps):
+                bufs[k & 1].copy_(iq_host, non_blocking=True)
+            e1.record(cs)
+        torch.cuda.synchronize()
+        bare_ms = e0.elapsed_time(e1) / steps
+        sig_s = n_dsp / 240_000.0
+        nbytes = W * stride
+        rtf = sig_s / (step_ms * 1e-3)
+        return {"ms_per_step": step_ms, "realtime_factor": rtf, "realtime_captures_per_gpu": W * rtf,
                 "h2d_bytes_per_step": nbytes, "h2d_gbs_in_step": nbytes / (h2d_ms * 1e-3) / 1e9,
                 "h2d_gbs_bare_copy": nbytes / (bare_ms * 1e-3) / 1e9}
-    return {"workload": kind, "captures": W, "wide_rate": wide, "decimation": D, "carriers_per_capture": Cn,
-            "c0": c0s, "taps": D * 16, "steps": steps, "reps": reps, "signal_ms_per_step": sig_s * 1e3,
-            "channelizer": chan, "full_step": full_rec}
+
+
+def run_formats(fm, torch, steps, reps, seed):
+    """32 full-band sites as cu8, cs8 and cs16 captures of the same number of pairs."""
+    W, wide, D, Cn = 32, 24_000_000, 100, 100
+    dev = torch.device("cuda", 0)
+    n_in = B * BLOCK * D
+    n_dsp = B * BLOCK
+    g = torch.Generator(device=dev)
+    g.manual_seed(seed)
+    iq = {"cu8": torch.randint(0, 256, (W, 2 * n_in), dtype=torch.uint8, device=dev, generator=g),
+          "cs8": torch.randint(-128, 128, (W, 2 * n_in), dtype=torch.int8, device=dev, generator=g),
+          "cs16": torch.randint(-32768, 32768, (W, 2 * n_in), dtype=torch.int16, device=dev, generator=g)}
+    s = torch.cuda.Stream()
+    sp = s.cuda_stream
+    firsts = [-49.5 * SP] * W
+    zs = {f: fm.Channelizer(first_center_hz=firsts, wide_rate=wide, decimation=D, n_channels=Cn, spacing_hz=SP,
+                            taps_per_phase=16, cutoff_hz=100_000.0, sample_format=f) for f in iq}
+    out = torch.zeros((W * Cn, n_dsp, 2), dtype=torch.float32, device=dev)
+
+    def timed(f):
+        z, x = zs[f], iq[f]
+        e0, e1 = ev(), ev()
+        torch.cuda.synchronize()
+        e0.record(s)
+        for _ in range(steps):
+            z.process(x.data_ptr(), n_in, out.data_ptr(), n_dsp, stream=sp)
+        e1.record(s)
+        e1.synchronize()
+        return e0.elapsed_time(e1) / steps
+
+    for f in iq:                                # warm-up
+        for _ in range(2):
+            zs[f].process(iq[f].data_ptr(), n_in, out.data_ptr(), n_dsp, stream=sp)
+    chan = {f: [] for f in iq}
+    for _ in range(reps):
+        for f in iq:
+            chan[f].append(timed(f))
+    eng = FullStep(fm, torch, W * Cn, s)
+    full = {f: [] for f in iq}
+    for _ in range(reps):
+        for f in iq:
+            full[f].append(eng.run(zs[f], iq[f], n_in, out, steps))
+    eng.close()
+    for z in zs.values():
+        z.close()
+    rec = {"workload": "formats", "captures": W, "wide_rate": wide, "decimation": D, "carriers_per_capture": Cn,
+           "c0": [-49.5], "taps": D * 16, "form": "polyphase", "pairs_per_capture_per_step": n_in,
+           "steps": steps, "reps": reps, "signal_ms_per_step": n_dsp / 240.0, "formats": {}}
+    for f in iq:
+        ms = chan[f]
+        fs = sorted(full[f], key=lambda r: r["ms_per_step"])
+        med = fs[len(fs) // 2]
+        rec["formats"][f] = {
+            "pair_bytes": iq[f].element_size() * 2,
+            "channelizer": {"ms_per_step_median": statistics.median(ms), "ms_per_step_min": min(ms),
+                            "ms_per_step_max": max(ms)},
+            "full_step": dict(med, ms_per_step_min=fs[0]["ms_per_step"], ms_per_step_max=fs[-1]["ms_per_step"])}
+    return rec
 
 
 def main():
@@ -185,7 +272,7 @@ def main():
     ap.add_argument("out_dir")
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--only", choices=["a", "b"])
+    ap.add_argument("--only", choices=["a", "b", "formats"])
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -193,6 +280,14 @@ def main():
     import fmtuner_sdr_b200 as fm
     info = card()
     os.makedirs(args.out_dir, exist_ok=True)
+    if args.only == "formats":
+        rec = run_formats(fm, torch, args.steps, args.reps, seed=2000)
+        rec["card"] = info
+        line = json.dumps(rec)
+        print(line, flush=True)
+        with open(os.path.join(args.out_dir, "wideband_formats.jsonl"), "w") as f:
+            f.write(line + "\n")
+        return
     path = os.path.join(args.out_dir, "wideband_ingest.jsonl")
     with open(path, "w") as f:
         for i, (tag, kind, W, wide, D, Cn, c0s) in enumerate(WORKLOADS):
