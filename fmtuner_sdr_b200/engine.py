@@ -127,6 +127,13 @@ def load_library(build: bool = True):
                                                   C.c_double, i32, C.c_double, C.c_float, C.POINTER(vp)]
     L.fmgpu_channelizer_sample_format.argtypes = [vp]
     L.fmgpu_channelizer_process_iq.argtypes = [vp, vp, sz, sz, i32, i32, f32p, sz, vp]
+    L.fmgpu_channelizer_create_rate.argtypes = [i32, i32, i32, i32, i32, i32, C.POINTER(C.c_double),
+                                                C.c_double, i32, C.c_double, C.c_float, C.POINTER(vp)]
+    L.fmgpu_channelizer_interpolation.argtypes = [vp]
+    L.fmgpu_channelizer_decimation.argtypes = [vp]
+    L.fmgpu_channelizer_outputs.argtypes = [vp, sz]
+    L.fmgpu_channelizer_outputs.restype = sz
+    L.fmgpu_channelizer_process_stream.argtypes = [vp, vp, sz, sz, i32, i32, f32p, sz, C.POINTER(sz), vp]
     L.fmgpu_submit_host.argtypes = [vp, u8p, sz, i32, f32p, sz, vp, vp, sz, vp, vp]
     L.fmgpu_wait_host.argtypes = [vp, i32]
     L.fmgpu_decimate.restype = sz
@@ -527,11 +534,15 @@ class Channelizer:
 
     first_center_hz may be a sequence: one capture per entry, all advancing together, capture w's
     carrier k at first_center_hz[w] + k * spacing_hz from its own centre; its outputs are
-    n_captures * ch_count rows, capture-major."""
+    n_captures * ch_count rows, capture-major.
+
+    output_rate, when given, replaces decimation: the object resamples by the reduced ratio
+    U / D = output_rate / wide_rate (fmgpu_channelizer_create_rate, U <= 64), and a call writes a
+    varying number of outputs (outputs(), process_stream())."""
 
     def __init__(self, wide_rate=24_000_000, decimation=100, n_channels=100,
                  first_center_hz=-9_900_000.0, spacing_hz=200_000.0, taps_per_phase=16,
-                 cutoff_hz=100_000.0, atten_db=60.0, device=0, sample_format="cu8"):
+                 cutoff_hz=100_000.0, atten_db=60.0, device=0, sample_format="cu8", output_rate=None):
         if sample_format not in SAMPLE_FORMATS:
             raise ValueError(f"sample_format must be one of {sorted(SAMPLE_FORMATS)}, not {sample_format!r}")
         self.L = load_library()
@@ -540,21 +551,30 @@ class Channelizer:
         firsts = [float(first_center_hz)] if np.ndim(first_center_hz) == 0 else \
             [float(f) for f in first_center_hz]
         arr = (C.c_double * len(firsts))(*firsts)
-        rc = self.L.fmgpu_channelizer_create_format(device, SAMPLE_FORMATS[sample_format], len(firsts),
-                                                    wide_rate, decimation, n_channels, arr, spacing_hz,
-                                                    taps_per_phase, cutoff_hz, atten_db, C.byref(h))
+        if output_rate is None:
+            create, rate = self.L.fmgpu_channelizer_create_format, decimation
+        else:
+            create, rate = self.L.fmgpu_channelizer_create_rate, output_rate
+        rc = create(device, SAMPLE_FORMATS[sample_format], len(firsts), wide_rate, rate, n_channels, arr,
+                    spacing_hz, taps_per_phase, cutoff_hz, atten_db, C.byref(h))
         if rc != 0:
-            raise EngineError(f"fmgpu_channelizer_create_format failed ({rc}); no CPU fallback")
+            raise EngineError(f"{create.__name__} failed ({rc}); no CPU fallback")
         if np.ndim(first_center_hz) != 0:
             first_center_hz = firsts
         self.h = h
         self._format = sample_format
-        self.wide_rate, self.decimation, self.n_channels = wide_rate, decimation, n_channels
+        self.wide_rate, self.n_channels = wide_rate, n_channels
+        self.decimation = self.L.fmgpu_channelizer_decimation(h)
         self.first_center_hz, self.spacing_hz = first_center_hz, spacing_hz
 
     @property
     def output_rate(self) -> int:
         return self.L.fmgpu_channelizer_output_rate(self.h)
+
+    @property
+    def interpolation(self) -> int:
+        """U of the rate ratio U / D (1 unless output_rate was given)."""
+        return self.L.fmgpu_channelizer_interpolation(self.h)
 
     @property
     def n_captures(self) -> int:
@@ -585,6 +605,23 @@ class Channelizer:
                                                  out_dev_ptr, out_stride_samples, stream)
         if rc != 0:
             raise EngineError(f"fmgpu_channelizer_process_iq failed ({rc})")
+
+    def outputs(self, n_in) -> int:
+        """Outputs per row the next call with n_in pairs per capture writes."""
+        return self.L.fmgpu_channelizer_outputs(self.h, n_in)
+
+    def process_stream(self, iq_dev_ptr, n_in, out_dev_ptr, out_stride_samples, ch_first=0, ch_count=None,
+                       stream=None, iq_stride_bytes=None) -> int:
+        """As process, for any object and any n_in >= 1 (fmgpu_channelizer_process_stream): writes
+        outputs [0, n_out) of every row and returns n_out."""
+        ch_count = self.n_channels - ch_first if ch_count is None else ch_count
+        stride = self.pair_bytes * n_in if iq_stride_bytes is None else iq_stride_bytes
+        n_out = C.c_size_t()
+        rc = self.L.fmgpu_channelizer_process_stream(self.h, iq_dev_ptr, stride, n_in, ch_first, ch_count,
+                                                     out_dev_ptr, out_stride_samples, C.byref(n_out), stream)
+        if rc != 0:
+            raise EngineError(f"fmgpu_channelizer_process_stream failed ({rc})")
+        return n_out.value
 
     def close(self):
         if self.h:

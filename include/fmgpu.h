@@ -266,8 +266,20 @@ int fmgpu_xdr_rds_lines(fmgpu_xdr_rds_state *s, const fmgpu_rds_group *g, char l
  * Sample formats: all captures of one object share one format (a mixed fleet uses one object per
  * format). Only the load of a pair differs; the filter, the bank and the outputs' layout do not.
  * bladeRF's SC16_Q11 samples are cs16 with full scale 2048, so their outputs come out 16x smaller,
- * which the scale-invariant discriminator behind the channelizer does not notice. */
-#define FMGPU_IQ_CU8 0   /* uint8 I,Q, offset binary: RTL-SDR */
+ * which the scale-invariant discriminator behind the channelizer does not notice.
+ *
+ * Rational rates (fmgpu_channelizer_create_rate): with U/D the reduced ratio output_rate / wide_rate
+ * (gcd(U, D) = 1, U <= 64), the prototype h has L = D * taps_per_phase taps, designed at rate
+ * U * wide_rate with cut-off cutoff_hz / (U * wide_rate) and scaled by 2 fc U for unity pass-band
+ * gain, and
+ *   y_k[m] = sum_{n = 0..L-1, (mD - n) = 0 mod U} h[n] x[(mD - n)/U] exp(-j 2 pi f_k ((mD - n)/U) / wide_rate).
+ * Output m reads inputs up to s_m = floor(mD / U) through the phase filter g_q[i] = h[q + iU],
+ * q = mD mod U, at most Lin = ceil(L / U) taps. For U = 1 this is the definition above with the same
+ * taps. After T pairs per capture since creation, outputs 0 .. ceil(T U / D) - 1 exist, so a call
+ * with n_in pairs writes ceil((T + n_in) U / D) - ceil(T U / D) outputs: a count that varies from
+ * call to call (fmgpu_channelizer_outputs). create, create_multi and create_format are create_rate's
+ * U = 1 objects; fmgpu_channelizer_process_stream serves every object. */
+#define FMGPU_IQ_CU8 0  /* uint8 I,Q, offset binary: RTL-SDR */
 #define FMGPU_IQ_CS8 1   /* int8 I,Q: HackRF */
 #define FMGPU_IQ_CS16 2  /* int16 I,Q, native (little-endian) order: USRP, bladeRF, LimeSDR,
                             SDRplay (SoapySDR CS16) */
@@ -286,12 +298,27 @@ int fmgpu_channelizer_create_format(int device, int sample_format, int n_capture
                                     int decimation, int n_channels, const double *first_center_hz,
                                     double spacing_hz, int taps_per_phase, double cutoff_hz,
                                     float atten_db, fmgpu_channelizer **out);
+/* An object whose output rate is output_rate, a rational fraction U/D of wide_rate (see "Rational
+ * rates" above). FMGPU_EINVAL when output_rate < 1, output_rate > wide_rate or U > 64; the other
+ * checks are create_format's. With U = 1 it is the create_format object of decimation D, bit for bit. */
+int fmgpu_channelizer_create_rate(int device, int sample_format, int n_captures, int wide_rate,
+                                  int output_rate, int n_channels, const double *first_center_hz,
+                                  double spacing_hz, int taps_per_phase, double cutoff_hz, float atten_db,
+                                  fmgpu_channelizer **out);
 void fmgpu_channelizer_destroy(fmgpu_channelizer *z);
+/* wide_rate * U / D, an exact integer for create_rate objects (wide_rate / decimation, rounded down,
+ * for create_format objects) */
 int fmgpu_channelizer_output_rate(const fmgpu_channelizer *z);
+int fmgpu_channelizer_interpolation(const fmgpu_channelizer *z);   /* U (1 unless create_rate) */
+int fmgpu_channelizer_decimation(const fmgpu_channelizer *z);      /* D */
 int fmgpu_channelizer_n_captures(const fmgpu_channelizer *z);
 /* the FMGPU_IQ_* format the object was created for */
 int fmgpu_channelizer_sample_format(const fmgpu_channelizer *z);
+/* the prototype's L = D * taps_per_phase taps, at rate U * wide_rate */
 size_t fmgpu_channelizer_taps(const fmgpu_channelizer *z, float *out, size_t cap);
+/* outputs per row that the next process call with n_in pairs per capture writes. Host state only:
+ * no device synchronisation. */
+size_t fmgpu_channelizer_outputs(const fmgpu_channelizer *z, size_t n_in);
 /* iq_dev: n_in uint8 I,Q pairs (n_in a multiple of the decimation) continuing the stream of the
  * previous call; out_cf32_dev [ch_count][out_stride_samples] complex float for channels
  * ch_first .. ch_first + ch_count - 1 (a rank of a sharded job extracts only its own channels from
@@ -314,10 +341,20 @@ int fmgpu_channelizer_process_multi(fmgpu_channelizer *z, const uint8_t *iq_dev,
 /* Any format, any number of captures: iq_dev [n_captures][iq_stride_bytes] holds n_in pairs of the
  * object's format per capture (pair size 2 bytes for cu8 and cs8, 4 for cs16). FMGPU_EINVAL when the
  * stride is not a multiple of the pair size or shorter than pair size * n_in, or iq_dev is not
- * aligned to the pair size; otherwise as fmgpu_channelizer_process_multi. */
+ * aligned to the pair size; otherwise as fmgpu_channelizer_process_multi. FMGPU_EINVAL on an object
+ * with U > 1: it is fmgpu_channelizer_process_stream restricted to U = 1 and n_in a multiple of D. */
 int fmgpu_channelizer_process_iq(fmgpu_channelizer *z, const void *iq_dev, size_t iq_stride_bytes,
                                  size_t n_in, int ch_first, int ch_count, float *out_cf32_dev,
                                  size_t out_stride_samples, void *stream);
+/* Any object, any n_in >= 1 pairs per capture (a multiple of D or not): writes outputs
+ * [0, fmgpu_channelizer_outputs(z, n_in)) of every row of out_cf32_dev
+ * [n_captures][ch_count][out_stride_samples] and stores that count in *n_out (n_out may be NULL).
+ * A call that completes no output only carries the history. FMGPU_EINVAL when out_stride_samples is
+ * less than that count; the input stride, alignment and channel checks are process_iq's.
+ * Asynchronous on `stream`. */
+int fmgpu_channelizer_process_stream(fmgpu_channelizer *z, const void *iq_dev, size_t iq_stride_bytes,
+                                     size_t n_in, int ch_first, int ch_count, float *out_cf32_dev,
+                                     size_t out_stride_samples, size_t *n_out, void *stream);
 
 /* fmgpu_process_batch with complex-float input at the DSP rate (engine created with
  * decimation = 1): x_cf32_dev [C][stride_samples] interleaved re,im; base and stride 16-byte

@@ -1,10 +1,11 @@
 #!/usr/bin/env python
 """Many wideband captures through one channelizer: what batching the captures buys.
 
-Usage: python tools/wideband_ingest.py OUT_DIR [--steps K] [--reps R] [--only a|b|formats]
+Usage: python tools/wideband_ingest.py OUT_DIR [--steps K] [--reps R] [--only a|b|formats|rational]
 
 Writes OUT_DIR/wideband_ingest.jsonl, one JSON line per workload (the formats workload runs only
-with --only formats and writes OUT_DIR/wideband_formats.jsonl), each with the card name, power
+with --only formats and writes OUT_DIR/wideband_formats.jsonl; the rational workloads run only with
+--only rational and write OUT_DIR/wideband_rational.jsonl), each with the card name, power
 limit and maximum SM clock read (nvidia-smi, read-only) in the same run. One step is 68 ms of
 signal per capture: two 8192-sample blocks at 240 kS/s.
 
@@ -26,6 +27,13 @@ Per workload:
              (fmgpu_channelizer_create_format) on inputs of the same number of pairs (cs16: twice
              the bytes): the channelizer stage alone, formats alternated rep by rep, and the full
              step above for each format, reps alternated the same way, through one engine
+
+  (rational) 32 captures each, through fmgpu_channelizer_create_rate / _process_stream, with the
+             same 16384 output instants per step (the pairs per step vary where U > 1):
+               20 MS/s cs8  -> 240 kS/s (U = 3, D = 250), 100 carriers
+               24 MS/s cs8  -> 240 kS/s (U = 1, D = 100), 100 carriers
+               10 MS/s cs16 -> 256 kS/s (U = 16, D = 625), 50 carriers
+             the channelizer stage alone and the full step above, workloads alternated rep by rep
 
 Inputs are seeded random samples generated on the device. Needs a CUDA device: without one it fails.
 """
@@ -267,12 +275,104 @@ def run_formats(fm, torch, steps, reps, seed):
     return rec
 
 
+RATIONAL = [("20M_cs8_240k", 20_000_000, 240_000, 100, "cs8"), ("24M_cs8_240k", 24_000_000, 240_000, 100, "cs8"),
+            ("10M_cs16_256k", 10_000_000, 256_000, 50, "cs16")]
+
+
+class StreamSteps:
+    """A rational-rate object behind FullStep's process() call: step k feeds the pairs that complete
+    exactly B * BLOCK more outputs per row (fmgpu_channelizer_process_stream)."""
+
+    def __init__(self, z):
+        self.z, self.k = z, 0
+        U, D, n_dsp = z.interpolation, z.decimation, B * BLOCK
+        # smallest T with ceil(T U / D) >= m outputs: floor((m - 1) D / U) + 1
+        self.need = lambda m: ((m - 1) * D) // U + 1
+        self.max_in = max(self.need((k + 1) * n_dsp) - self.need(k * n_dsp) for k in range(1, 2 * U + 2))
+        self.T = 0
+
+    def process(self, iq_ptr, n_in, out_ptr, n_dsp, stream=None, iq_stride_bytes=None):
+        n = self.need((self.k + 1) * n_dsp) - self.T
+        got = self.z.process_stream(iq_ptr, n, out_ptr, n_dsp, stream=stream, iq_stride_bytes=iq_stride_bytes)
+        assert got == n_dsp, (got, n_dsp)
+        self.k += 1
+        self.T += n
+
+
+def run_rational(fm, torch, steps, reps, seed):
+    W = 32
+    dev = torch.device("cuda", 0)
+    n_dsp = B * BLOCK
+    s = torch.cuda.Stream()
+    sp = s.cuda_stream
+    g = torch.Generator(device=dev)
+    g.manual_seed(seed)
+    objs, iq = {}, {}
+    for name, wide, out_rate, Cn, fmt in RATIONAL:
+        c0 = -(Cn - 1) / 2.0
+        z = fm.Channelizer(wide_rate=wide, output_rate=out_rate, n_channels=Cn, first_center_hz=[c0 * SP] * W,
+                           spacing_hz=SP, taps_per_phase=16, cutoff_hz=100_000.0, sample_format=fmt)
+        objs[name] = StreamSteps(z)
+        row = 2 * objs[name].max_in
+        iq[name] = (torch.randint(-128, 128, (W, row), dtype=torch.int8, device=dev, generator=g) if fmt == "cs8" else
+                    torch.randint(-32768, 32768, (W, row), dtype=torch.int16, device=dev, generator=g))
+    Cmax = max(r[3] for r in RATIONAL)
+    out = torch.zeros((W * Cmax, n_dsp, 2), dtype=torch.float32, device=dev)
+
+    def timed(name):
+        st, x = objs[name], iq[name]
+        stride = x[0].numel() * x.element_size()
+        e0, e1 = ev(), ev()
+        torch.cuda.synchronize()
+        e0.record(s)
+        for _ in range(steps):
+            st.process(x.data_ptr(), None, out.data_ptr(), n_dsp, stream=sp, iq_stride_bytes=stride)
+        e1.record(s)
+        e1.synchronize()
+        return e0.elapsed_time(e1) / steps
+
+    for name in objs:                           # warm-up
+        for _ in range(2):
+            timed(name)
+    chan = {name: [] for name in objs}
+    for _ in range(reps):
+        for name in objs:
+            chan[name].append(timed(name))
+    full = {name: [] for name in objs}
+    engs = {Cn: FullStep(fm, torch, W * Cn, s) for Cn in sorted({r[3] for r in RATIONAL})}
+    for _ in range(reps):
+        for name, wide, out_rate, Cn, fmt in RATIONAL:
+            full[name].append(engs[Cn].run(objs[name], iq[name], None, out, steps))
+    for e in engs.values():
+        e.close()
+    rec = {"workload": "rational", "captures": W, "taps_per_phase": 16, "form": "polyphase", "steps": steps,
+           "reps": reps, "outputs_per_row_per_step": n_dsp, "workloads": {}}
+    for name, wide, out_rate, Cn, fmt in RATIONAL:
+        z = objs[name].z
+        U, D = z.interpolation, z.decimation
+        Lin = -(-D * 16 // U)
+        ms = chan[name]
+        fs = sorted(full[name], key=lambda r: r["ms_per_step"])
+        med = fs[len(fs) // 2]
+        rtf = n_dsp / out_rate / (med["ms_per_step"] * 1e-3)    # FullStep assumes 240 kS/s
+        rec["workloads"][name] = {
+            "wide_rate": wide, "output_rate": out_rate, "U": U, "D": D, "carriers_per_capture": Cn,
+            "sample_format": fmt, "P": int(wide // SP), "Lin": Lin, "pairs_per_capture_per_step": n_dsp * D / U,
+            "signal_ms_per_step": n_dsp / out_rate * 1e3,
+            "channelizer": {"ms_per_step_median": statistics.median(ms), "ms_per_step_min": min(ms),
+                            "ms_per_step_max": max(ms)},
+            "full_step": dict(med, realtime_factor=rtf, realtime_captures_per_gpu=W * rtf,
+                              ms_per_step_min=fs[0]["ms_per_step"], ms_per_step_max=fs[-1]["ms_per_step"])}
+        z.close()
+    return rec
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("out_dir")
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--only", choices=["a", "b", "formats"])
+    ap.add_argument("--only", choices=["a", "b", "formats", "rational"])
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -286,6 +386,14 @@ def main():
         line = json.dumps(rec)
         print(line, flush=True)
         with open(os.path.join(args.out_dir, "wideband_formats.jsonl"), "w") as f:
+            f.write(line + "\n")
+        return
+    if args.only == "rational":
+        rec = run_rational(fm, torch, args.steps, args.reps, seed=3000)
+        rec["card"] = info
+        line = json.dumps(rec)
+        print(line, flush=True)
+        with open(os.path.join(args.out_dir, "wideband_rational.jsonl"), "w") as f:
             f.write(line + "\n")
         return
     path = os.path.join(args.out_dir, "wideband_ingest.jsonl")
