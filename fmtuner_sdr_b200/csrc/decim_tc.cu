@@ -22,9 +22,11 @@
 //
 // One CTA per SM, persistent over (128-channel row tile, time segment) work items:
 //   warp 0     TMA producer: 16 KB chunks (128 rows x 128 B) into a ring of shared-memory slots
-//   warp 1     allocates TMEM, copies every chunk into the TMEM A ring (tcgen05.cp) and issues the MMAs
-//              with the A operand in TMEM (one elected lane); tcgen05.commit frees the ring slots
+//   warp 1     allocates TMEM and issues the MMAs with the A operand in TMEM (one elected lane)
 //   warps 2-5  epilogue: tcgen05.ld the 128 accumulator columns of a tile, recombine, store float2
+//   warp 6     copies every chunk from its shared-memory slot into the TMEM A ring (tcgen05.cp)
+// mbarrier pairs between them: full / empty (shared-memory ring), A full / A empty (TMEM A ring),
+// T full / T empty (accumulators); tcgen05.commit arrives as soon as the operations that read a slot retire.
 // Window of tile t (16 outputs): block-relative bytes [ADV*t - WS0, ADV*t - WS0 + 32*KS), ADV = 32*M,
 // WS0 = roundup(2L - 2, 32); the bytes in front of the block come from the per-channel history
 // buffer (hist tensor map), invalid history is byte 0 and is compensated in the offset term.
@@ -61,13 +63,13 @@ constexpr int TC_B_BYTES = TC_B_CHUNKS * TC_N * TC_CHUNK;   // 112 KB
 // TMEM: a slot is free again as soon as its four tcgen05.cp retire, so the ring only covers the TMA
 // latency (five slots; B takes 112 KB of the CTA's 194 KB).
 constexpr int TC_RING_TMEM_A = 5;
-constexpr int TC_ACC = 2;             // (the form with the A operand in shared memory is not built any more)
 // TMEM: columns [0, 256) hold a ring of eight chunks (32 columns = 128 bytes of K per lane; a tile's
 // window touches up to eight), columns [256, 512) two accumulators of 128 columns
 constexpr int TC_A_SLOTS = 8;
 constexpr int TC_A_COLS = 32;
-constexpr int TC_ACC_TS = 2;
-constexpr int TC_THREADS = 192;
+constexpr int TC_ACC = 2;
+constexpr int TC_COPY_WARP = 6;
+constexpr int TC_THREADS = 224;
 constexpr int TC_SHIFT = 26;          // taps are quantised to 2^-26
 constexpr size_t tcSmemBytes(int ring) { return 1024 + TC_B_BYTES + (size_t)ring * TC_CHUNK_BYTES + 512; }
 
@@ -102,34 +104,35 @@ constexpr int TC_MAX_KSTEPS = 4 * TC_B_CHUNKS;   // 28
 constexpr int TC_WIN_CHUNKS = 8;                 // an 896-byte window starting at a 32-byte phase touches <= 8 chunks
 
 // The MMAs of one tile, fully unrolled for the window's phase PH (its start inside a chunk, in
-// 32-byte steps): every shared-memory offset is then an immediate. cb[r] / eb[r]: descriptor low
-// word and `empty` barrier of the window's r-th chunk; the first n_free chunks are released.
-template <int PH, bool ATMEM, int KS>
-__device__ __forceinline__ void issueTile(int ksteps_rt, int n_free, const uint32_t (&cb)[TC_WIN_CHUNKS],
+// 32-byte steps): every operand offset is then an immediate. cb[r] / eb[r]: TMEM column and `A empty`
+// barrier of the window's r-th chunk; the first n_free chunks are released right behind the last K
+// step that reads them, so that the copy warp can refill their slots while the tile's later K steps run.
+// af[r] / ap[r]: `A full` barrier and parity of chunk r. The chunks from n_have on are waited for
+// right before the first K step that reads them: the K steps over chunks already in TMEM queue up
+// behind the previous tile while the copy warp still brings the new ones.
+template <int PH, int KS>
+__device__ __forceinline__ void issueTile(int ksteps_rt, int n_free, int n_have, const uint32_t (&af)[TC_WIN_CHUNKS],
+                                          const uint32_t (&ap)[TC_WIN_CHUNKS], const uint32_t (&cb)[TC_WIN_CHUNKS],
                                           const uint32_t (&eb)[TC_WIN_CHUNKS], uint32_t b_lo0,
                                           uint32_t desc_hi, uint32_t d_tmem, uint32_t idesc) {
-  // KS > 0: the K-step count is a compile-time constant (23 for /10, 18 for /8): no per-step test
+  // KS > 0: the K-step count is a compile-time constant (28 for /10, 22 for /8): no per-step test
   const int ksteps = (KS > 0) ? KS : ksteps_rt;
 #pragma unroll
   for (int ks = 0; ks < ((KS > 0) ? KS : TC_MAX_KSTEPS); ks++) {
     if (KS > 0 || ks < ksteps) {
-      constexpr int dummy = 0;
-      (void)dummy;
       const int byte = 32 * PH + 32 * ks;
       const int r = byte >> 7;
       const uint32_t b_lo = b_lo0 + (ks >> 2) * ((TC_N * TC_CHUNK) >> 4) + (ks & 3) * 2;
       const uint64_t b_desc = (static_cast<uint64_t>(desc_hi) << 32) | b_lo;
-      if (ATMEM) {
-        const uint32_t a_col = cb[r] + ((byte & (TC_CHUNK - 1)) >> 2);   // 4 bytes of K per column
-        ummaI8Ts(d_tmem, a_col, b_desc, idesc, ks == 0 ? 0u : 1u);
-      } else {
-        const uint32_t a_lo = cb[r] + ((byte & (TC_CHUNK - 1)) >> 4);
-        const uint64_t a_desc = (static_cast<uint64_t>(desc_hi) << 32) | a_lo;
-        ummaI8(d_tmem, a_desc, b_desc, idesc, ks == 0 ? 0u : 1u);
-        const bool chunk_done = (((byte + 32) & (TC_CHUNK - 1)) == 0) || (ks + 1 == ksteps);
-        if (chunk_done && r < n_free) {
-          ummaCommit(eb[r]);
-        }
+      const uint32_t a_col = cb[r] + ((byte & (TC_CHUNK - 1)) >> 2);   // 4 bytes of K per column
+      if ((ks == 0 || (byte & (TC_CHUNK - 1)) == 0) && r >= n_have) {
+        mbarWait(af[r], ap[r]);
+        tcFenceAfter();
+      }
+      ummaI8Ts(d_tmem, a_col, b_desc, idesc, ks == 0 ? 0u : 1u);
+      const bool chunk_done = (((byte + 32) & (TC_CHUNK - 1)) == 0) || (ks + 1 == ksteps);
+      if (chunk_done && r < n_free) {
+        ummaCommit(eb[r]);
       }
     }
   }
@@ -164,23 +167,24 @@ struct ChunkCursor {
   }
 };
 
-template <bool ATMEM, int KS>
+template <int KS>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_decim_tc(const __grid_constant__ CUtensorMap tm_iq, const __grid_constant__ CUtensorMap tm_hist,
            const uint4 *__restrict__ b_image, const int2 *__restrict__ offs, const int *__restrict__ hist_valid,
            float2 *__restrict__ x1, size_t x1_pitch, const TcParams p) {
-  static_assert(ATMEM, "the A operand lives in TMEM: with 16-output tiles B (112 KB) leaves no room for a ten-slot ring");
-  constexpr int NACC = ATMEM ? TC_ACC_TS : TC_ACC;
-  constexpr uint32_t ACC_COL0 = ATMEM ? TC_A_SLOTS * TC_A_COLS : 0;   // first accumulator column
+  constexpr int NACC = TC_ACC;
+  constexpr uint32_t ACC_COL0 = TC_A_SLOTS * TC_A_COLS;   // first accumulator column
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smemAddr(smem_raw) + 1023u) & ~1023u;
   const uint32_t sB = base;
   const uint32_t sA = base + TC_B_BYTES;
   const int RING = p.ring;
   const uint32_t sBar = sA + RING * TC_CHUNK_BYTES;
-  // barriers: full[RING], empty[RING], tfull[ACC], tempty[ACC]; then the TMEM base word
+  // barriers: full[RING], empty[RING], tfull[ACC], tempty[ACC], afull[A_SLOTS], aempty[A_SLOTS]; then
+  // the TMEM base word
   const uint32_t barFull = sBar, barEmpty = sBar + 8 * RING, barTFull = sBar + 16 * RING,
-                 barTEmpty = barTFull + 8 * NACC, sTmem = barTEmpty + 8 * NACC;
+                 barTEmpty = barTFull + 8 * NACC, barAFull = barTEmpty + 8 * NACC,
+                 barAEmpty = barAFull + 8 * TC_A_SLOTS, sTmem = barAEmpty + 8 * TC_A_SLOTS;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_work = p.row_tiles * p.n_seg;
 
@@ -200,6 +204,10 @@ k_decim_tc(const __grid_constant__ CUtensorMap tm_iq, const __grid_constant__ CU
     for (int i = 0; i < NACC; i++) {
       mbarInit(barTFull + 8 * i, 1);
       mbarInit(barTEmpty + 8 * i, 4);   // one arrival per epilogue warp
+    }
+    for (int i = 0; i < TC_A_SLOTS; i++) {
+      mbarInit(barAFull + 8 * i, 1);    // tcgen05.commit of the copy warp
+      mbarInit(barAEmpty + 8 * i, 1);   // tcgen05.commit of the MMA issuer
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -236,98 +244,112 @@ k_decim_tc(const __grid_constant__ CUtensorMap tm_iq, const __grid_constant__ CU
     }
   } else if (warp == 1) {
     // ===== MMA issuer: the whole warp keeps the (warp-uniform) books, one elected lane issues ======
-    {
-      // u8 x s8 -> s32, K-major A and B, N = 64, M = 128 (UMMA::InstrDescriptor)
-      const uint32_t idesc = (2u << 4) | (0u << 7) | (1u << 10) | ((TC_N >> 3) << 17) | ((TC_ROWS >> 4) << 24);
-      const uint32_t desc_hi = static_cast<uint32_t>(smemDesc(0) >> 32);
-      const uint32_t a_lo0 = static_cast<uint32_t>(smemDesc(sA));
-      const uint32_t b_lo0 = static_cast<uint32_t>(smemDesc(sB));
-      uint32_t ring = 0;    // ring slot and use count of the next chunk to wait for
-      uint32_t ring_use = 0;
-      uint32_t a_slot = 0;  // ATMEM: TMEM slot of the next chunk to copy
-      uint32_t tile_cnt = 0;
-      for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-        int row, t0, nt;
-        workItem(p, w, &row, &t0, &nt);
-        const int g0 = windowStart(p, t0) / TC_CHUNK;
-        const int g1 = (windowStart(p, t0 + nt - 1) + 32 * p.ksteps - 1) / TC_CHUNK;
-        int have = g0 - 1;          // chunks known to have landed
-        int gs = g0;                // first chunk of the current window ...
-        uint32_t gs_slot = ATMEM ? a_slot : ring;   // ... and its slot (TMEM A ring / smem ring)
-        for (int i = 0; i < nt; i++, tile_cnt++) {
-          const int ws = windowStart(p, t0 + i);
-          const int ge = (ws + 32 * p.ksteps - 1) / TC_CHUNK;
-          const uint32_t acc = tile_cnt % NACC;
-          const uint32_t ause = tile_cnt / NACC;
-          if (ause > 0) {
-            mbarWait(barTEmpty + 8 * acc, (ause - 1) & 1);
-          }
-          while (have < ge) {
-            have++;
-            mbarWait(barFull + 8 * ring, ring_use & 1);
-            if (ATMEM) {
-              // the chunk goes to TMEM once (4 x tcgen05.cp 128x256b = 128 lanes x 32 bytes each), every
-              // MMA that uses it reads it from there, and its shared-memory slot is free as soon as
-              // the copies retire. cp and mma execute in issue order, so a later copy into the same
-              // TMEM slot cannot overtake the MMAs still reading it (a window spans <= 7 of 8 slots).
-              tcFenceAfter();
-              if (electOne()) {
-                const uint32_t a_col = tmem_base + a_slot * TC_A_COLS;
-                const uint32_t src = a_lo0 + ring * (TC_CHUNK_BYTES >> 4);
+    // u8 x s8 -> s32, K-major A and B, N = 128, M = 128 (UMMA::InstrDescriptor)
+    const uint32_t idesc = (2u << 4) | (0u << 7) | (1u << 10) | ((TC_N >> 3) << 17) | ((TC_ROWS >> 4) << 24);
+    const uint32_t desc_hi = static_cast<uint32_t>(smemDesc(0) >> 32);
+    const uint32_t b_lo0 = static_cast<uint32_t>(smemDesc(sB));
+    uint32_t a_wait = 0, a_wait_use = 0;   // TMEM slot and use count of the next chunk to wait for
+    uint32_t gs_slot = 0;                  // TMEM slot of the current window's first chunk
+    uint32_t tile_cnt = 0;
+    for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
+      int row, t0, nt;
+      workItem(p, w, &row, &t0, &nt);
+      const int g0 = windowStart(p, t0) / TC_CHUNK;
+      const int g1 = (windowStart(p, t0 + nt - 1) + 32 * p.ksteps - 1) / TC_CHUNK;
+      int have = g0 - 1;   // chunks known to be in TMEM
+      int gs = g0;         // first chunk of the current window
+      for (int i = 0; i < nt; i++, tile_cnt++) {
+        const int ws = windowStart(p, t0 + i);
+        const int ge = (ws + 32 * p.ksteps - 1) / TC_CHUNK;
+        const uint32_t acc = tile_cnt % NACC;
+        const uint32_t ause = tile_cnt / NACC;
+        if (ause > 0) {
+          mbarWait(barTEmpty + 8 * acc, (ause - 1) & 1);
+        }
+        // the window's chunks up to `have` were waited for by earlier tiles; the issuing lane waits
+        // for the others inside issueTile
+        const int n_have = have - gs + 1;
+        uint32_t af[TC_WIN_CHUNKS], ap[TC_WIN_CHUNKS];   // A full barrier / parity per window chunk
+        {
 #pragma unroll
-                for (int sstep = 0; sstep < 4; sstep++) {
-                  tmemCp128x256(a_col + sstep * 8, (static_cast<uint64_t>(desc_hi) << 32) | (src + 2 * sstep));
-                }
-                ummaCommit(barEmpty + 8 * ring);
-              }
-              __syncwarp();
-              a_slot = (a_slot + 1 == TC_A_SLOTS) ? 0 : a_slot + 1;
-            }
-            if (++ring == static_cast<uint32_t>(RING)) {
-              ring = 0;
-              ring_use++;
-            }
+          for (int r = 0; r < TC_WIN_CHUNKS; r++) {
+            const uint32_t j = a_wait + static_cast<uint32_t>(max(r - n_have, 0));
+            af[r] = barAFull + 8 * (j % TC_A_SLOTS);
+            ap[r] = (a_wait_use + j / TC_A_SLOTS) & 1;
           }
-          tcFenceAfter();
-          // chunks in front of the next tile's window go back to the producer as soon as the MMAs
-          // that read them are done: a commit right behind the last K step inside them
-          const int keep = (i + 1 < nt) ? windowStart(p, t0 + i + 1) / TC_CHUNK : g1 + 1;
-          const int n_free = keep - gs;
-          uint32_t cb[TC_WIN_CHUNKS], eb[TC_WIN_CHUNKS];   // descriptor / empty barrier per window chunk
-          {
-            uint32_t slot = gs_slot;
+          const uint32_t j = a_wait + static_cast<uint32_t>(ge - have);
+          a_wait = j % TC_A_SLOTS;
+          a_wait_use += j / TC_A_SLOTS;
+          have = ge;
+        }
+        tcFenceAfter();
+        // chunks in front of the next tile's window go back to the copy warp as soon as the MMAs
+        // that read them are done: a commit right behind the last K step inside them
+        const int keep = (i + 1 < nt) ? windowStart(p, t0 + i + 1) / TC_CHUNK : g1 + 1;
+        const int n_free = keep - gs;
+        uint32_t cb[TC_WIN_CHUNKS], eb[TC_WIN_CHUNKS];   // TMEM column / A empty barrier per window chunk
+        {
+          uint32_t slot = gs_slot;
 #pragma unroll
-            for (int r = 0; r < TC_WIN_CHUNKS; r++) {
-              if (ATMEM) {
-                cb[r] = tmem_base + slot * TC_A_COLS;   // TMEM column of the chunk
-                eb[r] = 0;
-                slot = (slot + 1 == TC_A_SLOTS) ? 0 : slot + 1;
-              } else {
-                cb[r] = a_lo0 + slot * (TC_CHUNK_BYTES >> 4);
-                eb[r] = barEmpty + 8 * slot;
-                slot = (slot + 1 == static_cast<uint32_t>(RING)) ? 0 : slot + 1;
-              }
-            }
-          }
-          const uint32_t d_tmem = tmem_base + ACC_COL0 + acc * TC_N;
-          const uint32_t tfull = barTFull + 8 * acc;
-          if (electOne()) {
-            switch ((ws & (TC_CHUNK - 1)) >> 5) {
-              case 0: issueTile<0, ATMEM, KS>(p.ksteps, n_free, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
-              case 1: issueTile<1, ATMEM, KS>(p.ksteps, n_free, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
-              case 2: issueTile<2, ATMEM, KS>(p.ksteps, n_free, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
-              default: issueTile<3, ATMEM, KS>(p.ksteps, n_free, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
-            }
-            ummaCommit(tfull);
-          }
-          __syncwarp();
-          while (gs < keep) {   // the next window starts here
-            gs++;
-            if (++gs_slot == static_cast<uint32_t>(ATMEM ? TC_A_SLOTS : RING)) {
-              gs_slot = 0;
-            }
+          for (int r = 0; r < TC_WIN_CHUNKS; r++) {
+            cb[r] = tmem_base + slot * TC_A_COLS;
+            eb[r] = barAEmpty + 8 * slot;
+            slot = (slot + 1 == TC_A_SLOTS) ? 0 : slot + 1;
           }
         }
+        const uint32_t d_tmem = tmem_base + ACC_COL0 + acc * TC_N;
+        const uint32_t tfull = barTFull + 8 * acc;
+        if (electOne()) {
+          switch ((ws & (TC_CHUNK - 1)) >> 5) {
+            case 0: issueTile<0, KS>(p.ksteps, n_free, n_have, af, ap, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
+            case 1: issueTile<1, KS>(p.ksteps, n_free, n_have, af, ap, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
+            case 2: issueTile<2, KS>(p.ksteps, n_free, n_have, af, ap, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
+            default: issueTile<3, KS>(p.ksteps, n_free, n_have, af, ap, cb, eb, b_lo0, desc_hi, d_tmem, idesc); break;
+          }
+          ummaCommit(tfull);
+        }
+        __syncwarp();
+        gs = keep;   // the next window starts here
+        gs_slot = (gs_slot + n_free) % TC_A_SLOTS;
+      }
+    }
+  } else if (warp == TC_COPY_WARP) {
+    // ===== chunk copier: shared-memory ring -> TMEM A ring, in the producer's chunk order ==========
+    // Every chunk goes to TMEM once (4 x tcgen05.cp 128x256b = 128 lanes x 32 bytes each) and every MMA
+    // that uses it reads it from there. Its shared-memory slot is free as soon as the copies retire
+    // (empty); the MMA issuer waits for A full before the first MMA that reads the chunk. A copy into
+    // a TMEM slot waits for A empty, which the issuer commits behind the last MMA that reads the slot's
+    // previous chunk: cp and mma come from different warps, so the barrier, not issue order, keeps a
+    // copy from overtaking those MMAs. A window touches at most all eight slots, so the copies of the
+    // next tile's new chunks start as soon as the current tile's first K steps have retired.
+    const uint32_t desc_hi = static_cast<uint32_t>(smemDesc(0) >> 32);
+    const uint32_t a_lo0 = static_cast<uint32_t>(smemDesc(sA));
+    uint32_t ring = 0, ring_use = 0;   // shared-memory slot and use count of the next chunk
+    uint32_t a_slot = 0, a_use = 0;    // TMEM slot and use count it goes to
+    for (ChunkCursor cc(p, blockIdx.x, gridDim.x, n_work); cc.valid(); cc.next(p)) {
+      if (a_use > 0) {
+        mbarWait(barAEmpty + 8 * a_slot, (a_use - 1) & 1);
+      }
+      mbarWait(barFull + 8 * ring, ring_use & 1);
+      tcFenceAfter();
+      if (electOne()) {
+        const uint32_t a_col = tmem_base + a_slot * TC_A_COLS;
+        const uint32_t src = a_lo0 + ring * (TC_CHUNK_BYTES >> 4);
+#pragma unroll
+        for (int sstep = 0; sstep < 4; sstep++) {
+          tmemCp128x256(a_col + sstep * 8, (static_cast<uint64_t>(desc_hi) << 32) | (src + 2 * sstep));
+        }
+        ummaCommit(barEmpty + 8 * ring);
+        ummaCommit(barAFull + 8 * a_slot);
+      }
+      __syncwarp();
+      if (++a_slot == TC_A_SLOTS) {
+        a_slot = 0;
+        a_use++;
+      }
+      if (++ring == static_cast<uint32_t>(RING)) {
+        ring = 0;
+        ring_use++;
       }
     }
   } else {
@@ -543,8 +565,7 @@ cudaError_t launchDecimTc(int M, int L, const uint8_t *iq, size_t iq_stride, siz
                           cudaStream_t stream) {
   static DeviceOnce attrs;  // per device: device_once.h
   const cudaError_t attr_err = attrs.run([] {
-    const void *fs[] = {(const void *)k_decim_tc<true, 28>, (const void *)k_decim_tc<true, 22>,
-                        (const void *)k_decim_tc<true, 0>};
+    const void *fs[] = {(const void *)k_decim_tc<28>, (const void *)k_decim_tc<22>, (const void *)k_decim_tc<0>};
     cudaError_t err = cudaSuccess;
     for (const void *f : fs) {
       if (err == cudaSuccess) {
@@ -586,7 +607,7 @@ cudaError_t launchDecimTc(int M, int L, const uint8_t *iq, size_t iq_stride, siz
   const uint4 *bi = reinterpret_cast<const uint4 *>(b_image_dev);
   const int2 *of = reinterpret_cast<const int2 *>(offs_dev);
 #define FMGPU_TC_LAUNCH(KSV)                                                                              \
-  k_decim_tc<true, KSV><<<grid, TC_THREADS, smem_bytes, stream>>>(tm_iq, tm_hist, bi, of, hist_valid, x1, x1_pitch, p)
+  k_decim_tc<KSV><<<grid, TC_THREADS, smem_bytes, stream>>>(tm_iq, tm_hist, bi, of, hist_valid, x1, x1_pitch, p)
   if (p.ksteps == 28) {          // /10 at 2.4 MS/s
     FMGPU_TC_LAUNCH(28);
   } else if (p.ksteps == 22) {   // /8 at 2.048 MS/s

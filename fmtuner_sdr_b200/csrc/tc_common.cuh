@@ -63,18 +63,6 @@ __device__ __forceinline__ uint64_t smemDesc(uint32_t addr) {
   return d;
 }
 
-__device__ __forceinline__ void ummaI8(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                       uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t"
-      "}" ::"r"(tmem_d),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 // one lane of a converged warp; the region it guards is single-threaded and ptxas keeps its
 // warp-uniform operands in uniform registers (no waterfall loop around UTCIMMA / UTCBAR)
 __device__ __forceinline__ bool electOne() {
